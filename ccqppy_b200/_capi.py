@@ -25,7 +25,8 @@ EXPORTS = ["ccqp_abi_version", "ccqp_status_string", "ccqp_last_error", "ccqp_cr
            "ccqp_solve_batched", "ccqp_gemv", "ccqp_gemv_timed", "ccqp_project", "ccqp_normal", "ccqp_comm_export",
            "ccqp_comm_attach", "ccqp_comm_prepare", "ccqp_comm_detach", "ccqp_debug_divide", "ccqp_fp64_peak",
            "ccqp_microbench", "ccqp_debug_emulate_ranks", "ccqp_debug_solve_emulated", "ccqp_projected_gradient", "ccqp_solve_batched_table", "ccqp_solve_batched_sym",
-           "ccqp_get_upload_info", "ccqp_set_matrix_symmetric", "ccqp_host_matrix_is_block_symmetric", "ccqp_upload_block_rows"]
+           "ccqp_get_upload_info", "ccqp_set_matrix_symmetric", "ccqp_host_matrix_is_block_symmetric", "ccqp_upload_block_rows",
+           "ccqp_set_matrix_f32"]
 
 
 class Block(C.Structure):
@@ -86,6 +87,7 @@ def load():
     lib.ccqp_solve_batched_table.argtypes = [vp, i32, C.POINTER(Params), i64, i64, dp, dp, dp, C.POINTER(Block), i64, dp, i64, dp, i64,
                                              dp, i32, C.POINTER(Result), C.POINTER(Result)]
     lib.ccqp_set_matrix_symmetric.argtypes = [vp, dp, i64, i64, i32]
+    lib.ccqp_set_matrix_f32.argtypes = [vp, dp, i64, i64, i64, i64, i32]
     lib.ccqp_get_upload_info.argtypes = [vp, C.POINTER(i64), C.POINTER(i32)]
     lib.ccqp_host_matrix_is_block_symmetric.argtypes = [dp, i64, i64, i32]
     lib.ccqp_host_matrix_is_block_symmetric.restype = i32
@@ -171,6 +173,27 @@ class Handle:
         nbytes, mirrored = C.c_int64(), C.c_int32()
         check(self.h, self.lib.ccqp_get_upload_info(self.h, C.byref(nbytes), C.byref(mirrored)))
         return nbytes.value, bool(mirrored.value)
+
+    def set_matrix_f32(self, a, n, row_begin=0, n_rows=None):
+        """ccqp_set_matrix_f32 with rows [row_begin, row_begin + n_rows) of a float32 NumPy array or torch tensor of shape
+        (n_rows, n) whose rows are contiguous (lda = its row stride; a CUDA tensor is borrowed, anything else is copied
+        to the device)."""
+        n_rows = n if n_rows is None else n_rows
+        if isinstance(a, np.ndarray):
+            if a.dtype != np.float32:
+                raise TypeError("set_matrix_f32 takes float32, got %s" % a.dtype)
+            strides = tuple(s // 4 for s in a.strides) if a.ndim == 2 and all(s % 4 == 0 for s in a.strides) else None
+            ptr, mem = a.ctypes.data, MEM_HOST
+        else:
+            if str(a.dtype) != "torch.float32":
+                raise TypeError("set_matrix_f32 takes float32, got %s" % a.dtype)
+            strides = tuple(a.stride()) if a.dim() == 2 else None
+            ptr, mem = a.data_ptr(), (MEM_DEVICE if a.is_cuda else MEM_HOST)
+        if tuple(a.shape) != (n_rows, n) or strides is None or strides[1] != 1 or (n_rows > 1 and strides[0] < n):
+            raise ValueError("set_matrix_f32 needs an (%d, %d) matrix with contiguous rows, got shape %s strides %s"
+                             % (n_rows, n, tuple(a.shape), strides))
+        lda = strides[0] if n_rows > 1 else n
+        check(self.h, self.lib.ccqp_set_matrix_f32(self.h, C.c_void_p(ptr), int(n), int(lda), int(row_begin), int(n_rows), mem))
 
     def info(self):
         sm, grid, thr, smem = C.c_int32(), C.c_int32(), C.c_int32(), C.c_int64()

@@ -13,7 +13,7 @@
 #include <string>
 #include <vector>
 
-#define CCQP_DENSE_ONLY 1      // CSR Hessians run csr.cu's build of the kernels (emulated ranks: emu.cu's)
+#define CCQP_DENSE_ONLY 1      // CSR Hessians run csr.cu's build of the kernels (emulated ranks: emu.cu's), fp32 Hessians dense_f32.cu's
 #include "dense.cuh"
 #include "internal.h"
 #include "microbench.cuh"
@@ -42,8 +42,9 @@ struct ccqp_handle {
     bool own_stream = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::string last_error;
-    // matrix shard
+    // matrix shard (a_f32: dA points at floats, lda counts floats -- ccqp_set_matrix_f32)
     const double* dA = nullptr;
+    bool a_f32 = false;
     DevBuf a_own;
     // operator-form (CSR) alternative to dA
     const long long* d_ptr = nullptr;
@@ -225,7 +226,9 @@ void fill_ctx(ccqp_handle* h, DenseCtx& c, const Tiling& t) {
     std::memset(&c, 0, sizeof(c));
     double* w = reinterpret_cast<double*>(h->work.as<char>() + kSymVecOff);
     c.A = h->dA; c.lda = h->lda; c.n = (int)h->n; c.row0 = (int)h->row0; c.nrows = (int)h->nrows;
-    c.aligned = ((reinterpret_cast<uintptr_t>(h->dA) & 31) == 0 && (h->lda % 4) == 0) ? 1 : 0;
+    // 4 entries per vector load: 32-byte (fp64) / 16-byte (fp32) aligned rows; a contiguous widened copy of an fp32 matrix
+    // takes the same loop as the fp32 original
+    c.aligned = ((reinterpret_cast<uintptr_t>(h->dA) & (h->a_f32 ? 15 : 31)) == 0 && (h->lda % 4) == 0) ? 1 : 0;
     c.csr_ptr = h->d_ptr; c.csr_idx = h->d_idx; c.csr_val = h->d_val;
     {
         const double mean = h->d_val ? (double)h->nnz / (double)std::max<long long>(h->nrows, 1) : 0.0;
@@ -263,10 +266,11 @@ void fill_ctx(ccqp_handle* h, DenseCtx& c, const Tiling& t) {
     if (h->world == 1) c.x.base[0] = h->work.as<char>();
     c.out = h->out_dev.as<DenseOut>();
     c.CW = t.CW; c.SW = t.SW; c.np = t.np; c.nseg = t.nseg; c.rows_max = t.rows_max; c.psum_accum = t.accum;
-    c.evict_first = ((double)h->nrows * (double)h->n * 8.0 > 96.0 * 1024 * 1024) ? 1 : 0;
+    const double entry_bytes = h->a_f32 ? 4.0 : 8.0;
+    c.evict_first = ((double)h->nrows * (double)h->n * entry_bytes > 96.0 * 1024 * 1024) ? 1 : 0;
     c.evict_first = env_int("CCQP_EVICT_FIRST", c.evict_first, ok_bool);
     {   // a shard larger than L2: keep a fixed slice of it resident (same tasks every mat-vec), stream the rest evict-first
-        const double shard = (double)h->nrows * (double)h->n * 8.0;
+        const double shard = (double)h->nrows * (double)h->n * entry_bytes;
         const int mb = env_int("CCQP_L2_RESIDENT_MB", 64, [](int v) { return v >= 0 && v <= 120; });
         const double f = shard > 0 ? (double)mb * 1024.0 * 1024.0 / shard : 0.0;
         c.resident_256 = (int)std::min(256.0, std::floor(f * 256.0 + 0.5));
@@ -305,6 +309,12 @@ ccqp_status launch_dense(ccqp_handle* h, DenseCtx& c, const Tiling& t, bool coop
         static_assert(sizeof(DenseCtx) % 8 == 0, "DenseCtx");
         if (csr_variant_ctx_bytes() != sizeof(DenseCtx)) { h->last_error = "csr.cu was built from different headers"; return CCQP_ERR_CUDA; }
         CU(h, csr_variant_launch(OP, &c, t.grid, t.smem, cooperative, h->stream));
+        h->launches += 1;
+        return CCQP_OK;
+    }
+    if (h->a_f32) {         // fp32-stored Hessian: the build of the same kernels that widens A in registers (dense_f32.cu)
+        if (f32_variant_ctx_bytes() != sizeof(DenseCtx)) { h->last_error = "dense_f32.cu was built from different headers"; return CCQP_ERR_CUDA; }
+        CU(h, f32_variant_launch(OP, &c, t.grid, t.smem, cooperative, h->stream));
         h->launches += 1;
         return CCQP_OK;
     }
@@ -424,7 +434,7 @@ static ccqp_status set_matrix_dense(ccqp_handle* h, const double* A, int64_t n, 
     CU(h, cudaSetDevice(h->device));
     h->n = n; h->row0 = row_begin; h->nrows = n_rows;
     h->d_ptr = nullptr; h->d_idx = nullptr; h->d_val = nullptr; h->nnz = 0;
-    h->mirror_pending = false;
+    h->mirror_pending = false; h->a_f32 = false;
     if (memtype == CCQP_MEM_DEVICE) {
         h->dA = A; h->lda = lda;
         h->upload_mirrored = false; h->upload_bytes = 0;
@@ -453,6 +463,29 @@ ccqp_status ccqp_set_matrix_symmetric(ccqp_handle* h, const double* A, int64_t n
     return set_matrix_dense(h, A, n, lda, 0, n, memtype, true);
 }
 
+ccqp_status ccqp_set_matrix_f32(ccqp_handle* h, const float* A, int64_t n, int64_t lda, int64_t row_begin, int64_t n_rows,
+                                int memtype) {
+    if (!h || !A || n <= 0 || n >= (1LL << 31) - 256 || lda < n || row_begin < 0 || n_rows <= 0 || row_begin + n_rows > n)
+        return CCQP_ERR_INVALID_ARG;
+    CU(h, cudaSetDevice(h->device));
+    h->n = n; h->row0 = row_begin; h->nrows = n_rows;
+    h->d_ptr = nullptr; h->d_idx = nullptr; h->d_val = nullptr; h->nnz = 0;
+    h->mirror_pending = false; h->upload_mirrored = false;
+    if (memtype == CCQP_MEM_DEVICE) {
+        h->dA = reinterpret_cast<const double*>(A); h->lda = lda;
+        h->upload_bytes = 0;
+    } else {
+        const long long ldd = round_up(n, 4);   // keep rows 16-byte aligned for the 128-bit loads
+        CU(h, h->a_own.ensure((size_t)n_rows * ldd * 4 + 64));
+        CU(h, cudaMemcpy2DAsync(h->a_own.p, (size_t)ldd * 4, A, (size_t)lda * 4, (size_t)n * 4, (size_t)n_rows,
+                                cudaMemcpyHostToDevice, h->stream));
+        h->upload_bytes = n_rows * n * 4;
+        h->dA = h->a_own.as<double>(); h->lda = ldd;
+    }
+    h->a_f32 = true;
+    return CCQP_OK;
+}
+
 ccqp_status ccqp_get_upload_info(ccqp_handle* h, int64_t* bytes, int32_t* mirrored) {
     if (!h) return CCQP_ERR_INVALID_ARG;
     if (bytes) *bytes = h->upload_bytes;
@@ -474,7 +507,7 @@ ccqp_status ccqp_set_matrix_csr(ccqp_handle* h, const int64_t* indptr, const int
         return CCQP_ERR_INVALID_ARG;
     CU(h, cudaSetDevice(h->device));
     h->n = n; h->row0 = row_begin; h->nrows = n_rows; h->nnz = nnz;
-    h->dA = nullptr; h->lda = 0;
+    h->dA = nullptr; h->lda = 0; h->a_f32 = false;
     h->mirror_pending = false; h->upload_mirrored = false; h->upload_bytes = 0;
     if (memtype == CCQP_MEM_DEVICE) {
         h->d_ptr = reinterpret_cast<const long long*>(indptr); h->d_idx = indices; h->d_val = values;
@@ -615,8 +648,10 @@ void fill_result(const ccqp_handle* h, const DenseOut* o, float ms, long long la
     result->uniforms_used = o->draws;
     result->converged = o->converged;
     result->status = o->status;
+    // per mat-vec: CSR 12 bytes per stored entry + row pointers, dense 8 (fp32 Hessian: 4) bytes per entry, + v and y
+    const double entry_bytes = h->a_f32 ? 4.0 : 8.0;
     result->hbm_bytes = h->d_val ? (double)o->gemv * (12.0 * (double)h->nnz + 8.0 * (double)(h->nrows + 1) + 8.0 * (double)n + 8.0 * (double)h->nrows)
-                                 : (double)o->gemv * (8.0 * (double)h->nrows * (double)n + 8.0 * (double)n + 8.0 * (double)h->nrows);
+                                 : (double)o->gemv * (entry_bytes * (double)h->nrows * (double)n + 8.0 * (double)n + 8.0 * (double)h->nrows);
     result->kernel_launches = launches;
 }
 }  // namespace
@@ -951,6 +986,9 @@ ccqp_status ccqp_debug_solve_emulated(ccqp_handle* const* hs, int world, int sol
         if (!hs[r] || !hs[r]->emulated || hs[r]->world != world || hs[r]->rank != r) return CCQP_ERR_INVALID_ARG;
     ccqp_handle* h0 = hs[0];
     h0->last_error.clear();
+    for (int r = 1; r < world; ++r)
+        if (hs[r]->a_f32 != h0->a_f32) { h0->last_error = "ranks disagree on the matrix type (fp32 / fp64)"; return CCQP_ERR_INVALID_ARG; }
+    if (h0->a_f32 && f32_variant_ctx_bytes() != sizeof(DenseCtx)) { h0->last_error = "dense_f32.cu was built from different headers"; return CCQP_ERR_CUDA; }
     cudaStream_t stream = h0->stream;
     std::vector<DenseCtx> ctxs((size_t)world);
     size_t smem = 0;
@@ -969,7 +1007,8 @@ ccqp_status ccqp_debug_solve_emulated(ccqp_handle* const* hs, int world, int sol
     CU(h0, h0->emu_ctx.ensure(sizeof(DenseCtx) * world));
     CU(h0, cudaMemcpyAsync(h0->emu_ctx.p, ctxs.data(), sizeof(DenseCtx) * world, cudaMemcpyHostToDevice, stream));
     CU(h0, cudaEventRecord(h0->ev0, stream));
-    CU(h0, launch_dense_emu(solver, h0->emu_ctx.as<DenseCtx>(), world, G, smem, stream));
+    CU(h0, h0->a_f32 ? f32_variant_launch_emu(solver, h0->emu_ctx.p, world, G, smem, stream)
+                     : launch_dense_emu(solver, h0->emu_ctx.as<DenseCtx>(), world, G, smem, stream));
     CU(h0, cudaEventRecord(h0->ev1, stream));
     h0->launches += 1;
     std::vector<DenseOut> outs((size_t)world);

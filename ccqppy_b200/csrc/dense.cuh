@@ -18,6 +18,7 @@
 //     functor-based project_pass of proj.cuh.
 //
 // Algorithmic bytes per mat-vec: 8 * n_rows * n (A) + 8 n (v) + 8 n_rows (y)   (SURVEY 8d).
+// fp32 build (CCQP_A_F32, dense_f32.cu): A is stored as fp32 and widened in registers, 4 * n_rows * n for A.
 #pragma once
 #include "proj.cuh"
 
@@ -43,9 +44,22 @@ namespace ccqp {
 #ifndef CCQP_DENSE_ONLY
 #define CCQP_DENSE_ONLY 0     // 1: the CSR mat-vec phase is compiled out (capi.cu: the product's dense kernels carry no CSR code --
 #endif                        //    the register allocation and the schedule of the dense loop depend on everything inlined next to it)
+#ifndef CCQP_A_F32
+#define CCQP_A_F32 0          // 1: the dense Hessian is stored as fp32 and widened to fp64 in registers (dense_f32.cu)
+#endif
+#ifndef CCQP_UNROLL_F32
+#define CCQP_UNROLL_F32 32    // fp32 build: 128-bit loads in flight per lane (32 x 16 bytes = the fp64 loop's 16 x 32)
+#endif
 constexpr int kDenseThreads = CCQP_DENSE_THREADS;
 constexpr int kDenseWarps = kDenseThreads / 32;
 constexpr int kUnroll = CCQP_UNROLL;  // 256-bit loads in flight per lane
+constexpr int kUnrollF32 = CCQP_UNROLL_F32;
+static_assert(kUnrollF32 >= 1 && kUnrollF32 <= 32, "the fp32 loop's remainder chain (16/8/4/2/1) covers at most 31 chunks");
+#if CCQP_A_F32
+using AElem = float;                  // what DenseCtx::A points at
+#else
+using AElem = double;
+#endif
 constexpr int kMaxWindow = 64;        // SPG non-monotone window
 
 enum DenseOp : int {
@@ -62,12 +76,12 @@ struct DenseOut {          // written by CTA 0 / thread 0
 constexpr int kNumVec = 12;
 
 struct DenseCtx {
-    // Hessian row shard
+    // Hessian row shard (fp32 build: A points at floats, read as AElem; lda counts stored entries)
     const double* A;
     long long lda;
     int n;              // columns = unknowns
     int row0, nrows;    // rows [row0, row0+nrows) live on this device
-    int aligned;        // 256-bit path usable (A base and lda*8 multiples of 32 bytes)
+    int aligned;        // vector path usable (fp64: A base and lda*8 multiples of 32 bytes; fp32: base 16-byte aligned, lda % 4 == 0)
     // operator-form Hessian (CSR) instead of the dense rows: csr_val != nullptr
     const long long* csr_ptr;   // [nrows + 1], relative to this shard (csr_ptr[0] = 0)
     const int* csr_idx;         // [nnz] column indices
@@ -257,6 +271,65 @@ __device__ __forceinline__ double dot_seg_generic(const double* __restrict__ aro
         a1 = fma(x1, vs[c + 32], a1);
     }
     if (c < ncol) a0 = fma(ldg_stream(arow + c), vs[c], a0);
+    return a0 + a1;
+}
+
+// fp32 Hessian (dense_f32.cu).  The same lane -> column mapping, FMA chains and reductions as the two loops above, from
+// 128-bit loads of four floats (one chunk of 128 columns = 512 bytes per warp); every entry is widened exactly in a
+// register before its fma, so the result is bit-identical to the fp64 loop on the widened matrix.  kUnrollF32 loads in
+// flight per lane keep the fp64 loop's 512 bytes per lane; chunks are still consumed in order (remainders 16/8/4/2/1).
+// The vector panel is read with explicit ld.shared: with plain loads the compiler hoisted the 32 vector reads of a batch
+// next to the A loads, and APGD / APGD-AR / BBPGD / BBPGDf spilled (72-184 bytes, ptxas -v).
+template <bool kEF, int U>
+__device__ __forceinline__ void dot_chunks(const float* ap, const double* vp, double& a0, double& a1, double& a2, double& a3) {
+    float r[U][4];
+#pragma unroll
+    for (int u = 0; u < U; ++u) ldg128_stream<kEF>(ap + (size_t)u * 128, r[u]);
+    const uint32_t vp32 = smem_u32(vp);
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        double4 v;
+        asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(vp32 + (uint32_t)u * 1024u));
+        asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.z), "=d"(v.w) : "r"(vp32 + (uint32_t)u * 1024u + 16u));
+        a0 = fma((double)r[u][0], v.x, a0);
+        a1 = fma((double)r[u][1], v.y, a1);
+        a2 = fma((double)r[u][2], v.z, a2);
+        a3 = fma((double)r[u][3], v.w, a3);
+    }
+}
+
+template <bool kEF>
+__device__ __forceinline__ double dot_seg_aligned(const float* __restrict__ arow, const double* vs, int ncol, int lane) {
+    double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
+    const int nchunk = ncol >> 7;
+    const float* ap = arow + lane * 4;
+    const double* vp = vs + lane * 4;
+    int c = 0;
+    for (; c + kUnrollF32 <= nchunk; c += kUnrollF32) dot_chunks<kEF, kUnrollF32>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3);
+    if (kUnrollF32 > 16 && c + 16 <= nchunk) { dot_chunks<kEF, 16>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 16; }
+    if (kUnrollF32 > 8 && c + 8 <= nchunk) { dot_chunks<kEF, 8>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 8; }
+    if (kUnrollF32 > 4 && c + 4 <= nchunk) { dot_chunks<kEF, 4>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 4; }
+    if (kUnrollF32 > 2 && c + 2 <= nchunk) { dot_chunks<kEF, 2>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 2; }
+    if (c < nchunk) { dot_chunks<kEF, 1>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 1; }
+    const int col = (nchunk << 7) + lane * 4;
+    if (col < ncol) {
+        a0 = fma((double)ldg_stream(arow + col), vs[col], a0);
+        if (col + 1 < ncol) a1 = fma((double)ldg_stream(arow + col + 1), vs[col + 1], a1);
+        if (col + 2 < ncol) a2 = fma((double)ldg_stream(arow + col + 2), vs[col + 2], a2);
+        if (col + 3 < ncol) a3 = fma((double)ldg_stream(arow + col + 3), vs[col + 3], a3);
+    }
+    return (a0 + a1) + (a2 + a3);
+}
+
+__device__ __forceinline__ double dot_seg_generic(const float* __restrict__ arow, const double* vs, int ncol, int lane) {
+    double a0 = 0.0, a1 = 0.0;
+    int c = lane;
+    for (; c + 32 < ncol; c += 64) {
+        const double x0 = ldg_stream(arow + c), x1 = ldg_stream(arow + c + 32);
+        a0 = fma(x0, vs[c], a0);
+        a1 = fma(x1, vs[c + 32], a1);
+    }
+    if (c < ncol) a0 = fma((double)ldg_stream(arow + c), vs[c], a0);
     return a0 + a1;
 }
 
@@ -549,7 +622,7 @@ __device__ __forceinline__ void gemv_phase(Kst& k, const DenseCtx& c, const doub
             const int row = t / spp, seg = t - row * spp;
             const int col0 = seg * SW;
             const int ncol = min(SW, pc - col0);
-            const double* arow = c.A + (size_t)(k.r0 - c.row0 + row) * c.lda + (size_t)p * CW + col0;
+            const AElem* arow = reinterpret_cast<const AElem*>(c.A) + (size_t)(k.r0 - c.row0 + row) * c.lda + (size_t)p * CW + col0;
             double acc;
             if (c.aligned) acc = t >= t_res ? dot_seg_aligned<true>(arow, vb + col0, ncol, lane)
                                             : dot_seg_aligned<false>(arow, vb + col0, ncol, lane);

@@ -1,6 +1,7 @@
 // Entry points between the translation units of libccqp_b200.so (the kernels are split over several .cu files
 // only so that they compile in parallel): capi.cu (C-ABI, dense kernels), batched.cu (batched kernels),
-// emu.cu (emulated-ranks instantiations of the dense kernels, a test vehicle).
+// emu.cu (emulated-ranks instantiations of the dense kernels, a test vehicle), csr.cu (CSR Hessians),
+// dense_f32.cu (fp32-stored dense Hessians).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -45,5 +46,11 @@ size_t csr_variant_smem();
 int csr_variant_rows_max();
 size_t csr_variant_ctx_bytes();
 cudaError_t csr_variant_launch(int op, const void* ctx, int grid, size_t smem, bool cooperative, cudaStream_t stream);
+
+// dense_f32.cu -- the dense solver kernels compiled for an fp32-stored Hessian (widened in registers); `ctx` points at a
+// DenseCtx (`d_ctxs`: world of them in device memory), `op` is a DenseOp, `solver` a ccqp_solver
+size_t f32_variant_ctx_bytes();
+cudaError_t f32_variant_launch(int op, const void* ctx, int grid, size_t smem, bool cooperative, cudaStream_t stream);
+cudaError_t f32_variant_launch_emu(int solver, const void* d_ctxs, int world, int G, size_t smem, cudaStream_t stream);
 
 }  // namespace ccqp

@@ -16,6 +16,7 @@ import numpy as np
 
 from . import _capi
 from . import solution_spaces as ss
+from .solvers import _as_f32_matrix
 
 NORM_KINDS = (_capi.SPHERE, _capi.CONE_REF, _capi.SOC)
 
@@ -104,7 +105,8 @@ class ShardedResult:
 class ShardedSolver:
     """Binds a solver object (its tolerance / limits / hyper-parameters), one row shard of A and the
     full projection table to this rank's GPU.  `A` is either this rank's rows (`row_range` given)
-    or the full matrix (the shard is sliced out; nothing is copied for a CUDA tensor)."""
+    or the full matrix (the shard is sliced out; nothing is copied for a CUDA tensor).  A float32 A keeps float32
+    shards (`ccqp_set_matrix_f32`), with the bits of the widened matrix's solve."""
 
     def __init__(self, solver, A, convex_proj_op=None, rank=None, world=None, device=None, row_range=None, group=None):
         import torch
@@ -144,11 +146,16 @@ class ShardedSolver:
                 shard = A
             else:
                 shard = A[r0:r1]
-            if not (hasattr(shard, "is_cuda") and shard.is_cuda):
-                shard = torch.as_tensor(np.ascontiguousarray(shard, dtype=np.float64)).to(self.device)
-            self.shard = shard.to(dtype=torch.float64).contiguous()     # keeps the storage alive
-            _capi.check(self.h.h, lib.ccqp_set_matrix(self.h.h, ctypes.c_void_p(self.shard.data_ptr()), n,
-                                                      self.shard.stride(0), r0, r1 - r0, _capi.MEM_DEVICE))
+            A32 = _as_f32_matrix(shard)
+            if A32 is not None:
+                self.shard = A32 if (hasattr(A32, "is_cuda") and A32.is_cuda) else torch.as_tensor(A32).to(self.device)
+                self.h.set_matrix_f32(self.shard, n, r0, r1 - r0)
+            else:
+                if not (hasattr(shard, "is_cuda") and shard.is_cuda):
+                    shard = torch.as_tensor(np.ascontiguousarray(shard, dtype=np.float64)).to(self.device)
+                self.shard = shard.to(dtype=torch.float64).contiguous()     # keeps the storage alive
+                _capi.check(self.h.h, lib.ccqp_set_matrix(self.h.h, ctypes.c_void_p(self.shard.data_ptr()), n,
+                                                          self.shard.stride(0), r0, r1 - r0, _capi.MEM_DEVICE))
         pp, _, _keep = _capi.f64_ptr(params if params.size else np.zeros(1))
         _capi.check(self.h.h, lib.ccqp_set_projection(self.h.h, blocks.ptr, len(blocks), pp, params.size))
         if self.world > 1:
@@ -161,12 +168,17 @@ class ShardedSolver:
     def set_matrix(self, shard):
         """Replace this rank's rows of A.  `shard` is [r1 - r0, n]: a CUDA tensor (borrowed in place) or a
         host array / CPU tensor (copied to the device by the library; pinned memory makes the copy
-        asynchronous).  Every rank must call it before the next solve()."""
+        asynchronous); a float32 shard stays float32.  Every rank must call it before the next solve()."""
         import torch
         r0, r1 = self.ranges[self.rank]
         if tuple(shard.shape) != (r1 - r0, self.n):
             raise ValueError("shard must be %s" % ((r1 - r0, self.n),))
         lib = self.h.lib
+        A32 = _as_f32_matrix(shard)
+        if A32 is not None:
+            self.shard = A32
+            self.h.set_matrix_f32(A32, self.n, r0, r1 - r0)
+            return
         if hasattr(shard, "is_cuda") and shard.is_cuda:
             self.shard = shard.to(dtype=torch.float64).contiguous()
             ptr, lda, mem = self.shard.data_ptr(), self.shard.stride(0), _capi.MEM_DEVICE

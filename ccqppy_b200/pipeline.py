@@ -15,7 +15,8 @@ the solves to them round-robin through `ccqp_solve_async` / `ccqp_solve_wait`:
 
 Every solve is the same computation as `solver.solve(...)` (same kernel, same arguments); only the
 scheduling differs.  Host buffers must stay alive until their result has been collected; pinned
-memory (`torch.Tensor.pin_memory()`) is what makes the copies asynchronous.
+memory (`torch.Tensor.pin_memory()`) is what makes the copies asynchronous.  A float32 A is uploaded as float32
+straight from the caller's buffer (`ccqp_set_matrix_f32`: half the PCIe bytes, the same result bits as its widening).
 """
 import ctypes
 
@@ -23,7 +24,7 @@ import numpy as np
 
 from . import _capi
 from . import solution_spaces as ss
-from .solvers import _as_f64, _is_torch
+from .solvers import _as_f32_matrix, _as_f64, _is_torch
 
 
 class SolveResult:
@@ -98,27 +99,32 @@ class SolvePipeline:
         if slot.ticket is not None:
             self._collect(slot)
         h, lib = slot.handle, slot.handle.lib
-        A64, b64 = _as_f64(A), _as_f64(b)
+        A32 = None if symmetric else _as_f32_matrix(A)
+        Ah = A32 if A32 is not None else _as_f64(A)
+        b64 = _as_f64(b)
         x064 = None if x0 is None else _as_f64(x0)
         uni = None if uniforms is None else _as_f64(uniforms)
-        if any(_is_torch(v) and v.is_cuda for v in (A64, b64, x064, uni) if v is not None):
+        if any(_is_torch(v) and v.is_cuda for v in (Ah, b64, x064, uni) if v is not None):
             raise TypeError("SolvePipeline is for host-resident inputs; device tensors go through solve()")
         blocks, params, _rows = convex_proj_op.descriptor()
         par = params if params.size else np.zeros(1)
         # the (small) projection table first: ccqp_set_projection synchronises the handle's stream, which is idle here
         _capi.check(h.h, lib.ccqp_set_projection(h.h, blocks.ptr, len(blocks), ctypes.c_void_p(par.ctypes.data), params.size))
-        pa, mem, _ = _capi.f64_ptr(A64)
-        lda = A64.stride(0) if _is_torch(A64) else n
-        if symmetric:
-            _capi.check(h.h, lib.ccqp_set_matrix_symmetric(h.h, pa, n, lda, mem))
+        if A32 is not None:
+            h.set_matrix_f32(A32, n)                                                  # asynchronous from pinned memory too
         else:
-            _capi.check(h.h, lib.ccqp_set_matrix(h.h, pa, n, lda, 0, n, mem))  # the copies are asynchronous from pinned memory
+            pa, mem, _ = _capi.f64_ptr(Ah)
+            lda = Ah.stride(0) if _is_torch(Ah) else n
+            if symmetric:
+                _capi.check(h.h, lib.ccqp_set_matrix_symmetric(h.h, pa, n, lda, mem))
+            else:
+                _capi.check(h.h, lib.ccqp_set_matrix(h.h, pa, n, lda, 0, n, mem))  # the copies are asynchronous from pinned memory
         xout = self._pinned(n)
         ptr = lambda v: None if v is None else _capi.f64_ptr(v)[0]
         prm = s._params()
         _capi.check(h.h, lib.ccqp_solve_async(h.h, s._solver_id, ctypes.byref(prm), ptr(b64), ptr(x064), ptr(uni),
                                               0 if uni is None else int(uni.shape[0]), ptr(xout), _capi.MEM_HOST))
-        slot.keep = (A64, b64, x064, uni, blocks, par, prm)
+        slot.keep = (Ah, b64, x064, uni, blocks, par, prm)
         slot.xout = xout
         slot.ticket = self._next
         self._next += 1

@@ -15,7 +15,12 @@ Extensions beyond the reference API (all optional):
   * `solve(..., uniforms=...)`      explicit U[0,1) stream for SPG instead of the global NumPy RNG
   * `solve_batched(A, b, lb, ub)`   many small QPs in one persistent kernel (n <= 128; per-problem boxes or one shared table)
   * `solution_gpu_time`, `solution_hbm_bytes`, `solution_gemv_count` after a solve
-  * A / b / x0 may be torch tensors; a CUDA tensor A is used in place (no copy)
+  * A / b / x0 may be torch tensors; a CUDA tensor A is used in place (no copy) when it is float64, or float32,
+    contiguous and 16-byte aligned
+  * a float32 dense A stays float32 (`ccqp_set_matrix_f32`): the kernels stream it at 4 bytes per entry and widen every
+    entry exactly in a register, which is what NumPy does for the reference's `A.dot(v)` with a float32 A -- the result
+    has the same bits as the solve of `A.astype(np.float64)`, for half the HBM and PCIe bytes and half the device memory.
+    `symmetric=True`, sparse A and `solve_batched` widen a float32 A to float64 as before.
 """
 import ctypes
 import time
@@ -87,6 +92,20 @@ def _as_f64(a, like_device=None):
     return arr
 
 
+def _as_f32_matrix(a):
+    """A float32 dense NumPy array / torch tensor as the C-contiguous float32 array / tensor ccqp_set_matrix_f32 takes
+    (no widening); None for any other input.  A CUDA tensor is used as it is when it is contiguous and 16-byte aligned;
+    otherwise ONE contiguous copy is made, so its rows take the same mat-vec loop as a widened copy of `a` would."""
+    if isinstance(a, np.ndarray):
+        return np.ascontiguousarray(a) if a.dtype == np.float32 else None
+    if not _is_torch(a) or str(a.dtype) != "torch.float32" or str(a.layout) != "torch.strided":
+        return None
+    if a.is_contiguous() and (not a.is_cuda or a.data_ptr() % 16 == 0):
+        return a
+    import torch
+    return a.clone(memory_format=torch.contiguous_format)
+
+
 class CCQPSolverBase(ABC):
     """solvers.py:11-68.  Concrete classes set `_solver_id`, `_label` and `_name`."""
 
@@ -151,7 +170,10 @@ class CCQPSolverBase(ABC):
         A host-resident dense A that is symmetric crosses PCIe as its upper block triangle only (found out by a host-side
         test that runs while the copy engine works; the device copy is bit-identical to a full upload, and any other A is
         uploaded whole -- `ccqp_set_matrix`).  `symmetric=True` (extension) declares the symmetry instead: no test, the
-        blocks below the block diagonal of A are never read (`ccqp_set_matrix_symmetric`)."""
+        blocks below the block diagonal of A are never read (`ccqp_set_matrix_symmetric`).
+
+        A float32 dense A (NumPy array, host or CUDA tensor; `symmetric=False`) is neither widened nor copied on the device
+        (`ccqp_set_matrix_f32`): the solution, residual and counts are bit-identical to those of `A.astype(np.float64)`."""
         num_unknowns = b.shape[0]
         if convex_proj_op is None:
             convex_proj_op = ss.IdentityProjOp(num_unknowns)
@@ -168,12 +190,14 @@ class CCQPSolverBase(ABC):
         dev = A.device if on_device else None
         if on_device:
             device = A.device.index if A.device.index is not None else -1
-        A64 = None if sparse else _as_f64(A)
+        A32 = None if (sparse or symmetric) else _as_f32_matrix(A)
+        A64 = None if (sparse or A32 is not None) else _as_f64(A)
+        Ad = A32 if A32 is not None else A64
         # the vectors live where A lives (or where b lives, if only b is a CUDA tensor)
         vec_dev = dev if on_device else (b.device if (_is_torch(b) and b.is_cuda) else None)
         b64 = _as_f64(b, vec_dev)
         x064 = None if x0 is None else _as_f64(x0, vec_dev)
-        if tuple(A.shape if sparse else A64.shape) != (num_unknowns, num_unknowns):
+        if tuple(A.shape if sparse else Ad.shape) != (num_unknowns, num_unknowns):
             raise ValueError("A must be (n, n) with n = b.shape[0]")
 
         h = _capi.default_handle(device)
@@ -184,6 +208,8 @@ class CCQPSolverBase(ABC):
                 _capi.check(h.h, lib.ccqp_set_stream(h.h, ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
         if sparse:
             _ka = _set_sparse_matrix(h, A, num_unknowns)
+        elif A32 is not None:
+            h.set_matrix_f32(A32, num_unknowns)      # a host A is copied on the handle's stream before the solve's own copies
         else:
             pa, mem_a, _ka = _capi.f64_ptr(A64)
             lda = A64.stride(0) if _is_torch(A64) else num_unknowns

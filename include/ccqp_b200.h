@@ -12,7 +12,8 @@
  *     ccqp_status; ccqp_status_string() gives text.
  *   - Every data pointer is either a HOST or a DEVICE pointer, named by a ccqp_memtype argument.
  *     Host buffers are copied by the library (pinned host memory gives asynchronous copies).
- *   - All reals are IEEE fp64.  Matrices are row-major (C order) with leading dimension lda.
+ *   - All reals are IEEE fp64 (a dense Hessian may be stored as fp32: ccqp_set_matrix_f32).  Matrices are row-major
+ *     (C order) with leading dimension lda.
  *   - One handle per host thread; a handle owns one CUDA device, one stream and its workspaces.
  *   - There is no CPU fallback: with no usable device ccqp_create() fails with
  *     CCQP_ERR_NO_DEVICE.
@@ -99,7 +100,8 @@ typedef struct ccqp_params {
 typedef struct ccqp_result {
     double residual;       /* solution_residual (NaN where the reference would raise NameError) */
     double gpu_seconds;    /* device time of the solve, CUDA events on the handle's stream       */
-    double hbm_bytes;      /* algorithmic bytes moved: gemv_count * (8 n_rows n + 16 n)          */
+    double hbm_bytes;      /* algorithmic bytes moved: gemv_count * (8 n_rows n + 8 n + 8 n_rows);
+                              an fp32 Hessian (ccqp_set_matrix_f32): gemv_count * (4 n_rows n + 8 n + 8 n_rows) */
     int64_t mv_count;      /* solution_num_matrix_vector_multiplications (the REPORTED count)    */
     int64_t gemv_count;    /* mat-vec products actually executed on the device                   */
     int64_t iterations;    /* outer iterations completed                                         */
@@ -157,6 +159,17 @@ ccqp_status ccqp_set_matrix_symmetric(ccqp_handle* h, const double* A, int64_t n
  * process may run on. */
 int32_t ccqp_host_matrix_is_block_symmetric(const double* A, int64_t n, int64_t lda, int32_t threads);
 int32_t ccqp_upload_block_rows(void);
+
+/* ccqp_set_matrix() for a Hessian STORED as IEEE fp32 (lda counted in floats).  The arithmetic stays fp64: every entry is
+ * widened exactly in a register in front of its fma, which is what NumPy does for the reference's A.dot(v) with a float32 A
+ * (solvers.py:133), and the mat-vec keeps the fp64 kernels' summation order -- a solve returns the same bits as the fp64
+ * solve of the widened matrix (same lda parity: rows with 16-byte aligned starts and lda % 4 == 0 take the vector loop,
+ * like 32-byte aligned fp64 rows; others the scalar loop).  A DEVICE matrix is borrowed, neither copied nor widened; a
+ * HOST matrix is copied into padded fp32 rows (asynchronous from pinned memory, same lifetime rule as ccqp_set_matrix).
+ * Half the HBM bytes per mat-vec (result.hbm_bytes counts 4 per entry), half the PCIe bytes of an upload
+ * (ccqp_get_upload_info: 4 * n_rows * n, never mirrored).  Replaces any previous matrix of the handle. */
+ccqp_status ccqp_set_matrix_f32(ccqp_handle* h, const float* A, int64_t n, int64_t lda, int64_t row_begin, int64_t n_rows,
+                                int memtype);
 
 /* Operator-form Hessian in CSR.  The reference accepts any `A` with a .dot (solvers.py:133), in particular
  * scipy.sparse matrices (contact-style Hessians D^T M^-1 D are sparse); this is that case.  indptr has
