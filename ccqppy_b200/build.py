@@ -9,8 +9,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libccqp_b200.so")
-SOURCES = ["capi.cu", "batched.cu", "batched_sym.cu", "upload.cu", "emu.cu", "csr.cu", "dense_f32.cu"]      # separate translation units only so that they compile in parallel
-HEADERS = ["common.cuh", "proj.cuh", "dense.cuh", "batched.cuh", "microbench.cuh", "internal.h", "symcheck.h",
+SOURCES = ["capi.cu", "dense_f64.cu", "batched.cu", "batched_sym.cu", "upload.cu", "emu.cu", "csr.cu", "dense_f32.cu"]      # see csrc/internal.h
+HEADERS = ["common.cuh", "proj.cuh", "dense.cuh", "kernel_build.cuh", "batched.cuh", "microbench.cuh", "internal.h", "symcheck.h",
            os.path.join("..", "..", "include", "ccqp_b200.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -759,7 +759,7 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
                     const int row = row0 + (r ^ key);
                     if (row < n && col0 + j < n) {
                         double v[4];
-                        ldg256_stream<false>(Ap + (size_t)row * n + col0 + j, v);
+                        ldg_vec4_stream<false>(Ap + (size_t)row * n + col0 + j, v);
                         a[r][j] = v[0]; a[r][j + 1] = v[1]; a[r][j + 2] = v[2]; a[r][j + 3] = v[3];
                     } else { a[r][j] = 0.0; a[r][j + 1] = 0.0; a[r][j + 2] = 0.0; a[r][j + 3] = 0.0; }
                 }

@@ -13,8 +13,7 @@
 #include <string>
 #include <vector>
 
-#define CCQP_DENSE_ONLY 1      // CSR Hessians run csr.cu's build of the kernels (emulated ranks: emu.cu's), fp32 Hessians dense_f32.cu's
-#include "dense.cuh"
+#include "dense.cuh"        // DenseCtx, DenseOut and the tiling constants; the kernels are launched through KernelBuild (internal.h)
 #include "internal.h"
 #include "microbench.cuh"
 
@@ -42,8 +41,8 @@ struct ccqp_handle {
     bool own_stream = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::string last_error;
-    // matrix shard (a_f32: dA points at floats, lda counts floats -- ccqp_set_matrix_f32)
-    const double* dA = nullptr;
+    // matrix shard: doubles, or floats when a_f32 (ccqp_set_matrix_f32); lda counts entries
+    const void* dA = nullptr;
     bool a_f32 = false;
     DevBuf a_own;
     // operator-form (CSR) alternative to dA
@@ -79,8 +78,8 @@ struct ccqp_handle {
     bool emulated = false;          // rank of an emulated box (ccqp_debug_emulate_ranks): peers live on the same device
     DevBuf emu_ctx;                 // rank 0 of an emulated box: the ranks' kernel contexts
     // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-DEVICE attribute of each kernel instantiation: one bit per
-    // instantiation, kept per handle (a handle owns exactly one device)
-    unsigned smem_attr_mask = 0;
+    // instantiation (smem_bit), one mask per KernelBuild, kept per handle (a handle owns exactly one device)
+    unsigned smem_attr_mask[kNumBuilds] = {};
 };
 
 namespace {
@@ -150,6 +149,35 @@ ccqp_status ensure_work(ccqp_handle* h) {
 
 struct Tiling { int grid, CW, SW, np, nseg, rows_max, accum; size_t smem; };
 
+// The compilation of the solver kernels that runs a handle's launches (the only place that knows the rule).  The ranks
+// of an emulated box run in one launch of dense_kernel_emu: emu.cu's (fp64, dense and CSR phase at the product's CTA
+// width) or dense_f32.cu's.
+const KernelBuild& build_for(const ccqp_handle* h) {
+    if (h->emulated) return h->a_f32 ? kBuildF32 : kBuildEmu;
+    return h->d_val ? kBuildCsr : h->a_f32 ? kBuildF32 : kBuildF64;
+}
+
+// The kernels take DenseCtx as plain bytes: a build that sees another DenseCtx must not be launched
+static_assert(sizeof(DenseCtx) % 8 == 0, "DenseCtx");
+bool same_headers(ccqp_handle* h, const KernelBuild& b) {
+    if (b.ctx_bytes == sizeof(DenseCtx)) return true;
+    h->last_error = std::string(b.unit) + " was built from different headers";
+    return false;
+}
+
+// the bit of a kernel in smem_attr_mask[build]: dense_kernel<op> (OP_PROJGRAD -> bit 10), dense_kernel_emu<solver> from bit 16
+constexpr unsigned smem_bit(int op) { return 1u << (op < 100 ? op : 7 + (op - 100)); }
+constexpr unsigned emu_smem_bit(int solver) { return 1u << (16 + solver); }
+
+// the hooks that never touch the matrix (projection-only use): one row per CTA, one 128-column panel
+Tiling projection_tiling(const ccqp_handle* h) {
+    Tiling t;
+    t.grid = (int)std::max<long long>(1, std::min<long long>(h->sm_count, h->n));
+    t.CW = 128; t.SW = 128; t.np = 1; t.nseg = 1; t.rows_max = 1; t.accum = 0;
+    t.smem = dense_smem_bytes(128, 1, 1);
+    return t;
+}
+
 // Tuning overrides from the environment are accepted only when they are usable (a bad value is ignored, not obeyed)
 int env_int(const char* name, int fallback, bool (*ok)(int)) {
     const char* e = getenv(name);
@@ -184,11 +212,9 @@ Tiling choose_tiling(const ccqp_handle* h) {
     t.grid = (int)std::max(1LL, std::min<long long>(std::min<long long>(h->sm_count, rows_ref), std::max(1LL, work)));
     t.accum = 0;
     if (h->d_val) {     // CSR: the two panel buffers together are the ring of TMA stages of the entry stream
-        t.CW = kCsrCW; t.SW = kCsrCW; t.np = 1; t.nseg = 1; t.rows_max = kCsrRowsMax;   // (the psum region holds the row-pointer windows)
+        // (the psum region holds the row-pointer windows, whose size follows the CTA width of the build that runs them)
+        t.CW = kCsrCW; t.SW = kCsrCW; t.np = 1; t.nseg = 1; t.rows_max = build_for(h).csr_rows_max;
         t.smem = dense_smem_bytes(t.CW, t.rows_max, t.nseg);
-        // single-GPU and sharded solves run the many-warps build of the kernels (csr.cu), whose windows are larger;
-        // emulated ranks run this file's build (emu.cu), see launch_dense
-        if (!h->emulated) { t.rows_max = csr_variant_rows_max(); t.smem = csr_variant_smem(); }
         return t;
     }
     t.rows_max = (int)((nrows + t.grid - 1) / t.grid) + 1;
@@ -234,7 +260,7 @@ void fill_ctx(ccqp_handle* h, DenseCtx& c, const Tiling& t) {
         const double mean = h->d_val ? (double)h->nnz / (double)std::max<long long>(h->nrows, 1) : 0.0;
         // lanes that sum one row out of the shared-memory products: about 8-16 entries per lane
         // (a tile of 4096 entries should hold about as many rows as there are groups: one pass over the rows)
-        const double per_tile = (h->emulated ? kDenseThreads : csr_variant_threads()) * mean / kCsrTile;   // lanes per row of a tile
+        const double per_tile = build_for(h).threads * mean / kCsrTile;   // lanes per row of a tile
         c.csr_group = per_tile >= 32 ? 32 : per_tile >= 16 ? 16 : per_tile >= 8 ? 8 : per_tile >= 4 ? 4 : per_tile >= 2 ? 2 : 1;
         c.csr_group = env_int("CCQP_CSR_GROUP", c.csr_group, ok_csr_group);
         c.csr_l1 = env_int("CCQP_CSR_L1", 1, ok_bool);
@@ -277,8 +303,6 @@ void fill_ctx(ccqp_handle* h, DenseCtx& c, const Tiling& t) {
     }
 }
 
-constexpr int op_slot(int op) { return op < 100 ? op : 7 + (op - 100); }   // OP_PROJGRAD -> bit 10
-
 // the device copy of a symmetric host matrix is completed by its first user (upload.cu)
 ccqp_status finish_matrix(ccqp_handle* h) {
     if (h->mirror_pending) {
@@ -289,59 +313,33 @@ ccqp_status finish_matrix(ccqp_handle* h) {
     return CCQP_OK;
 }
 
-template <int OP>
-ccqp_status launch_dense(ccqp_handle* h, DenseCtx& c, const Tiling& t, bool cooperative) {
+ccqp_status launch_dense(ccqp_handle* h, int op, DenseCtx& c, const Tiling& t, bool cooperative) {
     if (ccqp_status fs = finish_matrix(h)) return fs;
     if (t.smem > kDenseSmemLimit) {
         h->last_error = "dense tiling needs more shared memory than one SM has";
         return CCQP_ERR_UNSUPPORTED;
     }
-    if (!(h->smem_attr_mask & (1u << op_slot(OP)))) {
-        CU(h, cudaFuncSetAttribute(dense_kernel<OP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDenseSmemLimit));
-        h->smem_attr_mask |= 1u << op_slot(OP);
+    const KernelBuild* b = &build_for(h);
+    if (!b->launch) {       // emu.cu has no dense_kernel: the hooks of an emulated fp64 rank run the product's build, which has no CSR phase
+        if (c.csr_val) {
+            h->last_error = "the unit-test hooks of an emulated rank do not take a CSR matrix";
+            return CCQP_ERR_UNSUPPORTED;
+        }
+        b = &kBuildF64;
     }
+    if (!same_headers(h, *b)) return CCQP_ERR_CUDA;
     if (cooperative) CU(h, cudaMemsetAsync(h->flags.p, 0, kSyncBytes, h->stream));   // barrier counters
-    if (c.csr_val && h->emulated) {
-        h->last_error = "the unit-test hooks of an emulated rank do not take a CSR matrix";
-        return CCQP_ERR_UNSUPPORTED;
-    }
-    if (c.csr_val) {        // operator-form Hessian: the many-warps build of the same kernels (csr.cu)
-        static_assert(sizeof(DenseCtx) % 8 == 0, "DenseCtx");
-        if (csr_variant_ctx_bytes() != sizeof(DenseCtx)) { h->last_error = "csr.cu was built from different headers"; return CCQP_ERR_CUDA; }
-        CU(h, csr_variant_launch(OP, &c, t.grid, t.smem, cooperative, h->stream));
-        h->launches += 1;
-        return CCQP_OK;
-    }
-    if (h->a_f32) {         // fp32-stored Hessian: the build of the same kernels that widens A in registers (dense_f32.cu)
-        if (f32_variant_ctx_bytes() != sizeof(DenseCtx)) { h->last_error = "dense_f32.cu was built from different headers"; return CCQP_ERR_CUDA; }
-        CU(h, f32_variant_launch(OP, &c, t.grid, t.smem, cooperative, h->stream));
-        h->launches += 1;
-        return CCQP_OK;
-    }
-    void* args[] = {&c};
-    if (cooperative)
-        CU(h, cudaLaunchCooperativeKernel((const void*)dense_kernel<OP>, dim3(t.grid), dim3(kDenseThreads), args, t.smem, h->stream));
-    else
-        CU(h, cudaLaunchKernel((const void*)dense_kernel<OP>, dim3(t.grid), dim3(kDenseThreads), args, t.smem, h->stream));
+    unsigned& mask = h->smem_attr_mask[b->index];
+    CU(h, b->launch(op, &c, t.grid, t.smem, cooperative, !(mask & smem_bit(op)), h->stream));
+    mask |= smem_bit(op);
     h->launches += 1;
     return CCQP_OK;
 }
 
 ccqp_status launch_by_solver(ccqp_handle* h, int solver, DenseCtx& c, const Tiling& t) {
-#ifdef CCQP_SWEEP_BUILD
-    return CCQP_ERR_UNSUPPORTED;   // tuning build: only the mat-vec hook is compiled
-#else
-    switch (solver) {
-        case CCQP_SOLVER_PGD: return launch_dense<OP_PGD>(h, c, t, true);
-        case CCQP_SOLVER_APGD: return launch_dense<OP_APGD>(h, c, t, true);
-        case CCQP_SOLVER_APGD_AR: return launch_dense<OP_APGD_AR>(h, c, t, true);
-        case CCQP_SOLVER_BBPGD: return launch_dense<OP_BBPGD>(h, c, t, true);
-        case CCQP_SOLVER_BBPGDF: return launch_dense<OP_BBPGDF>(h, c, t, true);
-        case CCQP_SOLVER_SPG: return launch_dense<OP_SPG>(h, c, t, true);
-        case CCQP_SOLVER_MPRGP: return launch_dense<OP_MPRGP>(h, c, t, true);
-    }
-    return CCQP_ERR_INVALID_ARG;
-#endif
+    constexpr int kSolverOp[] = {OP_PGD, OP_APGD, OP_APGD_AR, OP_BBPGD, OP_BBPGDF, OP_SPG, OP_MPRGP};   // by ccqp_solver
+    if (solver < CCQP_SOLVER_PGD || solver > CCQP_SOLVER_MPRGP) return CCQP_ERR_INVALID_ARG;
+    return launch_dense(h, kSolverOp[solver], c, t, true);
 }
 
 bool params_ok(const ccqp_params* p, int solver) {
@@ -427,44 +425,10 @@ ccqp_status ccqp_get_info(const ccqp_handle* h, int32_t* sm_count, int32_t* dens
     return CCQP_OK;
 }
 
-static ccqp_status set_matrix_dense(ccqp_handle* h, const double* A, int64_t n, int64_t lda, int64_t row_begin, int64_t n_rows,
-                                    int memtype, bool declared_symmetric) {
-    if (!h || !A || n <= 0 || n >= (1LL << 31) - 256 || lda < n || row_begin < 0 || n_rows <= 0 || row_begin + n_rows > n)
-        return CCQP_ERR_INVALID_ARG;
-    CU(h, cudaSetDevice(h->device));
-    h->n = n; h->row0 = row_begin; h->nrows = n_rows;
-    h->d_ptr = nullptr; h->d_idx = nullptr; h->d_val = nullptr; h->nnz = 0;
-    h->mirror_pending = false; h->a_f32 = false;
-    if (memtype == CCQP_MEM_DEVICE) {
-        h->dA = A; h->lda = lda;
-        h->upload_mirrored = false; h->upload_bytes = 0;
-    } else {
-        const long long ldd = round_up(n, 4);   // keep rows 32-byte aligned for the 256-bit loads
-        CU(h, h->a_own.ensure((size_t)n_rows * ldd * 8 + 64));
-        if (row_begin == 0 && n_rows == n) {    // a whole matrix: half of the PCIe traffic if it turns out to be symmetric (upload.cu)
-            CU(h, upload_square_matrix(h->stream, h->a_own.as<double>(), ldd, A, n, lda, declared_symmetric, &h->upload_mirrored, &h->upload_bytes));
-            h->mirror_pending = h->upload_mirrored;
-        } else {
-            CU(h, cudaMemcpy2DAsync(h->a_own.p, (size_t)ldd * 8, A, (size_t)lda * 8, (size_t)n * 8, (size_t)n_rows,
-                                    cudaMemcpyHostToDevice, h->stream));
-            h->upload_mirrored = false; h->upload_bytes = n_rows * n * 8;
-        }
-        h->dA = h->a_own.as<double>(); h->lda = ldd;
-    }
-    return CCQP_OK;
-}
-
-ccqp_status ccqp_set_matrix(ccqp_handle* h, const double* A, int64_t n, int64_t lda, int64_t row_begin, int64_t n_rows,
-                            int memtype) {
-    return set_matrix_dense(h, A, n, lda, row_begin, n_rows, memtype, false);
-}
-
-ccqp_status ccqp_set_matrix_symmetric(ccqp_handle* h, const double* A, int64_t n, int64_t lda, int memtype) {
-    return set_matrix_dense(h, A, n, lda, 0, n, memtype, true);
-}
-
-ccqp_status ccqp_set_matrix_f32(ccqp_handle* h, const float* A, int64_t n, int64_t lda, int64_t row_begin, int64_t n_rows,
-                                int memtype) {
+// A dense shard of `elem`-byte entries (8: fp64, 4: fp32), borrowed in place from device memory or copied from the host
+// into rows padded to a multiple of 4 entries (32- / 16-byte aligned rows for the 256- / 128-bit loads)
+static ccqp_status set_matrix_dense(ccqp_handle* h, const void* A, int elem, int64_t n, int64_t lda, int64_t row_begin,
+                                    int64_t n_rows, int memtype, bool declared_symmetric) {
     if (!h || !A || n <= 0 || n >= (1LL << 31) - 256 || lda < n || row_begin < 0 || n_rows <= 0 || row_begin + n_rows > n)
         return CCQP_ERR_INVALID_ARG;
     CU(h, cudaSetDevice(h->device));
@@ -472,18 +436,38 @@ ccqp_status ccqp_set_matrix_f32(ccqp_handle* h, const float* A, int64_t n, int64
     h->d_ptr = nullptr; h->d_idx = nullptr; h->d_val = nullptr; h->nnz = 0;
     h->mirror_pending = false; h->upload_mirrored = false;
     if (memtype == CCQP_MEM_DEVICE) {
-        h->dA = reinterpret_cast<const double*>(A); h->lda = lda;
+        h->dA = A; h->lda = lda;
         h->upload_bytes = 0;
     } else {
-        const long long ldd = round_up(n, 4);   // keep rows 16-byte aligned for the 128-bit loads
-        CU(h, h->a_own.ensure((size_t)n_rows * ldd * 4 + 64));
-        CU(h, cudaMemcpy2DAsync(h->a_own.p, (size_t)ldd * 4, A, (size_t)lda * 4, (size_t)n * 4, (size_t)n_rows,
-                                cudaMemcpyHostToDevice, h->stream));
-        h->upload_bytes = n_rows * n * 4;
-        h->dA = h->a_own.as<double>(); h->lda = ldd;
+        const long long ldd = round_up(n, 4);
+        CU(h, h->a_own.ensure((size_t)n_rows * ldd * elem + 64));
+        if (elem == 8 && row_begin == 0 && n_rows == n) {    // a whole fp64 matrix: half of the PCIe traffic if it turns out to be symmetric (upload.cu)
+            CU(h, upload_square_matrix(h->stream, h->a_own.as<double>(), ldd, static_cast<const double*>(A), n, lda, declared_symmetric,
+                                       &h->upload_mirrored, &h->upload_bytes));
+            h->mirror_pending = h->upload_mirrored;
+        } else {
+            CU(h, cudaMemcpy2DAsync(h->a_own.p, (size_t)ldd * elem, A, (size_t)lda * elem, (size_t)n * elem, (size_t)n_rows,
+                                    cudaMemcpyHostToDevice, h->stream));
+            h->upload_bytes = n_rows * n * elem;
+        }
+        h->dA = h->a_own.p; h->lda = ldd;
     }
-    h->a_f32 = true;
+    h->a_f32 = elem == 4;
     return CCQP_OK;
+}
+
+ccqp_status ccqp_set_matrix(ccqp_handle* h, const double* A, int64_t n, int64_t lda, int64_t row_begin, int64_t n_rows,
+                            int memtype) {
+    return set_matrix_dense(h, A, 8, n, lda, row_begin, n_rows, memtype, false);
+}
+
+ccqp_status ccqp_set_matrix_symmetric(ccqp_handle* h, const double* A, int64_t n, int64_t lda, int memtype) {
+    return set_matrix_dense(h, A, 8, n, lda, 0, n, memtype, true);
+}
+
+ccqp_status ccqp_set_matrix_f32(ccqp_handle* h, const float* A, int64_t n, int64_t lda, int64_t row_begin, int64_t n_rows,
+                                int memtype) {
+    return set_matrix_dense(h, A, 4, n, lda, row_begin, n_rows, memtype, false);
 }
 
 ccqp_status ccqp_get_upload_info(ccqp_handle* h, int64_t* bytes, int32_t* mirrored) {
@@ -757,15 +741,10 @@ static ccqp_status run_hook(ccqp_handle* h, int op, const double* in, double* ou
     double* w = reinterpret_cast<double*>(h->work.as<char>() + kSymVecOff);
     CU(h, cudaMemsetAsync(w + W_HIN * npad, 0, (size_t)2 * npad * 8, h->stream));
     if ((st = copy_in(h, w + W_HIN * npad, in, n_in, memtype)) != CCQP_OK) return st;
-    Tiling t;
-    if (h->have_matrix()) t = choose_tiling(h);
-    else { t.grid = (int)std::max<long long>(1, std::min<long long>(h->sm_count, h->n)); t.CW = 128; t.SW = 128; t.np = 1; t.nseg = 1; t.rows_max = 1; t.accum = 0; t.smem = dense_smem_bytes(128, 1, 1); }
+    const Tiling t = h->have_matrix() ? choose_tiling(h) : projection_tiling(h);
     DenseCtx c;
     fill_ctx(h, c, t);
-    if (op == OP_GEMV) st = launch_dense<OP_GEMV>(h, c, t, false);
-    else if (op == OP_PROJECT) st = launch_dense<OP_PROJECT>(h, c, t, false);
-    else st = launch_dense<OP_NORMAL>(h, c, t, false);
-    if (st != CCQP_OK) return st;
+    if ((st = launch_dense(h, op, c, t, false)) != CCQP_OK) return st;
     if ((st = copy_out(h, out, c.hook_out, n_out, memtype)) != CCQP_OK) return st;
     CU(h, cudaStreamSynchronize(h->stream));
     return CCQP_OK;
@@ -785,10 +764,10 @@ ccqp_status ccqp_gemv_timed(ccqp_handle* h, const double* v_dev, double* y_dev, 
     DenseCtx c;
     fill_ctx(h, c, t);
     c.hook_in = v_dev; c.hook_out = y_dev;
-    if ((st = launch_dense<OP_GEMV>(h, c, t, false)) != CCQP_OK) return st;   // warm-up
+    if ((st = launch_dense(h, OP_GEMV, c, t, false)) != CCQP_OK) return st;   // warm-up
     CU(h, cudaEventRecord(h->ev0, h->stream));
     for (int i = 0; i < repeats; ++i)
-        if ((st = launch_dense<OP_GEMV>(h, c, t, false)) != CCQP_OK) return st;
+        if ((st = launch_dense(h, OP_GEMV, c, t, false)) != CCQP_OK) return st;
     CU(h, cudaEventRecord(h->ev1, h->stream));
     CU(h, cudaStreamSynchronize(h->stream));
     float ms = 0.f;
@@ -823,14 +802,12 @@ ccqp_status ccqp_projected_gradient(ccqp_handle* h, const double* x, const doubl
     CU(h, cudaMemsetAsync(w + W_VEC0 * npad, 0, (size_t)3 * npad * 8, h->stream));
     if ((st = copy_in(h, w + W_HIN * npad, x, n, memtype)) != CCQP_OK) return st;
     if ((st = copy_in(h, w + W_VEC0 * npad, g, n, memtype)) != CCQP_OK) return st;
-    Tiling t;
-    t.grid = (int)std::max<long long>(1, std::min<long long>(h->sm_count, n)); t.CW = 128; t.SW = 128; t.np = 1; t.nseg = 1; t.rows_max = 1;
-    t.accum = 0; t.smem = dense_smem_bytes(128, 1, 1);
+    const Tiling t = projection_tiling(h);
     DenseCtx c;
     fill_ctx(h, c, t);
     c.csr_val = nullptr;              // the hooks never touch the matrix
-    if ((st = launch_dense<OP_NORMAL>(h, c, t, false)) != CCQP_OK) return st;
-    if ((st = launch_dense<OP_PROJGRAD>(h, c, t, false)) != CCQP_OK) return st;
+    if ((st = launch_dense(h, OP_NORMAL, c, t, false)) != CCQP_OK) return st;
+    if ((st = launch_dense(h, OP_PROJGRAD, c, t, false)) != CCQP_OK) return st;
     if ((st = copy_out(h, free_out, c.vec[1], n, memtype)) != CCQP_OK) return st;
     if ((st = copy_out(h, chopped_out, c.vec[2], n, memtype)) != CCQP_OK) return st;
     CU(h, cudaStreamSynchronize(h->stream));
@@ -988,7 +965,8 @@ ccqp_status ccqp_debug_solve_emulated(ccqp_handle* const* hs, int world, int sol
     h0->last_error.clear();
     for (int r = 1; r < world; ++r)
         if (hs[r]->a_f32 != h0->a_f32) { h0->last_error = "ranks disagree on the matrix type (fp32 / fp64)"; return CCQP_ERR_INVALID_ARG; }
-    if (h0->a_f32 && f32_variant_ctx_bytes() != sizeof(DenseCtx)) { h0->last_error = "dense_f32.cu was built from different headers"; return CCQP_ERR_CUDA; }
+    const KernelBuild& build = build_for(h0);
+    if (!same_headers(h0, build)) return CCQP_ERR_CUDA;
     cudaStream_t stream = h0->stream;
     std::vector<DenseCtx> ctxs((size_t)world);
     size_t smem = 0;
@@ -1007,8 +985,9 @@ ccqp_status ccqp_debug_solve_emulated(ccqp_handle* const* hs, int world, int sol
     CU(h0, h0->emu_ctx.ensure(sizeof(DenseCtx) * world));
     CU(h0, cudaMemcpyAsync(h0->emu_ctx.p, ctxs.data(), sizeof(DenseCtx) * world, cudaMemcpyHostToDevice, stream));
     CU(h0, cudaEventRecord(h0->ev0, stream));
-    CU(h0, h0->a_f32 ? f32_variant_launch_emu(solver, h0->emu_ctx.p, world, G, smem, stream)
-                     : launch_dense_emu(solver, h0->emu_ctx.as<DenseCtx>(), world, G, smem, stream));
+    unsigned& mask = h0->smem_attr_mask[build.index];
+    CU(h0, build.launch_emu(solver, h0->emu_ctx.p, world, G, smem, !(mask & emu_smem_bit(solver)), stream));
+    mask |= emu_smem_bit(solver);
     CU(h0, cudaEventRecord(h0->ev1, stream));
     h0->launches += 1;
     std::vector<DenseOut> outs((size_t)world);

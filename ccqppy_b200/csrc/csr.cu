@@ -8,55 +8,17 @@
 // the dense mat-vec loop compiled out (CCQP_CSR_ONLY) --
 // inside their own namespace: every `ccqp::` entity of the headers becomes `ccqp_csr::` in this file, so the two
 // compilations of the templates cannot collide.  capi.cu routes every launch of a handle that holds a CSR matrix
-// through csr_variant_launch(); the context struct is the same plain-data struct in both namespaces.
+// through kBuildCsr; the context struct is the same plain-data struct in every namespace.
 #ifndef CCQP_CSR_THREADS
 #define CCQP_CSR_THREADS 512
 #endif
+#undef CCQP_DENSE_THREADS          // the width of the dense builds (-D, tools/sweep_gemv.py) does not apply here
 #define CCQP_DENSE_THREADS CCQP_CSR_THREADS
 #define CCQP_CSR_ONLY 1
 #define ccqp ccqp_csr
 #include "dense.cuh"
+#include "kernel_build.cuh"
 #undef ccqp
 #include "internal.h"
 
-namespace ccqp_csr {
-
-template <int OP>
-static cudaError_t launch(const DenseCtx& c, int grid, size_t smem, bool cooperative, cudaStream_t stream) {
-    cudaError_t e = cudaFuncSetAttribute(dense_kernel<OP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDenseSmemLimit);
-    if (e != cudaSuccess) return e;
-    DenseCtx cc = c;
-    void* args[] = {&cc};
-    if (cooperative) return cudaLaunchCooperativeKernel((const void*)dense_kernel<OP>, dim3(grid), dim3(kDenseThreads), args, smem, stream);
-    return cudaLaunchKernel((const void*)dense_kernel<OP>, dim3(grid), dim3(kDenseThreads), args, smem, stream);
-}
-
-}  // namespace ccqp_csr
-
-namespace ccqp {
-
-int csr_variant_threads() { return ccqp_csr::kDenseThreads; }
-size_t csr_variant_smem() { return ccqp_csr::dense_smem_bytes(ccqp_csr::kCsrCW, ccqp_csr::kCsrRowsMax, 1); }
-int csr_variant_rows_max() { return ccqp_csr::kCsrRowsMax; }
-size_t csr_variant_ctx_bytes() { return sizeof(ccqp_csr::DenseCtx); }
-
-cudaError_t csr_variant_launch(int op, const void* ctx, int grid, size_t smem, bool cooperative, cudaStream_t stream) {
-    const ccqp_csr::DenseCtx& c = *static_cast<const ccqp_csr::DenseCtx*>(ctx);
-    using namespace ccqp_csr;
-    switch (op) {
-        case OP_PGD: return launch<OP_PGD>(c, grid, smem, cooperative, stream);
-        case OP_APGD: return launch<OP_APGD>(c, grid, smem, cooperative, stream);
-        case OP_APGD_AR: return launch<OP_APGD_AR>(c, grid, smem, cooperative, stream);
-        case OP_BBPGD: return launch<OP_BBPGD>(c, grid, smem, cooperative, stream);
-        case OP_BBPGDF: return launch<OP_BBPGDF>(c, grid, smem, cooperative, stream);
-        case OP_SPG: return launch<OP_SPG>(c, grid, smem, cooperative, stream);
-        case OP_MPRGP: return launch<OP_MPRGP>(c, grid, smem, cooperative, stream);
-        case OP_GEMV: return launch<OP_GEMV>(c, grid, smem, cooperative, stream);
-        case OP_PROJECT: return launch<OP_PROJECT>(c, grid, smem, cooperative, stream);
-        case OP_NORMAL: return launch<OP_NORMAL>(c, grid, smem, cooperative, stream);
-        case OP_PROJGRAD: return launch<OP_PROJGRAD>(c, grid, smem, cooperative, stream);
-    }
-    return cudaErrorInvalidValue;
-}
-
-}  // namespace ccqp
+const ccqp::KernelBuild ccqp::kBuildCsr = ccqp_csr::describe<ccqp::KernelBuild>("csr.cu", 2);

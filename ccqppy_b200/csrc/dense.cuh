@@ -42,7 +42,7 @@ namespace ccqp {
 #define CCQP_CSR_ONLY 0       // 1: the dense mat-vec loop is compiled out (csr.cu: the many-warps build of the solver programs)
 #endif
 #ifndef CCQP_DENSE_ONLY
-#define CCQP_DENSE_ONLY 0     // 1: the CSR mat-vec phase is compiled out (capi.cu: the product's dense kernels carry no CSR code --
+#define CCQP_DENSE_ONLY 0     // 1: the CSR mat-vec phase is compiled out (dense_f64.cu: the product's dense kernels carry no CSR code --
 #endif                        //    the register allocation and the schedule of the dense loop depend on everything inlined next to it)
 #ifndef CCQP_A_F32
 #define CCQP_A_F32 0          // 1: the dense Hessian is stored as fp32 and widened to fp64 in registers (dense_f32.cu)
@@ -54,7 +54,6 @@ constexpr int kDenseThreads = CCQP_DENSE_THREADS;
 constexpr int kDenseWarps = kDenseThreads / 32;
 constexpr int kUnroll = CCQP_UNROLL;  // 256-bit loads in flight per lane
 constexpr int kUnrollF32 = CCQP_UNROLL_F32;
-static_assert(kUnrollF32 >= 1 && kUnrollF32 <= 32, "the fp32 loop's remainder chain (16/8/4/2/1) covers at most 31 chunks");
 #if CCQP_A_F32
 using AElem = float;                  // what DenseCtx::A points at
 #else
@@ -76,8 +75,8 @@ struct DenseOut {          // written by CTA 0 / thread 0
 constexpr int kNumVec = 12;
 
 struct DenseCtx {
-    // Hessian row shard (fp32 build: A points at floats, read as AElem; lda counts stored entries)
-    const double* A;
+    // Hessian row shard: AElem (fp64, or fp32 in the fp32 build) entries; lda counts entries
+    const void* A;
     long long lda;
     int n;              // columns = unknowns
     int row0, nrows;    // rows [row0, row0+nrows) live on this device
@@ -208,89 +207,33 @@ __device__ __forceinline__ unsigned long long and_sync(Kst& k, const DenseCtx& c
 // ------------------------------------------------------------------------------------------
 // mat-vec phase
 // ------------------------------------------------------------------------------------------
-// U consecutive 128-column chunks: all U 256-bit loads of the lane are issued before the first FMA
-template <bool kEF, int U>
-__device__ __forceinline__ void dot_chunks(const double* ap, const double* vp, double& a0, double& a1, double& a2,
-                                           double& a3) {
-    double r[U][4];
-#pragma unroll
-    for (int u = 0; u < U; ++u) ldg256_stream<kEF>(ap + (size_t)u * 128, r[u]);
-#if CCQP_DENSE_LDS
-    const uint32_t vp32 = smem_u32(vp);       // explicit LDS.128 pairs instead of the generic LD.E.128 the compiler emits for vp
-#endif
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-#if CCQP_DENSE_LDS
-        double4 v;
-        asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(vp32 + (uint32_t)u * 1024u));
-        asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.z), "=d"(v.w) : "r"(vp32 + (uint32_t)u * 1024u + 16u));
-#else
-        const double4 v = *reinterpret_cast<const double4*>(vp + (size_t)u * 128);
-#endif
-        a0 = fma(r[u][0], v.x, a0);
-        a1 = fma(r[u][1], v.y, a1);
-        a2 = fma(r[u][2], v.z, a2);
-        a3 = fma(r[u][3], v.w, a3);
-    }
-}
+// A is read as fp64 (256-bit loads of four doubles) or, in the fp32 build (dense_f32.cu), as fp32 (128-bit loads of four
+// floats, one chunk of 128 columns = 512 bytes per warp), with the same lane -> column mapping, FMA chains and reductions:
+// every fp32 entry is widened exactly in a register before its fma, so the result is bit-identical to the fp64 loop on
+// the widened matrix.  kUnrollF32 loads in flight per lane keep the fp64 loop's 512 bytes per lane.
+template <class T> constexpr int kUnrollOf = sizeof(T) == 8 ? kUnroll : kUnrollF32;
+static_assert(kUnroll >= 1 && kUnroll <= 32 && kUnrollF32 >= 1 && kUnrollF32 <= 32,
+              "the remainder chain of dot_seg_aligned (16/8/4/2/1) covers at most 31 chunks");
 
-// One (row, segment) task of a warp: lanes own 4 consecutive columns of every 128-column chunk.
-// Chunks are consumed in order (kUnroll at a time, then 8/4/2/1 for the remainder), so the
-// summation order does not depend on the blocking.
-template <bool kEF>
-__device__ __forceinline__ double dot_seg_aligned(const double* __restrict__ arow, const double* vs, int ncol,
-                                                  int lane) {
-    double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
-    const int nchunk = ncol >> 7;
-    const double* ap = arow + lane * 4;
-    const double* vp = vs + lane * 4;
-    int c = 0;
-    for (; c + kUnroll <= nchunk; c += kUnroll) dot_chunks<kEF, kUnroll>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3);
-    if (kUnroll > 8 && c + 8 <= nchunk) { dot_chunks<kEF, 8>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 8; }
-    if (kUnroll > 4 && c + 4 <= nchunk) { dot_chunks<kEF, 4>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 4; }
-    if (kUnroll > 2 && c + 2 <= nchunk) { dot_chunks<kEF, 2>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 2; }
-    if (c < nchunk) { dot_chunks<kEF, 1>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 1; }
-    const int col = (nchunk << 7) + lane * 4;
-    if (col < ncol) {
-        a0 = fma(ldg_stream(arow + col), vs[col], a0);
-        if (col + 1 < ncol) a1 = fma(ldg_stream(arow + col + 1), vs[col + 1], a1);
-        if (col + 2 < ncol) a2 = fma(ldg_stream(arow + col + 2), vs[col + 2], a2);
-        if (col + 3 < ncol) a3 = fma(ldg_stream(arow + col + 3), vs[col + 3], a3);
-    }
-    return (a0 + a1) + (a2 + a3);
-}
-
-// any alignment / any lda: 64-bit loads, lanes contiguous
-__device__ __forceinline__ double dot_seg_generic(const double* __restrict__ arow, const double* vs, int ncol,
-                                                  int lane) {
-    double a0 = 0.0, a1 = 0.0;
-    int c = lane;
-    for (; c + 32 < ncol; c += 64) {
-        const double x0 = ldg_stream(arow + c), x1 = ldg_stream(arow + c + 32);
-        a0 = fma(x0, vs[c], a0);
-        a1 = fma(x1, vs[c + 32], a1);
-    }
-    if (c < ncol) a0 = fma(ldg_stream(arow + c), vs[c], a0);
-    return a0 + a1;
-}
-
-// fp32 Hessian (dense_f32.cu).  The same lane -> column mapping, FMA chains and reductions as the two loops above, from
-// 128-bit loads of four floats (one chunk of 128 columns = 512 bytes per warp); every entry is widened exactly in a
-// register before its fma, so the result is bit-identical to the fp64 loop on the widened matrix.  kUnrollF32 loads in
-// flight per lane keep the fp64 loop's 512 bytes per lane; chunks are still consumed in order (remainders 16/8/4/2/1).
-// The vector panel is read with explicit ld.shared: with plain loads the compiler hoisted the 32 vector reads of a batch
-// next to the A loads, and APGD / APGD-AR / BBPGD / BBPGDf spilled (72-184 bytes, ptxas -v).
-template <bool kEF, int U>
-__device__ __forceinline__ void dot_chunks(const float* ap, const double* vp, double& a0, double& a1, double& a2, double& a3) {
-    float r[U][4];
+// U consecutive 128-column chunks: all U vector loads of the lane are issued before the first FMA.
+// The fp32 loop reads the vector panel with explicit ld.shared: with plain loads the compiler hoisted the 32 vector reads
+// of a batch next to the A loads, and APGD / APGD-AR / BBPGD / BBPGDf spilled (72-184 bytes, ptxas -v).
+template <bool kEF, int U, class T>
+__device__ __forceinline__ void dot_chunks(const T* ap, const double* vp, double& a0, double& a1, double& a2, double& a3) {
+    constexpr bool kLds = CCQP_DENSE_LDS || sizeof(T) == 4;
+    T r[U][4];
 #pragma unroll
-    for (int u = 0; u < U; ++u) ldg128_stream<kEF>(ap + (size_t)u * 128, r[u]);
-    const uint32_t vp32 = smem_u32(vp);
+    for (int u = 0; u < U; ++u) ldg_vec4_stream<kEF>(ap + (size_t)u * 128, r[u]);
+    const uint32_t vp32 = smem_u32(vp);       // kLds: explicit LDS.128 pairs instead of the generic LD.E.128 the compiler emits for vp
 #pragma unroll
     for (int u = 0; u < U; ++u) {
         double4 v;
-        asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(vp32 + (uint32_t)u * 1024u));
-        asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.z), "=d"(v.w) : "r"(vp32 + (uint32_t)u * 1024u + 16u));
+        if constexpr (kLds) {
+            asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(vp32 + (uint32_t)u * 1024u));
+            asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.z), "=d"(v.w) : "r"(vp32 + (uint32_t)u * 1024u + 16u));
+        } else {
+            v = *reinterpret_cast<const double4*>(vp + (size_t)u * 128);
+        }
         a0 = fma((double)r[u][0], v.x, a0);
         a1 = fma((double)r[u][1], v.y, a1);
         a2 = fma((double)r[u][2], v.z, a2);
@@ -298,18 +241,22 @@ __device__ __forceinline__ void dot_chunks(const float* ap, const double* vp, do
     }
 }
 
-template <bool kEF>
-__device__ __forceinline__ double dot_seg_aligned(const float* __restrict__ arow, const double* vs, int ncol, int lane) {
+// One (row, segment) task of a warp: lanes own 4 consecutive columns of every 128-column chunk.
+// Chunks are consumed in order (kUnrollOf<T> at a time, then 16/8/4/2/1 for the remainder), so the
+// summation order does not depend on the blocking.
+template <bool kEF, class T>
+__device__ __forceinline__ double dot_seg_aligned(const T* __restrict__ arow, const double* vs, int ncol, int lane) {
+    constexpr int kU = kUnrollOf<T>;
     double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
     const int nchunk = ncol >> 7;
-    const float* ap = arow + lane * 4;
+    const T* ap = arow + lane * 4;
     const double* vp = vs + lane * 4;
     int c = 0;
-    for (; c + kUnrollF32 <= nchunk; c += kUnrollF32) dot_chunks<kEF, kUnrollF32>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3);
-    if (kUnrollF32 > 16 && c + 16 <= nchunk) { dot_chunks<kEF, 16>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 16; }
-    if (kUnrollF32 > 8 && c + 8 <= nchunk) { dot_chunks<kEF, 8>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 8; }
-    if (kUnrollF32 > 4 && c + 4 <= nchunk) { dot_chunks<kEF, 4>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 4; }
-    if (kUnrollF32 > 2 && c + 2 <= nchunk) { dot_chunks<kEF, 2>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 2; }
+    for (; c + kU <= nchunk; c += kU) dot_chunks<kEF, kU>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3);
+    if (kU > 16 && c + 16 <= nchunk) { dot_chunks<kEF, 16>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 16; }
+    if (kU > 8 && c + 8 <= nchunk) { dot_chunks<kEF, 8>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 8; }
+    if (kU > 4 && c + 4 <= nchunk) { dot_chunks<kEF, 4>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 4; }
+    if (kU > 2 && c + 2 <= nchunk) { dot_chunks<kEF, 2>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 2; }
     if (c < nchunk) { dot_chunks<kEF, 1>(ap + (size_t)c * 128, vp + (size_t)c * 128, a0, a1, a2, a3); c += 1; }
     const int col = (nchunk << 7) + lane * 4;
     if (col < ncol) {
@@ -321,7 +268,9 @@ __device__ __forceinline__ double dot_seg_aligned(const float* __restrict__ arow
     return (a0 + a1) + (a2 + a3);
 }
 
-__device__ __forceinline__ double dot_seg_generic(const float* __restrict__ arow, const double* vs, int ncol, int lane) {
+// any alignment / any lda: scalar loads, lanes contiguous
+template <class T>
+__device__ __forceinline__ double dot_seg_generic(const T* __restrict__ arow, const double* vs, int ncol, int lane) {
     double a0 = 0.0, a1 = 0.0;
     int c = lane;
     for (; c + 32 < ncol; c += 64) {
@@ -622,7 +571,7 @@ __device__ __forceinline__ void gemv_phase(Kst& k, const DenseCtx& c, const doub
             const int row = t / spp, seg = t - row * spp;
             const int col0 = seg * SW;
             const int ncol = min(SW, pc - col0);
-            const AElem* arow = reinterpret_cast<const AElem*>(c.A) + (size_t)(k.r0 - c.row0 + row) * c.lda + (size_t)p * CW + col0;
+            const AElem* arow = static_cast<const AElem*>(c.A) + (size_t)(k.r0 - c.row0 + row) * c.lda + (size_t)p * CW + col0;
             double acc;
             if (c.aligned) acc = t >= t_res ? dot_seg_aligned<true>(arow, vb + col0, ncol, lane)
                                             : dot_seg_aligned<false>(arow, vb + col0, ncol, lane);

@@ -1,29 +1,12 @@
-// Translation unit of the emulated-ranks instantiations of the dense solver kernels (dense.cuh
-// dense_kernel_emu); see internal.h.  Test vehicle only: ccqp_debug_solve_emulated().
+// Translation unit of the emulated-ranks instantiations of the dense solver kernels (dense.cuh dense_kernel_emu, fp64
+// Hessians, dense and CSR phase), in their own namespace (`ccqp::` becomes `ccqp_emu::`).  Test vehicle only:
+// ccqp_debug_solve_emulated().
+#define CCQP_DENSE_KERNELS 0
+#define CCQP_EMU_KERNELS 1
+#define ccqp ccqp_emu
 #include "dense.cuh"
+#include "kernel_build.cuh"
+#undef ccqp
 #include "internal.h"
 
-namespace ccqp {
-
-template <int OP>
-static cudaError_t launch_emu(const DenseCtx* d_ctxs, int world, int G, size_t smem, cudaStream_t stream) {
-    cudaError_t e = cudaFuncSetAttribute(dense_kernel_emu<OP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDenseSmemLimit);
-    if (e != cudaSuccess) return e;
-    void* args[] = {(void*)&d_ctxs, (void*)&G};
-    return cudaLaunchCooperativeKernel((const void*)dense_kernel_emu<OP>, dim3(world * G), dim3(kDenseThreads), args, smem, stream);
-}
-
-cudaError_t launch_dense_emu(int solver, const DenseCtx* d_ctxs, int world, int G, size_t smem, cudaStream_t stream) {
-    switch (solver) {
-        case CCQP_SOLVER_PGD: return launch_emu<OP_PGD>(d_ctxs, world, G, smem, stream);
-        case CCQP_SOLVER_APGD: return launch_emu<OP_APGD>(d_ctxs, world, G, smem, stream);
-        case CCQP_SOLVER_APGD_AR: return launch_emu<OP_APGD_AR>(d_ctxs, world, G, smem, stream);
-        case CCQP_SOLVER_BBPGD: return launch_emu<OP_BBPGD>(d_ctxs, world, G, smem, stream);
-        case CCQP_SOLVER_BBPGDF: return launch_emu<OP_BBPGDF>(d_ctxs, world, G, smem, stream);
-        case CCQP_SOLVER_SPG: return launch_emu<OP_SPG>(d_ctxs, world, G, smem, stream);
-        case CCQP_SOLVER_MPRGP: return launch_emu<OP_MPRGP>(d_ctxs, world, G, smem, stream);
-    }
-    return cudaErrorInvalidValue;
-}
-
-}  // namespace ccqp
+const ccqp::KernelBuild ccqp::kBuildEmu = ccqp_emu::describe<ccqp::KernelBuild>("emu.cu", 3);

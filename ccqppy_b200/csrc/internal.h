@@ -1,7 +1,8 @@
-// Entry points between the translation units of libccqp_b200.so (the kernels are split over several .cu files
-// only so that they compile in parallel): capi.cu (C-ABI, dense kernels), batched.cu (batched kernels),
-// emu.cu (emulated-ranks instantiations of the dense kernels, a test vehicle), csr.cu (CSR Hessians),
-// dense_f32.cu (fp32-stored dense Hessians).
+// Entry points between the translation units of libccqp_b200.so: capi.cu (C-ABI, host code), batched.cu + batched_sym.cu
+// (batched kernels), upload.cu (host -> device matrix copies), and the four compilations of the dense solver kernels, one
+// unit each because each sees dense.cuh with different macros: dense_f64.cu (fp64 Hessians), dense_f32.cu (fp32-stored
+// Hessians), csr.cu (CSR Hessians), emu.cu (emulated ranks, a test vehicle).  The rest are separate units only so that
+// they compile in parallel.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -36,21 +37,21 @@ cudaError_t mirror_lower(cudaStream_t stream, double* dst, long long n, long lon
 bool host_matrix_mirrors(const double* A, long long n, long long lda, int threads);
 int upload_block_rows();
 
-// emu.cu -- one cooperative launch of dense_kernel_emu<solver> over world * G CTAs
-cudaError_t launch_dense_emu(int solver, const DenseCtx* d_ctxs, int world, int G, size_t smem, cudaStream_t stream);
-
-// csr.cu -- the solver kernels compiled for CSR Hessians (many warps per SM, dense mat-vec loop compiled out); `ctx` points
-// at a DenseCtx, `op` is a DenseOp.  csr_variant_smem(): dynamic shared memory of that build's CSR tiling.
-int csr_variant_threads();
-size_t csr_variant_smem();
-int csr_variant_rows_max();
-size_t csr_variant_ctx_bytes();
-cudaError_t csr_variant_launch(int op, const void* ctx, int grid, size_t smem, bool cooperative, cudaStream_t stream);
-
-// dense_f32.cu -- the dense solver kernels compiled for an fp32-stored Hessian (widened in registers); `ctx` points at a
-// DenseCtx (`d_ctxs`: world of them in device memory), `op` is a DenseOp, `solver` a ccqp_solver
-size_t f32_variant_ctx_bytes();
-cudaError_t f32_variant_launch(int op, const void* ctx, int grid, size_t smem, bool cooperative, cudaStream_t stream);
-cudaError_t f32_variant_launch_emu(int solver, const void* d_ctxs, int world, int G, size_t smem, cudaStream_t stream);
+// One compilation of the dense.cuh solver programs (kernel_build.cuh).  `ctx` points at a DenseCtx, `d_ctxs` at world of
+// them in device memory; `op` is a DenseOp, `solver` a ccqp_solver; set_smem_limit: first launch of that kernel on this
+// device, raise its dynamic shared-memory limit first.
+struct KernelBuild {
+    const char* unit;           // translation unit, for error messages
+    int index;                  // 0 .. kNumBuilds - 1
+    int threads;                // kDenseThreads of that build
+    size_t ctx_bytes;           // sizeof(DenseCtx) as that build sees it
+    int csr_rows_max;           // CSR tiling of that build (0: no CSR phase)
+    cudaError_t (*launch)(int op, const void* ctx, int grid, size_t smem, bool cooperative, bool set_smem_limit,
+                          cudaStream_t stream);                         // null: no dense_kernel
+    cudaError_t (*launch_emu)(int solver, const void* d_ctxs, int world, int G, size_t smem, bool set_smem_limit,
+                              cudaStream_t stream);                     // null: no dense_kernel_emu
+};
+constexpr int kNumBuilds = 4;
+extern const KernelBuild kBuildF64, kBuildF32, kBuildCsr, kBuildEmu;
 
 }  // namespace ccqp

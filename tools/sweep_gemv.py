@@ -10,15 +10,12 @@ import ctypes as C
 import itertools
 import json
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "ccqppy_b200", "csrc")
 VAR = os.path.join(CSRC, "variants")
 VARIANTS = [(512, 8), (512, 4), (256, 8), (256, 16), (1024, 4), (1024, 2)]
-FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-fmad=false",
-         "-Xcompiler", "-fPIC", "-shared", "-DCCQP_SWEEP_BUILD"]
 
 
 def lib_path(t, u):
@@ -26,14 +23,13 @@ def lib_path(t, u):
 
 
 def build():
-    os.makedirs(VAR, exist_ok=True)
-    procs = []
-    for t, u in VARIANTS:
-        cmd = ["nvcc"] + FLAGS + ["-DCCQP_DENSE_THREADS=%d" % t, "-DCCQP_UNROLL=%d" % u,
-                                  os.path.join(CSRC, "capi.cu"), "-o", lib_path(t, u)]
-        procs.append(subprocess.Popen(cmd, cwd=CSRC))
-    for p in procs:
-        assert p.wait() == 0
+    """Every unit of the library, with the tuning macros, and only the mat-vec hook instantiated (CCQP_SWEEP_BUILD)."""
+    from concurrent.futures import ThreadPoolExecutor
+    sys.path.insert(0, ROOT)
+    from ccqppy_b200 import build as lib_build
+    with ThreadPoolExecutor(len(VARIANTS)) as pool:
+        list(pool.map(lambda tu: lib_build.build(lib=lib_path(*tu), defines=["CCQP_DENSE_THREADS=%d" % tu[0], "CCQP_UNROLL=%d" % tu[1],
+                                                                            "CCQP_SWEEP_BUILD"]), VARIANTS))
 
 
 def run():
