@@ -26,7 +26,7 @@ EXPORTS = ["ccqp_abi_version", "ccqp_status_string", "ccqp_last_error", "ccqp_cr
            "ccqp_comm_attach", "ccqp_comm_prepare", "ccqp_comm_detach", "ccqp_debug_divide", "ccqp_fp64_peak",
            "ccqp_microbench", "ccqp_debug_emulate_ranks", "ccqp_debug_solve_emulated", "ccqp_projected_gradient", "ccqp_solve_batched_table", "ccqp_solve_batched_sym",
            "ccqp_get_upload_info", "ccqp_set_matrix_symmetric", "ccqp_host_matrix_is_block_symmetric", "ccqp_upload_block_rows",
-           "ccqp_set_matrix_f32"]
+           "ccqp_set_matrix_f32", "ccqp_solve_batched_tables"]
 
 
 class Block(C.Structure):
@@ -86,6 +86,7 @@ def load():
     lib.ccqp_solve_batched_sym.argtypes = lib.ccqp_solve_batched.argtypes
     lib.ccqp_solve_batched_table.argtypes = [vp, i32, C.POINTER(Params), i64, i64, dp, dp, dp, C.POINTER(Block), i64, dp, i64, dp, i64,
                                              dp, i32, C.POINTER(Result), C.POINTER(Result)]
+    lib.ccqp_solve_batched_tables.argtypes = lib.ccqp_solve_batched_table.argtypes
     lib.ccqp_set_matrix_symmetric.argtypes = [vp, dp, i64, i64, i32]
     lib.ccqp_set_matrix_f32.argtypes = [vp, dp, i64, i64, i64, i64, i32]
     lib.ccqp_get_upload_info.argtypes = [vp, C.POINTER(i64), C.POINTER(i32)]

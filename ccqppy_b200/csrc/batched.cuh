@@ -2,15 +2,17 @@
 // reference inside one persistent kernel (no host round trips).  Problem i is
 //     CCQPSolverX(tol,max_mv).solve(A[i], b[i], x0[i], BoxProjOp(n, lb[i], ub[i]))          (ccqp_solve_batched)
 // or  CCQPSolverX(tol,max_mv).solve(A[i], b[i], x0[i], op)  with ONE operator of any kind    (ccqp_solve_batched_table)
+// or  CCQPSolverX(tol,max_mv).solve(A[i], b[i], x0[i], op_i), op_i one block structure with its own parameters
+//                                                                                         (ccqp_solve_batched_tables)
 // (solvers.py:94/220/393/583/719/878/1026 with solution_spaces.py:77-560).
 //
 // Data path per problem (n = 64: 32 KB of A, 2 KB of vectors in, 512 B out):
 //   * A lives in REGISTERS for the whole solve.  n <= 64: 64 threads, thread t = 8*rb + cb keeps the 8 x 8 sub-block
 //     A[8rb .. 8rb+7][8cb .. 8cb+7] (64 doubles = 128 registers), 6 CTAs per SM.  64 < n <= 128: 256 threads, a 16 x 16 grid
 //     of the same 8 x 8 sub-blocks, one CTA per SM (struct BL<NT>).  The problem AFTER the current one travels into a padded
-//     shared-memory tile by TMA row copies (cp.async.bulk + one mbarrier; its b / lb / ub rows ride on the same mbarrier)
-//     while the current one iterates; the register fill from the tile is conflict-free LDS.128.  The work queue is two
-//     problems deep, so neither the atomic that hands out problems nor any global load sits on a problem's dependent chain.
+//     shared-memory tile by TMA row copies (cp.async.bulk + one mbarrier; its b / lb / ub rows -- general table: b and its
+//     parameter row -- ride on the same mbarrier) while the current one iterates; the register fill from the tile is
+//     conflict-free LDS.128.  The work queue is two problems deep, so neither the atomic that hands out problems nor any global load sits on a problem's dependent chain.
 //   * mat-vec: the input vector is published through a double-buffered, bank-padded shared array (one barrier); a thread reads
 //     only its 8-entry slice (4 LDS.128), does 64 DFMAs (8 rows x 8 columns, 8 independent chains) and the lanes of a row
 //     block combine their partial rows with a 3-stage exchange butterfly (7 SHFL.64 + 7 DADD) after which the thread holds y
@@ -87,15 +89,17 @@ struct BatchedCtx {
     const double* A;        // [batch][n][n]
     const double* b;        // [batch][n]
     const double* x0;       // [batch][n] or null
-    const double* lb;       // [batch][n]; general table: [n], shared by all problems (bound_stride = 0)
+    const double* lb;       // [batch][n] (Box per problem; unused by the general table)
     const double* ub;
-    long long bound_stride; // n (per-problem bounds) or 0
-    // general projection table shared by all problems of the batch (ccqp_solve_batched_table); null = Box per problem
+    long long bound_stride; // n
+    // general projection table (ccqp_solve_batched_table / _tables): the block structure is shared by all problems of the
+    // batch, problem i takes its parameters from the row params + i * param_stride; null ekind = Box per problem
     const uint8_t* ekind;   // [n] kIdentity / kLower / kUpper / kBox / kElemNorm
     const int* eoff;        // [n] first element of the norm block the element belongs to
     const int* edim;        // [n] its dimension
     const int* enk;         // [n] its kind (kSphere / kConeRef / kSoc)
-    const double* epar;     // [n] its parameter (radius / aspect ratio)
+    const int4* eidx;       // [n] where the element's lower bound / upper bound / block parameter (radius / aspect ratio)
+                            // sit in a parameter row (x / y / z); -1: none (-inf / +inf / unused)
     int has_norm;           // some element belongs to a norm block
     const double* uniforms; // [batch][n_uniforms]
     long long n_uniforms;
@@ -106,19 +110,26 @@ struct BatchedCtx {
     int tma_ok;             // rows of A can be moved with 16-byte bulk copies (8n % 16 == 0, 16-byte aligned base)
     int vec_ok;             // rows of A can be read with 256-bit loads (n % 4 == 0, 32-byte aligned base)
     int pf_ok;              // whole problems can be bulk-prefetched into L2 (16-byte granularity)
-    int vtma_ok;            // b / lb / ub rows can be moved with 16-byte bulk copies (n even, 16-byte aligned bases)
+    int vtma_ok;            // b / lb / ub rows (general table: b and parameter rows) can be moved with 16-byte bulk copies
+                            // (n even, 16-byte aligned bases; general table: see prow_bytes)
     double tol, max_mv, step, tau, sig1, sig2;
     double thr_lt;          // q <  thr_lt  <=>  sqrt(q) <  tol      (solvers.py:156 etc.)
     double thr_le;          // q <= thr_le  <=>  sqrt(q) <= tol      (SPG, solvers.py:949)
     int max_mv_i;           // mv >= max_mv_i  <=>  (double)mv >= max_mv
     int m;
+    // general table: parameter rows (param_stride 0: one row shared by the whole batch)
+    const double* params;
+    long long param_stride;
+    int prow_bytes;         // bytes of a parameter row the bulk copy moves when vtma_ok: a multiple of 16, <= 16 N (the
+                            // vstage[1..2] area); 0: no parameters
 };
 
 template <bool GEN, int NT>
 struct BatchedSmem {
 #if CCQP_BATCHED_STAGE
     double tile[BL<NT>::N * BL<NT>::PITCH];   // the NEXT problem's A, landed by TMA while the current one iterates
-    double vstage[3][BL<NT>::N];              // ... and its b / lower / upper bounds (same mbarrier)
+    double vstage[3][BL<NT>::N];              // ... and its b / lower / upper bounds (general table: b / parameter row
+                                              // of up to 2 N entries in vstage[1..2]) on the same mbarrier
 #endif
     double xs[2][BL<NT>::XS];                 // mat-vec input, double buffered
     double red[2][BL<NT>::WARPS][4];          // [parity][warp][slot]
@@ -320,15 +331,14 @@ __device__ __forceinline__ double matvec(const double (&a)[kBRows][kBCols], cons
 }
 
 struct BState {                 // per-thread view of one problem (thread t <-> unknown t)
-    double b, lo, hi, x0;
+    double b, lo, hi, x0;       // general table: a member of a norm block has no bounds, its `lo` is the block's parameter
     double cs;                  // 1/(3 n gd)
     bool act;                   // the unknown exists (index < n)
     bool own;                   // ... and this thread is the lane that owns it (NT = 64: the same thing)
     int u;                      // index of the unknown
     // general table only
     int kind;                   // element kind
-    int boff, bdim, bnk;        // norm block of this element
-    double bpar;
+    int boff, bdim, bnk;        // norm block of this element (its parameter: lo)
     uint32_t pj;                // shared address of pj[0][0]
 };
 
@@ -345,7 +355,7 @@ __device__ __forceinline__ double project_general(const BState& s, bool has_norm
         __syncthreads();
         if (s.kind == kElemNorm) {
             NormRule R;
-            R.kind = s.bnk; R.par = s.bpar;
+            R.kind = s.bnk; R.par = s.lo;
             const int nsq = (s.bnk == kSoc) ? s.bdim - 1 : s.bdim;
             double ss = 0.0, last = 0.0;
             for (int j = 0; j < s.bdim; ++j) {
@@ -702,12 +712,23 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
     unsigned phase = 0;
     if (t == 0) { mbar_init(&sm.mbar, 1); mbar_fence_init(); }
     auto issue_load = [&](int prob) {       // one 8n-byte bulk copy per row into the padded tile (+ 3 for the vectors), one mbarrier
-        if (t == 0) mbar_expect_tx(&sm.mbar, (uint32_t)(prob_elems * 8) + (vstaged ? 3u * (uint32_t)(n * 8) : 0u));
-        if (t < n) bulk_g2s(sm.tile + t * L::PITCH, c.A + (size_t)prob * prob_elems + (size_t)t * n, (uint32_t)(n * 8), &sm.mbar);
-        if (vstaged && t >= NT - 3) {       // three otherwise idle-ish threads (the mbarrier's expect_tx is program-ordered only in thread 0,
-            const int w = t - (NT - 3);     // but a complete_tx that arrives first just drives the pending count negative: legal)
-            const double* src = w == 0 ? c.b + (size_t)prob * n : (w == 1 ? c.lb : c.ub) + (size_t)prob * c.bound_stride;
-            bulk_g2s(sm.vstage[w], src, (uint32_t)(n * 8), &sm.mbar);
+        if constexpr (GEN) {
+            // b into vstage[0], the problem's parameter row into vstage[1..2].  bb / pb are the one definition of what is
+            // copied: thread 0 announces exactly bb + pb bytes besides A, and a copy is issued iff its size is non-zero
+            // (announced bytes that never arrive would leave mbar_wait spinning forever).
+            const uint32_t bb = vstaged ? (uint32_t)(n * 8) : 0u, pb = vstaged ? (uint32_t)c.prow_bytes : 0u;
+            if (t == 0) mbar_expect_tx(&sm.mbar, (uint32_t)(prob_elems * 8) + bb + pb);
+            if (t < n) bulk_g2s(sm.tile + t * L::PITCH, c.A + (size_t)prob * prob_elems + (size_t)t * n, (uint32_t)(n * 8), &sm.mbar);
+            if (bb != 0u && t == NT - 1) bulk_g2s(sm.vstage[0], c.b + (size_t)prob * n, bb, &sm.mbar);
+            if (pb != 0u && t == NT - 2) bulk_g2s(sm.vstage[1], c.params + (size_t)prob * c.param_stride, pb, &sm.mbar);
+        } else {
+            if (t == 0) mbar_expect_tx(&sm.mbar, (uint32_t)(prob_elems * 8) + (vstaged ? 3u * (uint32_t)(n * 8) : 0u));
+            if (t < n) bulk_g2s(sm.tile + t * L::PITCH, c.A + (size_t)prob * prob_elems + (size_t)t * n, (uint32_t)(n * 8), &sm.mbar);
+            if (vstaged && t >= NT - 3) {   // three otherwise idle-ish threads (the mbarrier's expect_tx is program-ordered only in thread 0,
+                const int w = t - (NT - 3); // but a complete_tx that arrives first just drives the pending count negative: legal)
+                const double* src = w == 0 ? c.b + (size_t)prob * n : (w == 1 ? c.lb : c.ub) + (size_t)prob * c.bound_stride;
+                bulk_g2s(sm.vstage[w], src, (uint32_t)(n * 8), &sm.mbar);
+            }
         }
     };
 #else
@@ -747,8 +768,10 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
             }
             if (vstaged) {
                 s.b = s.act ? sm.vstage[0][u] : 0.0;
-                s.lo = s.act ? sm.vstage[1][u] : 0.0;
-                s.hi = s.act ? sm.vstage[2][u] : 0.0;
+                if constexpr (!GEN) {
+                    s.lo = s.act ? sm.vstage[1][u] : 0.0;
+                    s.hi = s.act ? sm.vstage[2][u] : 0.0;
+                }
             }
 #endif
         } else if (c.vec_ok) {
@@ -773,13 +796,28 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
         }
         if (!vstaged) {
             s.b = s.act ? c.b[vo] : 0.0;
-            s.lo = s.act ? c.lb[bo] : 0.0;
-            s.hi = s.act ? c.ub[bo] : 0.0;
+            if constexpr (!GEN) {
+                s.lo = s.act ? c.lb[bo] : 0.0;
+                s.hi = s.act ? c.ub[bo] : 0.0;
+            }
         }
         if constexpr (GEN) {
             s.kind = s.act ? c.ekind[u] : kIdentity;
             s.boff = s.act ? c.eoff[u] : 0; s.bdim = s.act ? c.edim[u] : 0; s.bnk = s.act ? c.enk[u] : 0;
-            s.bpar = s.act ? c.epar[u] : 0.0;
+            // this problem's bounds / block parameter: its parameter row (staged next to b, or in global memory) at the
+            // element's indices
+            const int4 e = s.act ? __ldg(c.eidx + u) : make_int4(-1, -1, -1, -1);
+            const double* prow = c.params + (size_t)cur * c.param_stride;
+            auto prm = [&](int k, double none) {
+                if (k < 0) return none;
+#if CCQP_BATCHED_STAGE
+                if (vstaged) return lds_f64(smem_u32(&sm.vstage[1][0]) + (uint32_t)k * 8u);   // the row runs on into vstage[2]
+#endif
+                return __ldg(prow + k);
+            };
+            const bool nb = s.kind == kElemNorm;
+            s.lo = prm(nb ? e.z : e.x, nb ? 0.0 : -INFINITY);
+            s.hi = prm(e.y, INFINITY);
             s.pj = smem_u32(&sm.pj[0][0]);
         }
         s.x0 = (s.act && c.x0) ? c.x0[vo] : 0.0;
@@ -861,12 +899,17 @@ inline cudaError_t launch_batched(const BatchedCtx& c, int sm_count, cudaStream_
                       : launch_batched_nt<SOLVER, WREG, GEN, 256>(c, sm_count, stream);
 }
 
-// One projection table shared by every problem of a batch (ccqp_solve_batched_table), per element, on the HOST
+// The block structure of a general table, per element, on the HOST (batched.cu batched_table_layout), and where its
+// parameters are: one row shared by every problem (ccqp_solve_batched_table, a host array) or one row per problem
+// (ccqp_solve_batched_tables, [batch][n_params] where A lives)
 struct BatchedTable {
-    std::vector<double> lo, hi, epar;
     std::vector<uint8_t> ekind;
     std::vector<int> eoff, edim, enk;
+    std::vector<int> eidx;          // [n][4]: lower bound / upper bound / block parameter index into a row, -1: none
     int has_norm = 0;
+    const double* params = nullptr;
+    long long n_params = 0;
+    bool per_problem = false;
 };
 
 // batched_sym.cu: the one-warp-per-problem kernels for symmetric Hessians (n <= 64; PGD / BBPGD / BBPGDf / SPG, Box per problem)
@@ -893,7 +936,11 @@ inline int batched_solve(cudaStream_t stream, int sm_count, const BatchedTable* 
     const size_t szU = (solver == CCQP_SOLVER_SPG) ? (size_t)batch * n_uniforms * 8 : 0;
     const size_t szO = (size_t)batch * sizeof(BatchedOut);
     auto al = [](size_t v) { return (v + 255) / 256 * 256; };
-    size_t total = 256 + al(szO) + 8 * al((size_t)kBNMax * 8);
+    // parameter rows of a general table: a shared row and the rows of a host array are copied with an even pitch, so that
+    // every row starts 16-byte aligned and its bulk copy (rounded up to 16 bytes) stays inside the copy
+    const long long np = tab ? std::max(tab->n_params, 0LL) : 0, ppitch = np + (np & 1);
+    const size_t szP = !tab ? 0 : !tab->per_problem ? (size_t)ppitch * 8 : host ? (size_t)batch * ppitch * 8 : 0;
+    size_t total = 256 + al(szO) + 8 * al((size_t)kBNMax * 8) + al(szP);
     if (host) total += al(szA) + 4 * al(szV) + al(szV) + al(szU);
     unsigned char* ws = static_cast<unsigned char*>(alloc(total));
     if (!ws) { err = "workspace allocation failed"; return CCQP_ERR_CUDA; }
@@ -923,21 +970,32 @@ inline int batched_solve(cudaStream_t stream, int sm_count, const BatchedTable* 
         c.x_out = x_out;
     }
     c.bound_stride = n;
-    if (tab) {        // the shared table: seven small per-element arrays, uploaded once per call
+    if (tab) {        // the block structure: five small per-element arrays, uploaded once per call
         auto up = [&](const void* src, size_t bytes) -> void* {
-            void* d = take((size_t)kBNMax * 8);
+            void* d = take(bytes);
             return cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, stream) == cudaSuccess ? d : nullptr;
         };
-        c.lb = static_cast<const double*>(up(tab->lo.data(), (size_t)n * 8));
-        c.ub = static_cast<const double*>(up(tab->hi.data(), (size_t)n * 8));
-        c.epar = static_cast<const double*>(up(tab->epar.data(), (size_t)n * 8));
         c.ekind = static_cast<const uint8_t*>(up(tab->ekind.data(), (size_t)n));
         c.eoff = static_cast<const int*>(up(tab->eoff.data(), (size_t)n * 4));
         c.edim = static_cast<const int*>(up(tab->edim.data(), (size_t)n * 4));
         c.enk = static_cast<const int*>(up(tab->enk.data(), (size_t)n * 4));
-        if (!c.lb || !c.ub || !c.epar || !c.ekind || !c.eoff || !c.edim || !c.enk) { err = "table upload failed"; return CCQP_ERR_CUDA; }
+        c.eidx = static_cast<const int4*>(up(tab->eidx.data(), (size_t)n * 16));
+        if (!c.ekind || !c.eoff || !c.edim || !c.enk || !c.eidx) { err = "table upload failed"; return CCQP_ERR_CUDA; }
         c.has_norm = tab->has_norm;
-        c.bound_stride = 0;
+        c.lb = c.ub = nullptr;
+        // the parameter rows: one shared row (stride 0), a host array copied with an even pitch, or a device array in place
+        if (np > 0 && (!tab->per_problem || host)) {
+            double* dp = reinterpret_cast<double*>(take(szP));
+            const long long rows = tab->per_problem ? batch : 1;
+            if (ppitch == np) BCU(cudaMemcpyAsync(dp, tab->params, (size_t)rows * np * 8, cudaMemcpyHostToDevice, stream));
+            else BCU(cudaMemcpy2DAsync(dp, (size_t)ppitch * 8, tab->params, (size_t)np * 8, (size_t)np * 8, (size_t)rows,
+                                       cudaMemcpyHostToDevice, stream));
+            c.params = dp;
+            c.param_stride = tab->per_problem ? ppitch : 0;
+        } else {
+            c.params = np > 0 ? tab->params : nullptr;
+            c.param_stride = np;
+        }
     }
     c.n_uniforms = (solver == CCQP_SOLVER_SPG) ? n_uniforms : 0;
     c.out = dout; c.counter = counter;
@@ -946,6 +1004,12 @@ inline int batched_solve(cudaStream_t stream, int sm_count, const BatchedTable* 
     c.vec_ok = (n % 4 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 31) == 0) ? 1 : 0;
     c.pf_ok = ((n * n * 8) % 16 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 15) == 0) ? 1 : 0;
     c.vtma_ok = (n % 2 == 0 && ((reinterpret_cast<uintptr_t>(c.b) | reinterpret_cast<uintptr_t>(c.lb) | reinterpret_cast<uintptr_t>(c.ub)) & 15) == 0) ? 1 : 0;
+    if (tab) {        // a parameter row is staged with b when every row is 16-byte aligned and fits vstage[1..2] (2 N doubles)
+        const long long N = n <= kBN ? kBN : kBNMax;
+        const bool rows_ok = np == 0 || (c.param_stride % 2 == 0 && (reinterpret_cast<uintptr_t>(c.params) & 15) == 0 && ppitch <= 2 * N);
+        c.vtma_ok = (c.vtma_ok && rows_ok) ? 1 : 0;
+        c.prow_bytes = c.vtma_ok ? (int)(ppitch * 8) : 0;
+    }
     c.tol = prm.tol; c.max_mv = prm.max_mv; c.step = prm.step_size;
     c.tau = prm.tau; c.sig1 = prm.sigma1; c.sig2 = prm.sigma2; c.m = prm.m;
     c.thr_lt = sqrt_threshold(prm.tol, true);
@@ -996,6 +1060,7 @@ inline int batched_solve(cudaStream_t stream, int sm_count, const BatchedTable* 
     int first_status = 0;
     double hbmA = 8.0 * n * n;                  // bytes of A[i] the kernel reads
     if (use_sym) { hbmA = 0; for (long long i = 0; i < n; ++i) hbmA += 8.0 * (double)(n - 8 * (i / 8)); }
+    if (tab && tab->per_problem) hbmA += 8.0 * (double)np;     // the problem's parameter row
     for (long long i = 0; i < batch; ++i) {
         const BatchedOut& o = hout[(size_t)i];
         if (results) {

@@ -847,23 +847,39 @@ ccqp_status ccqp_solve_batched_sym(ccqp_handle* h, int solver, const ccqp_params
     return solve_batched_box(h, true, solver, params, batch, n, A, b, x0, lb, ub, uniforms, n_uniforms, x_out, memtype, results, summary);
 }
 
-ccqp_status ccqp_solve_batched_table(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
-                                     const double* A, const double* b, const double* x0, const ccqp_block* blocks, int64_t n_blocks,
-                                     const double* block_params, int64_t n_params, const double* uniforms, int64_t n_uniforms,
-                                     double* x_out, int memtype, ccqp_result* results, ccqp_result* summary) {
+static ccqp_status solve_batched_tab(ccqp_handle* h, bool per_problem, int solver, const ccqp_params* params, int64_t batch,
+                                     int64_t n, const double* A, const double* b, const double* x0, const ccqp_block* blocks,
+                                     int64_t n_blocks, const double* block_params, int64_t n_params, const double* uniforms,
+                                     int64_t n_uniforms, double* x_out, int memtype, ccqp_result* results, ccqp_result* summary) {
     if (!h || !params_ok(params, solver) || batch <= 0 || n <= 0 || !A || !b || !x_out || !blocks || n_blocks <= 0 ||
-        (n_params > 0 && !block_params))
+        (n_params > 0 && !block_params) || (per_problem && n_params < 0))
         return CCQP_ERR_INVALID_ARG;
     CU(h, cudaSetDevice(h->device));
     std::string err;
     int launches = 0;
     ccqp_status st = (ccqp_status)batched_solve_table_entry(h->stream, h->sm_count, solver, *params, batch, n, A, b, x0, blocks, n_blocks,
-                                                            block_params, n_params, uniforms, n_uniforms, x_out, memtype, results, summary,
-                                                            h->ev0, h->ev1, &launches, err,
+                                                            block_params, n_params, per_problem, uniforms, n_uniforms, x_out, memtype,
+                                                            results, summary, h->ev0, h->ev1, &launches, err,
                                                             [&](size_t bytes) -> void* { return h->batched_ws.ensure(bytes) == cudaSuccess ? h->batched_ws.p : nullptr; });
     h->launches += launches;
     if (st == CCQP_ERR_CUDA) h->last_error = err;
     return st;
+}
+
+ccqp_status ccqp_solve_batched_table(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
+                                     const double* A, const double* b, const double* x0, const ccqp_block* blocks, int64_t n_blocks,
+                                     const double* block_params, int64_t n_params, const double* uniforms, int64_t n_uniforms,
+                                     double* x_out, int memtype, ccqp_result* results, ccqp_result* summary) {
+    return solve_batched_tab(h, false, solver, params, batch, n, A, b, x0, blocks, n_blocks, block_params, n_params, uniforms,
+                             n_uniforms, x_out, memtype, results, summary);
+}
+
+ccqp_status ccqp_solve_batched_tables(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
+                                      const double* A, const double* b, const double* x0, const ccqp_block* blocks, int64_t n_blocks,
+                                      const double* block_params, int64_t n_params, const double* uniforms, int64_t n_uniforms,
+                                      double* x_out, int memtype, ccqp_result* results, ccqp_result* summary) {
+    return solve_batched_tab(h, true, solver, params, batch, n, A, b, x0, blocks, n_blocks, block_params, n_params, uniforms,
+                             n_uniforms, x_out, memtype, results, summary);
 }
 
 namespace {

@@ -22,12 +22,15 @@ int batched_solve_entry(cudaStream_t stream, int sm_count, int solver, const ccq
                         ccqp_result* summary, cudaEvent_t ev0, cudaEvent_t ev1, int* launches, std::string& err,
                         const std::function<void*(size_t)>& alloc, bool symmetric = false);
 
-// the same with ONE projection table (any block kinds) shared by all problems of the batch instead of a Box per problem
+// the same with a projection table (any block kinds) instead of a Box per problem: the block structure is shared by all
+// problems of the batch; per_problem = false: ONE host parameter array `params` for all of them, true: params is
+// [batch][n_params] in `memtype` memory, row i for problem i
 int batched_solve_table_entry(cudaStream_t stream, int sm_count, int solver, const ccqp_params& prm, long long batch, long long n,
                               const double* A, const double* b, const double* x0, const ccqp_block* blocks, long long n_blocks,
-                              const double* params, long long n_params, const double* uniforms, long long n_uniforms, double* x_out,
-                              int memtype, ccqp_result* results, ccqp_result* summary, cudaEvent_t ev0, cudaEvent_t ev1, int* launches,
-                              std::string& err, const std::function<void*(size_t)>& alloc);
+                              const double* params, long long n_params, bool per_problem, const double* uniforms,
+                              long long n_uniforms, double* x_out, int memtype, ccqp_result* results, ccqp_result* summary,
+                              cudaEvent_t ev0, cudaEvent_t ev1, int* launches, std::string& err,
+                              const std::function<void*(size_t)>& alloc);
 
 // upload.cu -- host -> device copy of a square matrix; a symmetric one crosses PCIe as its upper block triangle (checked on the host
 // while the copies run) and is mirrored on the device: the device copy is bit-identical to a full upload either way

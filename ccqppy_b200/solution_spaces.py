@@ -279,6 +279,27 @@ class SOCProjOp(ProjOpBase):
         return [(_capi.SOC, offset, self.dim, poff)]
 
 
+def stacked_descriptor(ops):
+    """Extension (not star-exported).  Block table shared by a sequence of operators and their parameter arrays stacked
+    row by row: (ctypes ccqp_block array, float64 [len(ops), n_params]).  Row i is exactly `ops[i].descriptor()[1]`.  The operators must have the same
+    block structure -- identical `descriptor()` rows (kind, offset, dim, param_off) -- or ValueError names the first one
+    that differs.  This is the input of a batched solve with per-problem parameters (`solve_batched`)."""
+    ops = list(ops)
+    if not ops:
+        raise ValueError("stacked_descriptor needs at least one operator")
+    blocks, first, rows = ops[0].descriptor()
+    ref = np.asarray(rows, dtype=np.int64).reshape(-1, 4)
+    P = np.empty((len(ops), first.size))
+    P[0] = first
+    for i, op in enumerate(ops[1:], 1):
+        _, par, r = op.descriptor()
+        r = np.asarray(r, dtype=np.int64).reshape(-1, 4)
+        if r.shape != ref.shape or not np.array_equal(r, ref) or par.size != first.size:
+            raise ValueError("operator %d has a different block structure (kind, offset, dim, param_off) than operator 0" % i)
+        P[i] = par
+    return blocks, P
+
+
 class DisjointProjOp(ProjOpBase):
     """solution_spaces.py:495-560: concatenation of operators acting on consecutive slices."""
 

@@ -13,7 +13,9 @@ the host.
 
 Extensions beyond the reference API (all optional):
   * `solve(..., uniforms=...)`      explicit U[0,1) stream for SPG instead of the global NumPy RNG
-  * `solve_batched(A, b, lb, ub)`   many small QPs in one persistent kernel (n <= 128; per-problem boxes or one shared table)
+  * `solve_batched(A, b, lb, ub)`   many small QPs in one persistent kernel (n <= 128; per-problem boxes, one shared table,
+                                    or one block structure with per-problem parameters: `convex_proj_op=op, op_params=P`
+                                    or a sequence of operators)
   * `solution_gpu_time`, `solution_hbm_bytes`, `solution_gemv_count` after a solve
   * A / b / x0 may be torch tensors; a CUDA tensor A is used in place (no copy) when it is float64, or float32,
     contiguous and 16-byte aligned
@@ -272,12 +274,22 @@ class CCQPSolverBase(ABC):
         return max(1, int(min(mx, cap))) if np.isfinite(mx) else min(cap, 4096)
 
     def solve_batched(self, A, b, lower_bound=None, upper_bound=None, x0=None, seeds=None, uniforms=None, n_uniforms=None,
-                      device=-1, convex_proj_op=None, symmetric=False):
+                      device=-1, convex_proj_op=None, symmetric=False, op_params=None):
         """Extension: solve `batch` independent constrained QPs in one persistent kernel.
 
-        Either per-problem boxes (`lower_bound` / `upper_bound` [batch, n]) or ONE operator of
-        `ccqppy_b200.solution_spaces` shared by all problems (`convex_proj_op`, any block kinds: the
-        contact-style case where every problem has the same friction-disc structure; all solvers except MPRGP).
+        The feasible set is one of
+          * per-problem boxes (`lower_bound` / `upper_bound` [batch, n]);
+          * ONE operator of `ccqppy_b200.solution_spaces` shared by all problems (`convex_proj_op=op`, any block kinds:
+            the contact-style case where every problem has the same friction-disc structure);
+          * one block structure with per-problem parameters: `convex_proj_op=op, op_params=P`, P [batch, n_params]
+            (NumPy or torch, host or device; a CUDA tensor is used in place when A is on the device), row i laid out as
+            `op.descriptor()[1]` -- problem i is solved with op's blocks and the bounds / radii / aspect ratios of P[i],
+            e.g. friction discs of radius mu * f_n computed on the GPU;
+          * a sequence of `batch` operators `[op_0, ..., op_{batch-1}]` with identical `descriptor()` rows (kind, offset,
+            dim, param_off): problem i is `solve(A[i], b[i], x0[i], op_i)`.  Their parameters are stacked into P.
+        Tables run every solver except MPRGP (CCQPError).  A P of the wrong shape, a sequence of the wrong length or
+        structure, `op_params` without `convex_proj_op` or together with bounds, and an operator of the wrong dimension
+        raise ValueError before anything reaches the device.
 
         A [batch, n, n], b / lower_bound / upper_bound / x0 [batch, n] (NumPy or torch, host or
         device).  Problem i equals `type(self)(tol, max_mv).solve(A[i], b[i], x0[i],
@@ -302,13 +314,38 @@ class CCQPSolverBase(ABC):
         A64 = _as_f64(A, dev)
         batch, n = int(A64.shape[0]), int(A64.shape[1])
         b64 = _as_f64(b, dev)
+        P64 = None          # per-problem parameter rows [batch, n_params], where A lives
+        if op_params is not None and convex_proj_op is None:
+            raise ValueError("op_params needs convex_proj_op: the operator that supplies the block structure")
         if convex_proj_op is not None:
             if lower_bound is not None or upper_bound is not None:
                 raise ValueError("give either lower_bound / upper_bound or convex_proj_op")
-            if not isinstance(convex_proj_op, ss.ProjOpBase):
-                raise TypeError("convex_proj_op must be an operator from ccqppy_b200.solution_spaces")
-            if convex_proj_op.embedded_dimension != n:
-                raise ValueError("convex_proj_op has dimension %d, the problems %d" % (convex_proj_op.embedded_dimension, n))
+            seq = isinstance(convex_proj_op, (list, tuple))     # one operator per problem
+            ops = list(convex_proj_op) if seq else [convex_proj_op]
+            if seq and op_params is not None:
+                raise ValueError("give op_params with ONE operator (the structure), not with a sequence of operators")
+            if seq and len(ops) != batch:
+                raise ValueError("convex_proj_op has %d operators for %d problems" % (len(ops), batch))
+            for i, op in enumerate(ops):
+                if not isinstance(op, ss.ProjOpBase):
+                    raise TypeError("convex_proj_op must be an operator from ccqppy_b200.solution_spaces (or a sequence of them)")
+                if op.embedded_dimension != n:
+                    raise ValueError("convex_proj_op%s has dimension %d, the problems %d" % (
+                        "[%d]" % i if seq else "", op.embedded_dimension, n))
+            if seq:
+                blocks, op_params = ss.stacked_descriptor(ops)
+                n_params = op_params.shape[1]
+            else:
+                blocks, params, _rows = convex_proj_op.descriptor()
+                n_params = params.size
+            if op_params is not None:
+                shape = tuple(op_params.shape) if hasattr(op_params, "shape") else np.shape(op_params)
+                if tuple(shape) != (batch, n_params):
+                    raise ValueError("op_params has shape %s, expected (batch, n_params) = (%d, %d) (rows laid out as "
+                                     "convex_proj_op.descriptor()[1])" % (tuple(shape), batch, n_params))
+                P64 = _as_f64(op_params, dev)
+                if dev is None and _is_torch(P64) and P64.is_cuda:
+                    P64 = P64.cpu()                     # the rows live where A lives
             lb64 = ub64 = None
         else:
             if lower_bound is None or upper_bound is None:
@@ -343,8 +380,12 @@ class CCQPSolverBase(ABC):
         results = (_capi.Result * batch)()
         summary = _capi.Result()
         prm = self._params()
-        if convex_proj_op is not None:
-            blocks, params, _rows = convex_proj_op.descriptor()
+        if P64 is not None:
+            pp, _, _kp = _capi.f64_ptr(P64)
+            st = lib.ccqp_solve_batched_tables(h.h, self._solver_id, ctypes.byref(prm), batch, n, ptrs[0][0], ptrs[1][0],
+                                               ptrs[2][0], blocks.ptr, len(blocks), pp, int(P64.shape[1]), ptrs[5][0], K,
+                                               ptrs[6][0], mem, results, ctypes.byref(summary))
+        elif convex_proj_op is not None:
             pp, _, _kp = _capi.f64_ptr(params if params.size else np.zeros(1))
             st = lib.ccqp_solve_batched_table(h.h, self._solver_id, ctypes.byref(prm), batch, n, ptrs[0][0], ptrs[1][0],
                                               ptrs[2][0], blocks.ptr, len(blocks), pp, params.size, ptrs[5][0], K,

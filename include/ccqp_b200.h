@@ -240,6 +240,20 @@ ccqp_status ccqp_solve_batched_table(ccqp_handle* h, int solver, const ccqp_para
                                      int64_t n_params, const double* uniforms, int64_t n_uniforms, double* x_out,
                                      int memtype, ccqp_result* results, ccqp_result* summary);
 
+/* The same block STRUCTURE for all problems, each problem with its own parameter VALUES (bounds, radii, aspect ratios) --
+ * a batch of contact problems: k friction discs in every scene, disc radius mu * f_n of each contact.  Problem i equals
+ *     CCQPSolverX(tol,max_mv).solve(A[i], b[i], x0[i], op_i)
+ * where op_i is the table `blocks` (HOST pointer, shared) with the parameter array block_params + i * n_params: block_params
+ * is [batch][n_params], row i laid out as op_i's own parameter array, and lives where A lives (`memtype`: a device array is
+ * read in place, a host array is copied with the other inputs).  Argument checks as ccqp_solve_batched_table; n > 128:
+ * CCQP_ERR_UNSUPPORTED; all solvers except MPRGP (CCQP_ERR_UNSUPPORTED).  result.hbm_bytes counts the 8 * n_params bytes
+ * of each problem's row. */
+ccqp_status ccqp_solve_batched_tables(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch,
+                                      int64_t n, const double* A, const double* b, const double* x0,
+                                      const ccqp_block* blocks, int64_t n_blocks, const double* block_params,
+                                      int64_t n_params, const double* uniforms, int64_t n_uniforms, double* x_out,
+                                      int memtype, ccqp_result* results, ccqp_result* summary);
+
 /* ---- unit-test hooks for the pieces of the path ---------------------------------------------- */
 /* y = A v for the handle's row shard (y has n_rows entries).  A.dot(v), solvers.py:133 etc. */
 ccqp_status ccqp_gemv(ccqp_handle* h, const double* v, double* y, int memtype);
