@@ -24,8 +24,8 @@
 //     blocking needs 32 crossbar cycles for x plus 28 for the shuffles.  (A 4 x 16 blocking, 2-stage butterfly but 8 LDS.128
 //     per thread, measured slower and was removed in round 2.)
 //   * dot products: K <= 4 sums are reduced together with an exchange butterfly (6 SHFL.64 + 6 DADD for K = 3 instead of
-//     15 + 15), then the warps swap through shared memory (one barrier).  CCQP_BATCHED_DMMA=1 runs the 32-lane sums on the
-//     FP64 tensor path instead (measured equal, DESIGN.md 2.2).
+//     15 + 15), then the warps swap through shared memory (one barrier).  A variant that ran the 32-lane sums on the FP64
+//     tensor path measured equal and was removed (DESIGN.md 2.2).
 //   * stopping tests compare the SQUARED residual with a host-computed threshold that is exactly equivalent to the
 //     reference's sqrt(.) < tol (sqrt is monotone), so no sqrt is on the per-iteration critical path; the reported
 //     residual is computed once at the end.
@@ -37,21 +37,11 @@
 // Bounds: HBM bytes/problem = 8 n^2 + 32 n (+8 n for x0, + uniforms read by SPG);
 //         fp64 flops/problem = 2 n^2 * (mat-vecs executed).
 #pragma once
-#include <algorithm>
-#include <climits>
-#include <cstdlib>
 #include <cmath>
-#include <cstring>
-#include <functional>
-#include <string>
-#include <vector>
 
 #include "proj.cuh"
 #include "../../include/ccqp_b200.h"
 
-#ifndef CCQP_BATCHED_STAGE
-#define CCQP_BATCHED_STAGE 1    // 1: A reaches the registers through a TMA-filled shared tile (next problem in flight
-#endif                          //    during the solve); 0: straight from L2 (bulk L2 prefetch of the next problem)
 namespace ccqp {
 
 // Launch shape and layout of one problem.
@@ -126,17 +116,13 @@ struct BatchedCtx {
 
 template <bool GEN, int NT>
 struct BatchedSmem {
-#if CCQP_BATCHED_STAGE
     double tile[BL<NT>::N * BL<NT>::PITCH];   // the NEXT problem's A, landed by TMA while the current one iterates
     double vstage[3][BL<NT>::N];              // ... and its b / lower / upper bounds (general table: b / parameter row
                                               // of up to 2 N entries in vstage[1..2]) on the same mbarrier
-#endif
     double xs[2][BL<NT>::XS];                 // mat-vec input, double buffered
     double red[2][BL<NT>::WARPS][4];          // [parity][warp][slot]
     double pj[GEN ? 2 : 1][GEN ? BL<NT>::N : 2];   // general table: the vector being projected, for the members of norm blocks
-#if CCQP_BATCHED_STAGE
     uint64_t mbar;
-#endif
     int next;               // the problem after the next one (fetched during the solve of the current one)
     int first;              // prologue: this CTA's first problem
 };
@@ -167,14 +153,6 @@ __device__ __forceinline__ double shfl_xor_f64(double v, int mask) { return __sh
 // Sum K (<= 4) values over the 64 threads; result in every thread; ONE __syncthreads.
 // Exchange butterfly: after the first stages each lane carries ONE of the K sums, so the tree
 // costs max(K,2)+3 shuffles and adds instead of 5K.  Fixed order => deterministic.
-#ifndef CCQP_BATCHED_DMMA
-#define CCQP_BATCHED_DMMA 0     // 1: the 32-lane sums of cta64_sum run on the FP64 tensor path (2 DMMA.8x8x4 + 1 DADD per sum)
-#endif
-// D(8x8) = A(8x4) B(4x8) + C, FP64 (SASS DMMA.8x8x4): lane l holds A[l/4][l%4], B[l%4][l/4], C/D[l/4][2(l%4)], [2(l%4)+1]
-__device__ __forceinline__ void dmma884_ones(double& d0, double& d1, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%4,%5};"
-                 : "=d"(d0), "=d"(d1) : "d"(1.0), "d"(b), "d"(0.0), "d"(0.0));
-}
 
 // Cross-warp part of bsum: the warps' partial sums (red[parity][warp][slot]) are added in warp order
 template <int K, int NT>
@@ -219,29 +197,6 @@ __device__ __forceinline__ void bsum(double (&a)[K], const BShared& sh, int& par
 #pragma unroll
         for (int j = 0; j < K; ++j) a[j] = own ? a[j] : 0.0;
     }
-#if CCQP_BATCHED_DMMA
-    // With A = ones the first product leaves the sums of the 8 quads of lanes (a lane receives the two quads of ITS octet
-    // l%4), one add makes the octet sums, and the second product adds the four octets: the warp total in every lane.
-    // K independent chains, 2 DMMA + 1 DADD deep, against 5 dependent SHFL.64 + DADD stages; fixed order => deterministic.
-    {
-        double p[K], e0, e1;
-#pragma unroll
-        for (int j = 0; j < K; ++j) { dmma884_ones(e0, e1, a[j]); p[j] = e0 + e1; }
-#pragma unroll
-        for (int j = 0; j < K; ++j) { dmma884_ones(e0, e1, p[j]); p[j] = e0; }
-        const uint32_t base = sh.red + (uint32_t)parity * BL<NT>::RED_BYTES;
-        if (lane < K) {
-            double v = p[0];
-#pragma unroll
-            for (int j = 1; j < K; ++j) v = (lane == j) ? p[j] : v;
-            sts_f64(base + (uint32_t)(warp * 4 + lane) * 8u, v);
-        }
-        __syncthreads();
-        bsum_collect<K, NT>(a, base);
-        parity ^= 1;
-        return;
-    }
-#endif
     double v;
     int slot;            // which of the K sums this lane ends up carrying (lanes 0..3 are used)
     if constexpr (K == 1) {
@@ -674,11 +629,9 @@ __device__ __forceinline__ void solve_one(const BatchedCtx& c, const double (&a)
     o.status = status;
 }
 
-#ifndef CCQP_BATCHED_CTAS
-#define CCQP_BATCHED_CTAS 6     // resident CTAs per SM the register budget is cut for (6 -> 168 registers)
-#endif
+constexpr int kBatchedCtas = 6;         // resident CTAs per SM the register budget is cut for (6 -> 168 registers)
 constexpr int batched_min_ctas(int solver) {
-    return (solver == CCQP_SOLVER_PGD || solver == CCQP_SOLVER_BBPGD || solver == CCQP_SOLVER_SPG) ? CCQP_BATCHED_CTAS : 5;
+    return (solver == CCQP_SOLVER_PGD || solver == CCQP_SOLVER_BBPGD || solver == CCQP_SOLVER_SPG) ? kBatchedCtas : 5;
 }
 
 extern __shared__ __align__(16) unsigned char batched_dyn_smem[];       // NT = 256: the 141 KB of BatchedSmem are dynamic
@@ -706,7 +659,6 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
             asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(c.A + (size_t)prob * prob_elems),
                          "r"((unsigned)(prob_elems * 8)) : "memory");
     };
-#if CCQP_BATCHED_STAGE
     const bool staged = c.tma_ok != 0;
     const bool vstaged = staged && c.vtma_ok != 0;
     unsigned phase = 0;
@@ -731,17 +683,12 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
             }
         }
     };
-#else
-    const bool staged = false, vstaged = false;
-#endif
     // Work queue, two problems deep: `cur` is being solved, `nxt` is known (its A is in flight), and the index after that is
     // fetched by thread 0 at the start of a solve and published at its end -- the atomic's round trip hides behind the solve.
     if (t == 0) { sm.first = (int)atomicAdd(c.counter, 1u); sm.next = (int)atomicAdd(c.counter, 1u); }
     __syncthreads();
     int cur = sm.first;
-#if CCQP_BATCHED_STAGE
     if (staged && cur < c.batch) { fence_proxy_async(); issue_load(cur); }
-#endif
     while (cur < c.batch) {
         // ---- register fill: this thread's sub-block; register row r <- row row0 + (r ^ key) (see matvec)
         double a[kBRows][kBCols];
@@ -753,7 +700,6 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
         const size_t vo = (size_t)cur * n + u;
         const size_t bo = (size_t)cur * c.bound_stride + u;
         if (staged) {
-#if CCQP_BATCHED_STAGE
             mbar_wait(&sm.mbar, phase);
             phase ^= 1u;
             const uint32_t tb = smem_u32(sm.tile);
@@ -773,7 +719,6 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
                     s.hi = s.act ? sm.vstage[2][u] : 0.0;
                 }
             }
-#endif
         } else if (c.vec_ok) {
 #pragma unroll
             for (int r = 0; r < kBRows; ++r) {
@@ -810,9 +755,7 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
             const double* prow = c.params + (size_t)cur * c.param_stride;
             auto prm = [&](int k, double none) {
                 if (k < 0) return none;
-#if CCQP_BATCHED_STAGE
                 if (vstaged) return lds_f64(smem_u32(&sm.vstage[1][0]) + (uint32_t)k * 8u);   // the row runs on into vstage[2]
-#endif
                 return __ldg(prow + k);
             };
             const bool nb = s.kind == kElemNorm;
@@ -826,10 +769,8 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
         const int nxt = sm.next;               // thread 0 at the end of the previous solve) is visible
         unsigned after = 0;
         if (nxt < c.batch) {                   // the next problem travels while this one iterates
-#if CCQP_BATCHED_STAGE
-            if (staged) { fence_proxy_async(); issue_load(nxt); } else
-#endif
-            prefetch_l2(nxt);
+            if (staged) { fence_proxy_async(); issue_load(nxt); }
+            else prefetch_l2(nxt);
             if (c.x0 && s.own) asm volatile("prefetch.global.L2 [%0];" ::"l"(c.x0 + (size_t)nxt * n + u));
             if (t == 0) after = atomicAdd(c.counter, 1u);     // consumed at the end of the solve
         } else if (t == 0) after = (unsigned)c.batch;
@@ -844,248 +785,12 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
     }
 }
 
-// ------------------------------------------------------------------------------------------
-// host side
-// ------------------------------------------------------------------------------------------
-// Smallest double q >= 0 with pred(sqrt(q)) false ... expressed through the bit pattern: for
-// non-negative doubles the IEEE ordering equals the ordering of the bit patterns, and sqrt is
-// monotone and correctly rounded on both host and device, so the reference's test on sqrt(q)
-// is equivalent to a comparison of q with a threshold found by bisection.
-inline double sqrt_threshold(double tol, bool strict) {
-    // strict:  returns thr with  (q <  thr) <=> (sqrt(q) <  tol)
-    // !strict: returns thr with  (q <= thr) <=> (sqrt(q) <= tol)
-    if (tol != tol) return NAN;                                   // every comparison is false
-    auto holds = [&](unsigned long long bits) {
-        double q; std::memcpy(&q, &bits, 8);
-        const double r = std::sqrt(q);
-        return strict ? (r < tol) : (r <= tol);
-    };
-    const unsigned long long inf_bits = 0x7ff0000000000000ULL;
-    if (!holds(0)) return strict ? 0.0 : -1.0;                    // never true for q >= 0
-    if (holds(inf_bits)) return strict ? NAN : INFINITY;          // tol = +inf (strict: inf < inf is false, handled below)
-    unsigned long long lo = 0, hi = inf_bits;                     // holds(lo), !holds(hi)
-    while (hi - lo > 1) {
-        const unsigned long long mid = lo + (hi - lo) / 2;
-        if (holds(mid)) lo = mid; else hi = mid;
-    }
-    double out;
-    const unsigned long long pick = strict ? hi : lo;
-    std::memcpy(&out, &pick, 8);
-    return out;
-}
-
-#ifndef CCQP_BATCHED_DEVICE_ONLY        // batched_sym.cu shares the context / helpers above, not the launchers below
-template <int SOLVER, bool WREG, bool GEN, int NT>
-inline cudaError_t launch_batched_nt(const BatchedCtx& c, int sm_count, cudaStream_t stream) {
-    int per_sm = 0;
-    const size_t dyn = NT == 64 ? 0 : sizeof(BatchedSmem<GEN, NT>);
-    auto kern = batched_kernel<SOLVER, WREG, GEN, NT>;
-    cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    cudaError_t e = dyn ? cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn) : cudaSuccess;
-    if (e != cudaSuccess) return e;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, NT, dyn);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) per_sm = 1;
-    if (const char* e = getenv("CCQP_BATCHED_CTAS_PER_SM")) per_sm = std::max(1, std::min(per_sm, atoi(e)));   // tuning hook
-    long long grid = (long long)sm_count * per_sm;
-    if (grid > c.batch) grid = c.batch;
-    kern<<<(unsigned)grid, NT, dyn, stream>>>(c);
-    return cudaGetLastError();
-}
-// n <= 64: 64 threads per problem, A in 128 registers per thread, up to 6 problems per SM; 64 < n <= 128: 256 threads, one per SM
-template <int SOLVER, bool WREG, bool GEN = false>
-inline cudaError_t launch_batched(const BatchedCtx& c, int sm_count, cudaStream_t stream) {
-    return c.n <= kBN ? launch_batched_nt<SOLVER, WREG, GEN, 64>(c, sm_count, stream)
-                      : launch_batched_nt<SOLVER, WREG, GEN, 256>(c, sm_count, stream);
-}
-
-// The block structure of a general table, per element, on the HOST (batched.cu batched_table_layout), and where its
-// parameters are: one row shared by every problem (ccqp_solve_batched_table, a host array) or one row per problem
-// (ccqp_solve_batched_tables, [batch][n_params] where A lives)
-struct BatchedTable {
-    std::vector<uint8_t> ekind;
-    std::vector<int> eoff, edim, enk;
-    std::vector<int> eidx;          // [n][4]: lower bound / upper bound / block parameter index into a row, -1: none
-    int has_norm = 0;
-    const double* params = nullptr;
-    long long n_params = 0;
-    bool per_problem = false;
-};
+// batched.cu: launches a persistent batched kernel (batched_kernel / batched_sym_kernel, `threads` per CTA, `dyn` bytes of
+// dynamic shared memory) with as many CTAs as fit on the device, at most one per problem
+cudaError_t launch_persistent(const void* kern, int threads, size_t dyn, const BatchedCtx& c, int sm_count, cudaStream_t stream);
 
 // batched_sym.cu: the one-warp-per-problem kernels for symmetric Hessians (n <= 64; PGD / BBPGD / BBPGDf / SPG, Box per problem)
 bool batched_sym_supported(int solver, long long n);
 cudaError_t launch_batched_sym(const BatchedCtx& c, int solver, bool wreg, int sm_count, cudaStream_t stream);
-
-// Returns a ccqp_status.  `alloc(bytes)` returns a device workspace of at least that size.
-// tab != nullptr: the general table replaces the per-problem Box (lb / ub are ignored).
-// sym: the caller declares every A[i] symmetric (ccqp_solve_batched_sym); where batched_sym_supported() the upper block triangle
-// alone is read, otherwise the general kernels run (same answer for a symmetric A).
-inline int batched_solve(cudaStream_t stream, int sm_count, const BatchedTable* tab, bool sym, int solver, const ccqp_params& prm,
-                         long long batch, long long n, const double* A, const double* b, const double* x0,
-                         const double* lb, const double* ub, const double* uniforms, long long n_uniforms, double* x_out,
-                         int memtype, ccqp_result* results, ccqp_result* summary, cudaEvent_t ev0, cudaEvent_t ev1,
-                         int* launches, std::string& err, const std::function<void*(size_t)>& alloc) {
-#define BCU(call)                                                                                  \
-    do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { err = std::string(#call) + ": " + cudaGetErrorString(e__); return CCQP_ERR_CUDA; } } while (0)
-    if (n > kBNMax) return CCQP_ERR_UNSUPPORTED;
-    if (tab && solver == CCQP_SOLVER_MPRGP) return CCQP_ERR_UNSUPPORTED;     // batched MPRGP: Box per problem only
-    if (batch >= (1LL << 31) - 1024) return CCQP_ERR_INVALID_ARG;
-    const bool host = memtype == CCQP_MEM_HOST;
-    if (solver == CCQP_SOLVER_SPG && (n_uniforms < 0 || (n_uniforms > 0 && !uniforms))) return CCQP_ERR_INVALID_ARG;
-    const size_t szA = (size_t)batch * n * n * 8, szV = (size_t)batch * n * 8;
-    const size_t szU = (solver == CCQP_SOLVER_SPG) ? (size_t)batch * n_uniforms * 8 : 0;
-    const size_t szO = (size_t)batch * sizeof(BatchedOut);
-    auto al = [](size_t v) { return (v + 255) / 256 * 256; };
-    // parameter rows of a general table: a shared row and the rows of a host array are copied with an even pitch, so that
-    // every row starts 16-byte aligned and its bulk copy (rounded up to 16 bytes) stays inside the copy
-    const long long np = tab ? std::max(tab->n_params, 0LL) : 0, ppitch = np + (np & 1);
-    const size_t szP = !tab ? 0 : !tab->per_problem ? (size_t)ppitch * 8 : host ? (size_t)batch * ppitch * 8 : 0;
-    size_t total = 256 + al(szO) + 8 * al((size_t)kBNMax * 8) + al(szP);
-    if (host) total += al(szA) + 4 * al(szV) + al(szV) + al(szU);
-    unsigned char* ws = static_cast<unsigned char*>(alloc(total));
-    if (!ws) { err = "workspace allocation failed"; return CCQP_ERR_CUDA; }
-    size_t off = 0;
-    auto take = [&](size_t bytes) { unsigned char* p = ws + off; off += al(bytes); return p; };
-    unsigned* counter = reinterpret_cast<unsigned*>(take(256));
-    BatchedOut* dout = reinterpret_cast<BatchedOut*>(take(szO));
-    BatchedCtx c;
-    std::memset(&c, 0, sizeof(c));
-    if (host) {
-        double* dA = reinterpret_cast<double*>(take(szA));
-        double* db = reinterpret_cast<double*>(take(szV));
-        double* dlb = reinterpret_cast<double*>(take(szV));
-        double* dub = reinterpret_cast<double*>(take(szV));
-        double* dx0 = reinterpret_cast<double*>(take(szV));
-        double* dxo = reinterpret_cast<double*>(take(szV));
-        double* du = szU ? reinterpret_cast<double*>(take(szU)) : nullptr;
-        BCU(cudaMemcpyAsync(dA, A, szA, cudaMemcpyHostToDevice, stream));
-        BCU(cudaMemcpyAsync(db, b, szV, cudaMemcpyHostToDevice, stream));
-        if (!tab) BCU(cudaMemcpyAsync(dlb, lb, szV, cudaMemcpyHostToDevice, stream));
-        if (!tab) BCU(cudaMemcpyAsync(dub, ub, szV, cudaMemcpyHostToDevice, stream));
-        if (x0) BCU(cudaMemcpyAsync(dx0, x0, szV, cudaMemcpyHostToDevice, stream));
-        if (du) BCU(cudaMemcpyAsync(du, uniforms, szU, cudaMemcpyHostToDevice, stream));
-        c.A = dA; c.b = db; c.lb = dlb; c.ub = dub; c.x0 = x0 ? dx0 : nullptr; c.uniforms = du; c.x_out = dxo;
-    } else {
-        c.A = A; c.b = b; c.lb = lb; c.ub = ub; c.x0 = x0; c.uniforms = (solver == CCQP_SOLVER_SPG) ? uniforms : nullptr;
-        c.x_out = x_out;
-    }
-    c.bound_stride = n;
-    if (tab) {        // the block structure: five small per-element arrays, uploaded once per call
-        auto up = [&](const void* src, size_t bytes) -> void* {
-            void* d = take(bytes);
-            return cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, stream) == cudaSuccess ? d : nullptr;
-        };
-        c.ekind = static_cast<const uint8_t*>(up(tab->ekind.data(), (size_t)n));
-        c.eoff = static_cast<const int*>(up(tab->eoff.data(), (size_t)n * 4));
-        c.edim = static_cast<const int*>(up(tab->edim.data(), (size_t)n * 4));
-        c.enk = static_cast<const int*>(up(tab->enk.data(), (size_t)n * 4));
-        c.eidx = static_cast<const int4*>(up(tab->eidx.data(), (size_t)n * 16));
-        if (!c.ekind || !c.eoff || !c.edim || !c.enk || !c.eidx) { err = "table upload failed"; return CCQP_ERR_CUDA; }
-        c.has_norm = tab->has_norm;
-        c.lb = c.ub = nullptr;
-        // the parameter rows: one shared row (stride 0), a host array copied with an even pitch, or a device array in place
-        if (np > 0 && (!tab->per_problem || host)) {
-            double* dp = reinterpret_cast<double*>(take(szP));
-            const long long rows = tab->per_problem ? batch : 1;
-            if (ppitch == np) BCU(cudaMemcpyAsync(dp, tab->params, (size_t)rows * np * 8, cudaMemcpyHostToDevice, stream));
-            else BCU(cudaMemcpy2DAsync(dp, (size_t)ppitch * 8, tab->params, (size_t)np * 8, (size_t)np * 8, (size_t)rows,
-                                       cudaMemcpyHostToDevice, stream));
-            c.params = dp;
-            c.param_stride = tab->per_problem ? ppitch : 0;
-        } else {
-            c.params = np > 0 ? tab->params : nullptr;
-            c.param_stride = np;
-        }
-    }
-    c.n_uniforms = (solver == CCQP_SOLVER_SPG) ? n_uniforms : 0;
-    c.out = dout; c.counter = counter;
-    c.batch = (int)batch; c.n = (int)n;
-    c.tma_ok = ((n * 8) % 16 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 15) == 0) ? 1 : 0;
-    c.vec_ok = (n % 4 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 31) == 0) ? 1 : 0;
-    c.pf_ok = ((n * n * 8) % 16 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 15) == 0) ? 1 : 0;
-    c.vtma_ok = (n % 2 == 0 && ((reinterpret_cast<uintptr_t>(c.b) | reinterpret_cast<uintptr_t>(c.lb) | reinterpret_cast<uintptr_t>(c.ub)) & 15) == 0) ? 1 : 0;
-    if (tab) {        // a parameter row is staged with b when every row is 16-byte aligned and fits vstage[1..2] (2 N doubles)
-        const long long N = n <= kBN ? kBN : kBNMax;
-        const bool rows_ok = np == 0 || (c.param_stride % 2 == 0 && (reinterpret_cast<uintptr_t>(c.params) & 15) == 0 && ppitch <= 2 * N);
-        c.vtma_ok = (c.vtma_ok && rows_ok) ? 1 : 0;
-        c.prow_bytes = c.vtma_ok ? (int)(ppitch * 8) : 0;
-    }
-    c.tol = prm.tol; c.max_mv = prm.max_mv; c.step = prm.step_size;
-    c.tau = prm.tau; c.sig1 = prm.sigma1; c.sig2 = prm.sigma2; c.m = prm.m;
-    c.thr_lt = sqrt_threshold(prm.tol, true);
-    c.thr_le = sqrt_threshold(prm.tol, false);
-    c.max_mv_i = (prm.max_mv != prm.max_mv || prm.max_mv >= 2147483000.0) ? INT_MAX
-                 : (prm.max_mv <= -2147483000.0 ? INT_MIN : (int)std::ceil(prm.max_mv));
-    BCU(cudaMemsetAsync(counter, 0, 256, stream));
-    BCU(cudaEventRecord(ev0, stream));
-    cudaError_t le;
-    const bool wreg = prm.m == kBWinReg;
-    const bool use_sym = sym && !tab && batched_sym_supported(solver, n);
-    if (use_sym) le = launch_batched_sym(c, solver, wreg, sm_count, stream);
-    else if (tab) switch (solver) {
-        case CCQP_SOLVER_PGD: le = launch_batched<CCQP_SOLVER_PGD, true, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_APGD: le = launch_batched<CCQP_SOLVER_APGD, true, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_APGD_AR: le = launch_batched<CCQP_SOLVER_APGD_AR, true, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_BBPGD: le = launch_batched<CCQP_SOLVER_BBPGD, true, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_BBPGDF: le = launch_batched<CCQP_SOLVER_BBPGDF, true, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_SPG:
-            le = wreg ? launch_batched<CCQP_SOLVER_SPG, true, true>(c, sm_count, stream)
-                      : launch_batched<CCQP_SOLVER_SPG, false, true>(c, sm_count, stream);
-            break;
-        default: return CCQP_ERR_INVALID_ARG;
-    }
-    else switch (solver) {
-        case CCQP_SOLVER_PGD: le = launch_batched<CCQP_SOLVER_PGD, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_APGD: le = launch_batched<CCQP_SOLVER_APGD, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_APGD_AR: le = launch_batched<CCQP_SOLVER_APGD_AR, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_BBPGD: le = launch_batched<CCQP_SOLVER_BBPGD, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_BBPGDF: le = launch_batched<CCQP_SOLVER_BBPGDF, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_MPRGP: le = launch_batched<CCQP_SOLVER_MPRGP, true>(c, sm_count, stream); break;
-        case CCQP_SOLVER_SPG:
-            le = wreg ? launch_batched<CCQP_SOLVER_SPG, true>(c, sm_count, stream)
-                      : launch_batched<CCQP_SOLVER_SPG, false>(c, sm_count, stream);
-            break;
-        default: return CCQP_ERR_INVALID_ARG;
-    }
-    BCU(le);
-    *launches = 1;
-    BCU(cudaEventRecord(ev1, stream));
-    if (host) BCU(cudaMemcpyAsync(x_out, c.x_out, szV, cudaMemcpyDeviceToHost, stream));
-    std::vector<BatchedOut> hout((size_t)batch);
-    BCU(cudaMemcpyAsync(hout.data(), dout, szO, cudaMemcpyDeviceToHost, stream));
-    BCU(cudaStreamSynchronize(stream));
-    float ms = 0.f;
-    BCU(cudaEventElapsedTime(&ms, ev0, ev1));
-    long long tot_mv = 0, tot_gemv = 0, tot_it = 0, tot_dr = 0, nconv = 0;
-    int first_status = 0;
-    double hbmA = 8.0 * n * n;                  // bytes of A[i] the kernel reads
-    if (use_sym) { hbmA = 0; for (long long i = 0; i < n; ++i) hbmA += 8.0 * (double)(n - 8 * (i / 8)); }
-    if (tab && tab->per_problem) hbmA += 8.0 * (double)np;     // the problem's parameter row
-    for (long long i = 0; i < batch; ++i) {
-        const BatchedOut& o = hout[(size_t)i];
-        if (results) {
-            ccqp_result& r = results[i];
-            std::memset(&r, 0, sizeof(r));
-            r.residual = o.residual; r.mv_count = o.mv; r.gemv_count = o.gemv; r.iterations = o.iters;
-            r.uniforms_used = o.draws; r.converged = o.converged; r.status = o.status;
-            r.hbm_bytes = hbmA + 8.0 * n * (x0 ? 5 : 4);
-        }
-        tot_mv += o.mv; tot_gemv += o.gemv; tot_it += o.iters; tot_dr += o.draws; nconv += o.converged;
-        if (o.status && !first_status) first_status = o.status;
-    }
-    if (summary) {
-        std::memset(summary, 0, sizeof(*summary));
-        summary->gpu_seconds = ms * 1e-3;
-        summary->mv_count = tot_mv; summary->gemv_count = tot_gemv; summary->iterations = tot_it;
-        summary->uniforms_used = tot_dr; summary->converged = (nconv == batch) ? 1 : 0;
-        summary->status = first_status;
-        summary->hbm_bytes = (double)batch * (hbmA + 8.0 * n * (x0 ? 5 : 4)) + 8.0 * (double)tot_dr;
-        summary->kernel_launches = 1;
-        summary->residual = NAN;
-    }
-    return CCQP_OK;
-#undef BCU
-}
-#endif  // CCQP_BATCHED_DEVICE_ONLY
 
 }  // namespace ccqp

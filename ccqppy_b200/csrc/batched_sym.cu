@@ -31,9 +31,7 @@
 // over two sub-partitions.  The DFMA count per problem is the same in both layouts, so is their operand traffic; what the
 // symmetric layout buys is register space (and half of the HBM reads), what it costs is the exchange through shared memory.
 // Hence: an opt-in for callers whose solver is SPG (or whose batch is HBM- or capacity-bound), not the default.
-#define CCQP_BATCHED_DEVICE_ONLY
 #include "batched.cuh"
-#include "internal.h"
 
 namespace ccqp {
 namespace bsym {
@@ -483,21 +481,6 @@ __global__ void __launch_bounds__(32, kCtas) batched_sym_kernel(const BatchedCtx
     }
 }
 
-template <int SOLVER, bool WREG>
-cudaError_t launch(const BatchedCtx& c, int sm_count, cudaStream_t stream) {
-    auto kern = batched_sym_kernel<SOLVER, WREG>;
-    cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    int per_sm = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 32, 0);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) per_sm = 1;
-    if (const char* ev = getenv("CCQP_BATCHED_CTAS_PER_SM")) per_sm = std::max(1, std::min(per_sm, atoi(ev)));   // tuning hook
-    long long grid = (long long)sm_count * per_sm;
-    if (grid > c.batch) grid = c.batch;
-    kern<<<(unsigned)grid, 32, 0, stream>>>(c);
-    return cudaGetLastError();
-}
-
 }  // namespace bsym
 
 bool batched_sym_supported(int solver, long long n) {
@@ -506,15 +489,18 @@ bool batched_sym_supported(int solver, long long n) {
 }
 
 cudaError_t launch_batched_sym(const BatchedCtx& c, int solver, bool wreg, int sm_count, cudaStream_t stream) {
+    const void* kern;
     switch (solver) {
-        case CCQP_SOLVER_PGD: return bsym::launch<CCQP_SOLVER_PGD, true>(c, sm_count, stream);
-        case CCQP_SOLVER_BBPGD: return bsym::launch<CCQP_SOLVER_BBPGD, true>(c, sm_count, stream);
-        case CCQP_SOLVER_BBPGDF: return bsym::launch<CCQP_SOLVER_BBPGDF, true>(c, sm_count, stream);
+        case CCQP_SOLVER_PGD: kern = (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_PGD, true>; break;
+        case CCQP_SOLVER_BBPGD: kern = (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_BBPGD, true>; break;
+        case CCQP_SOLVER_BBPGDF: kern = (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_BBPGDF, true>; break;
         case CCQP_SOLVER_SPG:
-            return wreg ? bsym::launch<CCQP_SOLVER_SPG, true>(c, sm_count, stream)
-                        : bsym::launch<CCQP_SOLVER_SPG, false>(c, sm_count, stream);
+            kern = wreg ? (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_SPG, true>
+                        : (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_SPG, false>;
+            break;
         default: return cudaErrorInvalidValue;
     }
+    return launch_persistent(kern, 32, 0, c, sm_count, stream);
 }
 
 }  // namespace ccqp

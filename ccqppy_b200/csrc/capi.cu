@@ -19,21 +19,6 @@
 
 using namespace ccqp;
 
-struct DevBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-    cudaError_t ensure(size_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
-        cudaError_t e = cudaMalloc(&p, bytes);
-        if (e == cudaSuccess) cap = bytes;
-        return e;
-    }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
-    template <class T> T* as() const { return reinterpret_cast<T*>(p); }
-};
-
 struct ccqp_handle {
     int device = 0;
     int sm_count = 0;
@@ -350,6 +335,25 @@ bool params_ok(const ccqp_params* p, int solver) {
 
 }  // namespace
 
+long long ccqp::block_param_count(int kind, long long dim) {
+    return kind == CCQP_BLOCK_IDENTITY ? 0 : kind == CCQP_BLOCK_BOX ? 2 * dim
+           : (kind == CCQP_BLOCK_LOWER || kind == CCQP_BLOCK_UPPER) ? dim : 1;
+}
+
+long long ccqp::block_table_unknowns(const ccqp_block* blocks, long long n_blocks, long long n_params) {
+    long long n = 0;
+    for (long long k = 0; k < n_blocks; ++k) {
+        const ccqp_block& b = blocks[k];
+        // written so that nothing overflows: n stays <= LLONG_MAX / 2 (so does 2 dim), and param_off <= n_params is
+        // tested before n_params - param_off is formed
+        if (b.offset != n || b.dim <= 0 || b.dim > LLONG_MAX / 2 - n || b.kind < 0 || b.kind > CCQP_BLOCK_SOC ||
+            b.param_off < 0 || b.param_off > n_params || block_param_count(b.kind, b.dim) > n_params - b.param_off)
+            return -1;
+        n += b.dim;
+    }
+    return n;
+}
+
 extern "C" {
 
 int ccqp_abi_version(void) { return CCQP_ABI_VERSION; }
@@ -522,16 +526,8 @@ ccqp_status ccqp_set_projection(ccqp_handle* h, const ccqp_block* blocks, int64_
                                 int64_t n_params) {
     if (!h || !blocks || n_blocks <= 0 || (n_params > 0 && !params)) return CCQP_ERR_INVALID_ARG;
     CU(h, cudaSetDevice(h->device));
-    long long n = 0;
-    for (int64_t k = 0; k < n_blocks; ++k) {
-        const ccqp_block& b = blocks[k];
-        if (b.offset != n || b.dim <= 0 || b.kind < 0 || b.kind > CCQP_BLOCK_SOC || b.param_off < 0) return CCQP_ERR_INVALID_ARG;
-        const long long need = (b.kind == CCQP_BLOCK_IDENTITY) ? 0 : (b.kind == CCQP_BLOCK_BOX) ? 2 * b.dim
-                               : (b.kind == CCQP_BLOCK_LOWER || b.kind == CCQP_BLOCK_UPPER) ? b.dim : 1;
-        if (b.param_off + need > n_params) return CCQP_ERR_INVALID_ARG;
-        n += b.dim;
-    }
-    if (n >= (1LL << 31) - 256) return CCQP_ERR_INVALID_ARG;
+    const long long n = block_table_unknowns(blocks, n_blocks, n_params);
+    if (n < 0 || n >= (1LL << 31) - 256) return CCQP_ERR_INVALID_ARG;
     const long long npad = round_up(n, 64) + 64;
     const double inf = std::numeric_limits<double>::infinity();
     std::vector<double> lo(npad, -inf), hi(npad, inf), bpar(n_blocks, 0.0);
@@ -814,72 +810,47 @@ ccqp_status ccqp_projected_gradient(ccqp_handle* h, const double* x, const doubl
     return CCQP_OK;
 }
 
-static ccqp_status solve_batched_box(ccqp_handle* h, bool symmetric, int solver, const ccqp_params* params, int64_t batch, int64_t n,
-                               const double* A, const double* b, const double* x0, const double* lb, const double* ub,
-                               const double* uniforms, int64_t n_uniforms, double* x_out, int memtype,
-                               ccqp_result* results, ccqp_result* summary) {
-    if (!h || !params_ok(params, solver) || batch <= 0 || n <= 0 || !A || !b || !lb || !ub || !x_out)
+// Every batched call: the checks of its arguments, then batched.cu.
+static ccqp_status solve_batched(ccqp_handle* h, const BatchedRequest& r) {
+    const bool box = r.set == BatchedSet::kBox;
+    if (!h || !params_ok(r.params, r.solver) || r.batch <= 0 || r.n <= 0 || !r.A || !r.b || !r.x_out ||
+        (box ? (!r.lb || !r.ub)
+             : (!r.blocks || r.n_blocks <= 0 || (r.n_params > 0 && !r.block_params) || (r.set == BatchedSet::kTables && r.n_params < 0))))
         return CCQP_ERR_INVALID_ARG;
     CU(h, cudaSetDevice(h->device));
-    std::string err;
-    int launches = 0;
-    ccqp_status st = (ccqp_status)batched_solve_entry(h->stream, h->sm_count, solver, *params,
-                                                batch, n, A, b, x0, lb, ub, uniforms, n_uniforms, x_out, memtype, results,
-                                                summary, h->ev0, h->ev1, &launches, err,
-                                                [&](size_t bytes) -> void* { return h->batched_ws.ensure(bytes) == cudaSuccess ? h->batched_ws.p : nullptr; },
-                                                symmetric);
-    h->launches += launches;
-    if (st == CCQP_ERR_CUDA) h->last_error = err;
-    return st;
+    return (ccqp_status)batched_solve(r, h->stream, h->sm_count, h->ev0, h->ev1, h->batched_ws, h->launches, h->last_error);
 }
 
 ccqp_status ccqp_solve_batched(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
                                const double* A, const double* b, const double* x0, const double* lb, const double* ub,
                                const double* uniforms, int64_t n_uniforms, double* x_out, int memtype,
                                ccqp_result* results, ccqp_result* summary) {
-    return solve_batched_box(h, false, solver, params, batch, n, A, b, x0, lb, ub, uniforms, n_uniforms, x_out, memtype, results, summary);
+    return solve_batched(h, {solver, params, batch, n, A, b, x0, uniforms, n_uniforms, x_out, memtype, results, summary,
+                             BatchedSet::kBox, lb, ub, false});
 }
 
 ccqp_status ccqp_solve_batched_sym(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
                                    const double* A, const double* b, const double* x0, const double* lb, const double* ub,
                                    const double* uniforms, int64_t n_uniforms, double* x_out, int memtype,
                                    ccqp_result* results, ccqp_result* summary) {
-    return solve_batched_box(h, true, solver, params, batch, n, A, b, x0, lb, ub, uniforms, n_uniforms, x_out, memtype, results, summary);
-}
-
-static ccqp_status solve_batched_tab(ccqp_handle* h, bool per_problem, int solver, const ccqp_params* params, int64_t batch,
-                                     int64_t n, const double* A, const double* b, const double* x0, const ccqp_block* blocks,
-                                     int64_t n_blocks, const double* block_params, int64_t n_params, const double* uniforms,
-                                     int64_t n_uniforms, double* x_out, int memtype, ccqp_result* results, ccqp_result* summary) {
-    if (!h || !params_ok(params, solver) || batch <= 0 || n <= 0 || !A || !b || !x_out || !blocks || n_blocks <= 0 ||
-        (n_params > 0 && !block_params) || (per_problem && n_params < 0))
-        return CCQP_ERR_INVALID_ARG;
-    CU(h, cudaSetDevice(h->device));
-    std::string err;
-    int launches = 0;
-    ccqp_status st = (ccqp_status)batched_solve_table_entry(h->stream, h->sm_count, solver, *params, batch, n, A, b, x0, blocks, n_blocks,
-                                                            block_params, n_params, per_problem, uniforms, n_uniforms, x_out, memtype,
-                                                            results, summary, h->ev0, h->ev1, &launches, err,
-                                                            [&](size_t bytes) -> void* { return h->batched_ws.ensure(bytes) == cudaSuccess ? h->batched_ws.p : nullptr; });
-    h->launches += launches;
-    if (st == CCQP_ERR_CUDA) h->last_error = err;
-    return st;
+    return solve_batched(h, {solver, params, batch, n, A, b, x0, uniforms, n_uniforms, x_out, memtype, results, summary,
+                             BatchedSet::kBox, lb, ub, true});
 }
 
 ccqp_status ccqp_solve_batched_table(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
                                      const double* A, const double* b, const double* x0, const ccqp_block* blocks, int64_t n_blocks,
                                      const double* block_params, int64_t n_params, const double* uniforms, int64_t n_uniforms,
                                      double* x_out, int memtype, ccqp_result* results, ccqp_result* summary) {
-    return solve_batched_tab(h, false, solver, params, batch, n, A, b, x0, blocks, n_blocks, block_params, n_params, uniforms,
-                             n_uniforms, x_out, memtype, results, summary);
+    return solve_batched(h, {solver, params, batch, n, A, b, x0, uniforms, n_uniforms, x_out, memtype, results, summary,
+                             BatchedSet::kTable, nullptr, nullptr, false, blocks, n_blocks, block_params, n_params});
 }
 
 ccqp_status ccqp_solve_batched_tables(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
                                       const double* A, const double* b, const double* x0, const ccqp_block* blocks, int64_t n_blocks,
                                       const double* block_params, int64_t n_params, const double* uniforms, int64_t n_uniforms,
                                       double* x_out, int memtype, ccqp_result* results, ccqp_result* summary) {
-    return solve_batched_tab(h, true, solver, params, batch, n, A, b, x0, blocks, n_blocks, block_params, n_params, uniforms,
-                             n_uniforms, x_out, memtype, results, summary);
+    return solve_batched(h, {solver, params, batch, n, A, b, x0, uniforms, n_uniforms, x_out, memtype, results, summary,
+                             BatchedSet::kTables, nullptr, nullptr, false, blocks, n_blocks, block_params, n_params});
 }
 
 namespace {

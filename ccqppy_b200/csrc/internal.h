@@ -1,12 +1,11 @@
-// Entry points between the translation units of libccqp_b200.so: capi.cu (C-ABI, host code), batched.cu + batched_sym.cu
-// (batched kernels), upload.cu (host -> device matrix copies), and the four compilations of the dense solver kernels, one
+// Entry points between the translation units of libccqp_b200.so: capi.cu (C-ABI, host code), batched.cu (batched kernels
+// and the host side of every batched call) + batched_sym.cu (batched kernels for symmetric Hessians), upload.cu (host -> device matrix copies), and the four compilations of the dense solver kernels, one
 // unit each because each sees dense.cuh with different macros: dense_f64.cu (fp64 Hessians), dense_f32.cu (fp32-stored
 // Hessians), csr.cu (CSR Hessians), emu.cu (emulated ranks, a test vehicle).  The rest are separate units only so that
 // they compile in parallel.
 #pragma once
 #include <cuda_runtime.h>
 
-#include <functional>
 #include <string>
 
 #include "../../include/ccqp_b200.h"
@@ -15,22 +14,66 @@ namespace ccqp {
 
 struct DenseCtx;
 
-// batched.cu (+ batched_sym.cu: the kernels behind `symmetric`) -- returns a ccqp_status; `alloc(bytes)` returns a device workspace of at least that size
-int batched_solve_entry(cudaStream_t stream, int sm_count, int solver, const ccqp_params& prm, long long batch, long long n,
-                        const double* A, const double* b, const double* x0, const double* lb, const double* ub,
-                        const double* uniforms, long long n_uniforms, double* x_out, int memtype, ccqp_result* results,
-                        ccqp_result* summary, cudaEvent_t ev0, cudaEvent_t ev1, int* launches, std::string& err,
-                        const std::function<void*(size_t)>& alloc, bool symmetric = false);
+// A device buffer that only grows: the handle's workspaces (capi.cu, batched.cu).
+struct DevBuf {
+    void* p = nullptr;
+    size_t cap = 0;
+    cudaError_t ensure(size_t bytes) {
+        if (bytes <= cap) return cudaSuccess;
+        if (p) cudaFree(p);
+        p = nullptr; cap = 0;
+        cudaError_t e = cudaMalloc(&p, bytes);
+        if (e == cudaSuccess) cap = bytes;
+        return e;
+    }
+    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+    template <class T> T* as() const { return reinterpret_cast<T*>(p); }
+};
 
-// the same with a projection table (any block kinds) instead of a Box per problem: the block structure is shared by all
-// problems of the batch; per_problem = false: ONE host parameter array `params` for all of them, true: params is
-// [batch][n_params] in `memtype` memory, row i for problem i
-int batched_solve_table_entry(cudaStream_t stream, int sm_count, int solver, const ccqp_params& prm, long long batch, long long n,
-                              const double* A, const double* b, const double* x0, const ccqp_block* blocks, long long n_blocks,
-                              const double* params, long long n_params, bool per_problem, const double* uniforms,
-                              long long n_uniforms, double* x_out, int memtype, ccqp_result* results, ccqp_result* summary,
-                              cudaEvent_t ev0, cudaEvent_t ev1, int* launches, std::string& err,
-                              const std::function<void*(size_t)>& alloc);
+// capi.cu -- the one check of a block table (ccqp_set_projection, batched tables): the blocks tile [0, n) in order from 0,
+// every dim > 0, every kind a ccqp_block_kind, param_off >= 0 and param_off + block_param_count() <= n_params, all of it
+// without overflow for any 64-bit input (n itself stays <= LLONG_MAX / 2).  Returns n, or -1 for a malformed table.
+long long block_table_unknowns(const ccqp_block* blocks, long long n_blocks, long long n_params);
+long long block_param_count(int kind, long long dim);      // parameters a block takes from params[param_off ..]
+
+// One batched call: problem i is solve(A[i], b[i], x0[i], op_i) for i < batch, each of n <= 128 unknowns.
+enum class BatchedSet {
+    kBox,           // Box per problem: lb[i] / ub[i] (ccqp_solve_batched, ccqp_solve_batched_sym)
+    kTable,         // one block table for every problem, parameters one host array (ccqp_solve_batched_table)
+    kTables,        // one block structure, row i of block_params [batch][n_params] for problem i (ccqp_solve_batched_tables)
+};
+// capi.cu fills it by aggregate initialisation in this field order: a field is never moved, only appended.
+struct BatchedRequest {
+    int solver;
+    const ccqp_params* params;
+    long long batch, n;
+    const double* A;                // [batch][n][n]
+    const double* b;                // [batch][n]
+    const double* x0;               // [batch][n] or null
+    const double* uniforms;         // SPG: [batch][n_uniforms]
+    long long n_uniforms;
+    double* x_out;                  // [batch][n]
+    int memtype;                    // where every array above, lb / ub and kTables' block_params live
+    ccqp_result* results;           // [batch] or null
+    ccqp_result* summary;           // or null
+    BatchedSet set;
+    // kBox
+    const double* lb;               // [batch][n]
+    const double* ub;
+    bool symmetric;                 // the caller declares every A[i] symmetric: where batched_sym_supported() (batched.cuh)
+                                    // only the upper block triangle is read, otherwise the general kernels run
+    // kTable / kTables
+    const ccqp_block* blocks;
+    long long n_blocks;
+    const double* block_params;
+    long long n_params;
+};
+
+// batched.cu (+ batched_sym.cu: the kernels behind `symmetric`) -- the request's arguments are checked for null and
+// size already; returns a ccqp_status, adds the kernels it launched to `launches` and, for CCQP_ERR_CUDA, names the failed
+// call in `err`.  `ws` is the device workspace, grown as needed.
+int batched_solve(const BatchedRequest& r, cudaStream_t stream, int sm_count, cudaEvent_t ev0, cudaEvent_t ev1, DevBuf& ws,
+                  long long& launches, std::string& err);
 
 // upload.cu -- host -> device copy of a square matrix; a symmetric one crosses PCIe as its upper block triangle (checked on the host
 // while the copies run) and is mirrored on the device: the device copy is bit-identical to a full upload either way

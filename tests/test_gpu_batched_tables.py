@@ -247,19 +247,37 @@ def test_capi_errors():
     res = (_capi.Result * batch)()
     summ = _capi.Result()
 
-    def call(blocks, params, n_params, solver=_capi.BBPGD, nn=n, AA=A, bb=b, xx=x):
-        return lib.ccqp_solve_batched_tables(h.h, solver, ctypes.byref(prm), batch, nn, P(AA), P(bb), None, blocks.ptr,
-                                             len(blocks), params, n_params, None, 0, P(xx), _capi.MEM_HOST, res,
-                                             ctypes.byref(summ))
-    good = _capi.make_blocks([(_capi.SPHERE, 0, 3, 0), (_capi.SPHERE, 3, 3, 1), (_capi.SPHERE, 6, 3, 2)])
+    def call(blocks, params, n_params, solver=_capi.BBPGD, nn=n, AA=A, bb=b, xx=x, entry=lib.ccqp_solve_batched_tables):
+        return entry(h.h, solver, ctypes.byref(prm), batch, nn, P(AA), P(bb), None, blocks.ptr, len(blocks), params, n_params,
+                     None, 0, P(xx), _capi.MEM_HOST, res, ctypes.byref(summ))
+    S, I31, I64 = _capi.SPHERE, 2**31 - 1, 2**63 - 1
+    good = _capi.make_blocks([(S, 0, 3, 0), (S, 3, 3, 1), (S, 6, 3, 2)])
     assert call(good, P(par), 3) == 0 and summ.converged == 1
     assert call(good, None, 3) == 1                                                        # null block_params
-    assert call(good, P(par), 2) == 1                                                      # a block overruns n_params
-    assert call(_capi.make_blocks([(_capi.SPHERE, 0, 3, 0), (_capi.SPHERE, 3, 3, 1)]), P(par), 3) == 1    # [0, 6) only
-    assert call(_capi.make_blocks([(_capi.SPHERE, 0, 3, 0), (_capi.SPHERE, 4, 3, 1), (_capi.SPHERE, 7, 2, 2)]),
-                P(par), 3) == 1                                                            # a gap at 3
+    assert call(_capi.make_blocks([(S, 0, 3, 0), (S, 3, 3, 1)]), P(par), 3) == 1          # [0, 6) only
+    # a table malformed by itself: the same code from the projection of a handle and from both batched table entries
+    malformed = {"a block overruns n_params": ([(S, 0, 3, 0), (S, 3, 3, 1), (S, 6, 3, 2)], 2),
+                 "a gap at 3": ([(S, 0, 3, 0), (S, 4, 3, 1), (S, 7, 2, 2)], 3),
+                 "unknown kind": ([(S, 0, 3, 0), (S, 3, 3, 1), (99, 6, 3, 2)], 3),
+                 "zero dim": ([(S, 0, 3, 0), (S, 3, 0, 1), (S, 3, 6, 2)], 3),
+                 "negative param_off": ([(S, 0, 3, 0), (S, 3, 3, -1), (S, 6, 3, 2)], 3),
+                 # 64-bit wrap-around: the dims sum to 9 modulo 2^64, a parameter range ends past INT64_MAX
+                 "n wraps around": ([(_capi.LOWER, 0, I31, 0), (_capi.IDENTITY, I31, I64 - I31, 0), (_capi.IDENTITY, I64, 1, 0),
+                                     (_capi.IDENTITY, -I64 - 1, I64, 0), (_capi.IDENTITY, -1, 10, 0)], I31 + 1),
+                 "param_off + need wraps around": ([(S, 0, 3, 0), (S, 3, 3, 1), (S, 6, 3, I64)], 3)}
+    for what, (rows, n_params) in malformed.items():
+        bad = _capi.make_blocks(rows)
+        codes = (lib.ccqp_set_projection(h.h, bad.ptr, len(bad), P(par), n_params),
+                 call(bad, P(par), n_params, entry=lib.ccqp_solve_batched_table), call(bad, P(par), n_params))
+        assert codes == (1, 1, 1), (what, codes)
+        for entry in (lib.ccqp_solve_batched_table, lib.ccqp_solve_batched_tables):      # malformed wins over MPRGP
+            assert call(bad, P(par), n_params, solver=_capi.MPRGP, entry=entry) == 1, what
     assert call(good, P(par), 3, solver=_capi.MPRGP) == 4                                  # MPRGP: unsupported
     big, vb = np.zeros((batch, 129, 129)), np.zeros((batch, 129))
-    wide = _capi.make_blocks([(_capi.SPHERE, 0, 129, 0)])
+    wide = _capi.make_blocks([(S, 0, 129, 0)])
     assert call(wide, P(par), 3, nn=129, AA=big, bb=vb, xx=vb) == 4                       # n > 128
+    assert call(wide, P(par), 3, solver=99, nn=129, AA=big, bb=vb, xx=vb) == 4            # ... wins over an unknown solver
+    assert lib.ccqp_solve_batched(h.h, 99, ctypes.byref(prm), batch, 129, P(big), P(vb), None, P(vb), P(vb), None, 0,
+                                  P(vb), _capi.MEM_HOST, res, ctypes.byref(summ)) == 4    # the same for a Box per problem
+    assert call(good, P(par), 3, solver=99) == 1                                           # unknown solver
     h.close()
