@@ -26,7 +26,8 @@ EXPORTS = ["ccqp_abi_version", "ccqp_status_string", "ccqp_last_error", "ccqp_cr
            "ccqp_comm_attach", "ccqp_comm_prepare", "ccqp_comm_detach", "ccqp_debug_divide", "ccqp_fp64_peak",
            "ccqp_microbench", "ccqp_debug_emulate_ranks", "ccqp_debug_solve_emulated", "ccqp_projected_gradient", "ccqp_solve_batched_table", "ccqp_solve_batched_sym",
            "ccqp_get_upload_info", "ccqp_set_matrix_symmetric", "ccqp_host_matrix_is_block_symmetric", "ccqp_upload_block_rows",
-           "ccqp_set_matrix_f32", "ccqp_solve_batched_tables"]
+           "ccqp_set_matrix_f32", "ccqp_solve_batched_tables", "ccqp_solve_batched_f32", "ccqp_solve_batched_sym_f32",
+           "ccqp_solve_batched_table_f32", "ccqp_solve_batched_tables_f32"]
 
 
 class Block(C.Structure):
@@ -87,6 +88,8 @@ def load():
     lib.ccqp_solve_batched_table.argtypes = [vp, i32, C.POINTER(Params), i64, i64, dp, dp, dp, C.POINTER(Block), i64, dp, i64, dp, i64,
                                              dp, i32, C.POINTER(Result), C.POINTER(Result)]
     lib.ccqp_solve_batched_tables.argtypes = lib.ccqp_solve_batched_table.argtypes
+    for name in ("ccqp_solve_batched", "ccqp_solve_batched_sym", "ccqp_solve_batched_table", "ccqp_solve_batched_tables"):
+        getattr(lib, name + "_f32").argtypes = getattr(lib, name).argtypes      # the fp32 twins: A is a float pointer
     lib.ccqp_set_matrix_symmetric.argtypes = [vp, dp, i64, i64, i32]
     lib.ccqp_set_matrix_f32.argtypes = [vp, dp, i64, i64, i64, i64, i32]
     lib.ccqp_get_upload_info.argtypes = [vp, C.POINTER(i64), C.POINTER(i32)]
@@ -236,13 +239,13 @@ def make_blocks(rows):
     return BlockArray(rows)
 
 
-def f64_ptr(a):
-    """(pointer, memtype, keepalive) of a float64 C-contiguous NumPy array or torch tensor."""
+def f64_ptr(a, dtype="float64"):
+    """(pointer, memtype, keepalive) of a float64 (or `dtype`) C-contiguous NumPy array or torch tensor."""
     if a is None:
         return None, None, None
     if isinstance(a, np.ndarray):
-        assert a.dtype == np.float64 and a.flags["C_CONTIGUOUS"]
+        assert a.dtype == np.dtype(dtype) and a.flags["C_CONTIGUOUS"]
         return C.c_void_p(a.ctypes.data), MEM_HOST, a
     # torch tensor (duck-typed to avoid importing torch here)
-    assert str(a.dtype) == "torch.float64" and a.is_contiguous()
+    assert str(a.dtype) == "torch." + dtype and a.is_contiguous()
     return C.c_void_p(a.data_ptr()), (MEM_DEVICE if a.is_cuda else MEM_HOST), a

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libccqp_b200.so")
-SOURCES = ["capi.cu", "dense_f64.cu", "batched.cu", "batched_sym.cu", "upload.cu", "emu.cu", "csr.cu", "dense_f32.cu"]      # see csrc/internal.h
+SOURCES = ["capi.cu", "dense_f64.cu", "batched.cu", "batched_f32.cu", "batched_sym.cu", "upload.cu", "emu.cu", "csr.cu", "dense_f32.cu"]      # see csrc/internal.h
 HEADERS = ["common.cuh", "proj.cuh", "dense.cuh", "kernel_build.cuh", "batched.cuh", "microbench.cuh", "internal.h", "symcheck.h",
            os.path.join("..", "..", "include", "ccqp_b200.h")]
 

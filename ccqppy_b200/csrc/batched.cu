@@ -1,5 +1,5 @@
-// Translation unit of the batched solver kernels (batched.cuh) and of the host side of every batched call: a
-// BatchedRequest (internal.h) becomes one kernel context and one persistent launch.
+// Translation unit of the fp64 batched solver kernels (batched.cuh; the fp32 ones: batched_f32.cu) and of the host side of
+// every batched call: a BatchedRequest (internal.h) becomes one kernel context and one persistent launch.
 #include <algorithm>
 #include <climits>
 #include <cmath>
@@ -31,33 +31,6 @@ cudaError_t launch_persistent(const void* kern, int threads, size_t dyn, const B
 }
 
 namespace {
-
-// n <= 64: 64 threads per problem, A in 128 registers per thread, up to 6 problems per SM; 64 < n <= 128: 256 threads, one per SM
-template <int SOLVER, bool WREG, bool GEN>
-cudaError_t launch_nt(const BatchedCtx& c, int sm_count, cudaStream_t stream) {
-    if (c.n <= kBN) return launch_persistent((const void*)batched_kernel<SOLVER, WREG, GEN, 64>, 64, 0, c, sm_count, stream);
-    return launch_persistent((const void*)batched_kernel<SOLVER, WREG, GEN, 256>, 256, sizeof(BatchedSmem<GEN, 256>), c,
-                             sm_count, stream);
-}
-
-// GEN: the general table instead of a Box per problem.  Unknown solvers, and MPRGP with a table, are rejected before.
-template <bool GEN>
-cudaError_t launch_batched(const BatchedCtx& c, int solver, bool wreg, int sm_count, cudaStream_t stream) {
-    switch (solver) {
-        case CCQP_SOLVER_PGD: return launch_nt<CCQP_SOLVER_PGD, true, GEN>(c, sm_count, stream);
-        case CCQP_SOLVER_APGD: return launch_nt<CCQP_SOLVER_APGD, true, GEN>(c, sm_count, stream);
-        case CCQP_SOLVER_APGD_AR: return launch_nt<CCQP_SOLVER_APGD_AR, true, GEN>(c, sm_count, stream);
-        case CCQP_SOLVER_BBPGD: return launch_nt<CCQP_SOLVER_BBPGD, true, GEN>(c, sm_count, stream);
-        case CCQP_SOLVER_BBPGDF: return launch_nt<CCQP_SOLVER_BBPGDF, true, GEN>(c, sm_count, stream);
-        case CCQP_SOLVER_SPG:
-            return wreg ? launch_nt<CCQP_SOLVER_SPG, true, GEN>(c, sm_count, stream)
-                        : launch_nt<CCQP_SOLVER_SPG, false, GEN>(c, sm_count, stream);
-        case CCQP_SOLVER_MPRGP:
-            if constexpr (!GEN) return launch_nt<CCQP_SOLVER_MPRGP, true, false>(c, sm_count, stream);
-            else return cudaErrorInvalidValue;
-        default: return cudaErrorInvalidValue;
-    }
-}
 
 // Smallest double q >= 0 with pred(sqrt(q)) false ... expressed through the bit pattern: for
 // non-negative doubles the IEEE ordering equals the ordering of the bit patterns, and sqrt is
@@ -141,7 +114,11 @@ int batched_solve(const BatchedRequest& r, cudaStream_t stream, int sm_count, cu
     const bool host = r.memtype == CCQP_MEM_HOST;
     if (solver == CCQP_SOLVER_SPG && (n_uniforms < 0 || (n_uniforms > 0 && !r.uniforms))) return CCQP_ERR_INVALID_ARG;
     if (solver < 0 || solver > CCQP_SOLVER_MPRGP) return CCQP_ERR_INVALID_ARG;
-    const size_t szA = (size_t)batch * n * n * 8, szV = (size_t)batch * n * 8;
+    // A is fp64, or fp32 for the _f32 entry points (r.A32): the kernels widen it in registers, nothing else changes
+    const bool f32 = r.A32 != nullptr;
+    const void* A = f32 ? static_cast<const void*>(r.A32) : static_cast<const void*>(r.A);
+    const long long esz = f32 ? 4 : 8;
+    const size_t szA = (size_t)batch * n * n * esz, szV = (size_t)batch * n * 8;
     const size_t szU = (solver == CCQP_SOLVER_SPG) ? (size_t)batch * n_uniforms * 8 : 0;
     const size_t szO = (size_t)batch * sizeof(BatchedOut);
     auto al = [](size_t v) { return (v + 255) / 256 * 256; };
@@ -160,14 +137,14 @@ int batched_solve(const BatchedRequest& r, cudaStream_t stream, int sm_count, cu
     BatchedCtx c;
     std::memset(&c, 0, sizeof(c));
     if (host) {
-        double* dA = reinterpret_cast<double*>(take(szA));
+        void* dA = take(szA);
         double* db = reinterpret_cast<double*>(take(szV));
         double* dlb = reinterpret_cast<double*>(take(szV));
         double* dub = reinterpret_cast<double*>(take(szV));
         double* dx0 = reinterpret_cast<double*>(take(szV));
         double* dxo = reinterpret_cast<double*>(take(szV));
         double* du = szU ? reinterpret_cast<double*>(take(szU)) : nullptr;
-        BCU(cudaMemcpyAsync(dA, r.A, szA, cudaMemcpyHostToDevice, stream));
+        BCU(cudaMemcpyAsync(dA, A, szA, cudaMemcpyHostToDevice, stream));
         BCU(cudaMemcpyAsync(db, r.b, szV, cudaMemcpyHostToDevice, stream));
         if (!table) BCU(cudaMemcpyAsync(dlb, r.lb, szV, cudaMemcpyHostToDevice, stream));
         if (!table) BCU(cudaMemcpyAsync(dub, r.ub, szV, cudaMemcpyHostToDevice, stream));
@@ -175,7 +152,7 @@ int batched_solve(const BatchedRequest& r, cudaStream_t stream, int sm_count, cu
         if (du) BCU(cudaMemcpyAsync(du, r.uniforms, szU, cudaMemcpyHostToDevice, stream));
         c.A = dA; c.b = db; c.lb = dlb; c.ub = dub; c.x0 = r.x0 ? dx0 : nullptr; c.uniforms = du; c.x_out = dxo;
     } else {
-        c.A = r.A; c.b = r.b; c.lb = r.lb; c.ub = r.ub; c.x0 = r.x0; c.uniforms = (solver == CCQP_SOLVER_SPG) ? r.uniforms : nullptr;
+        c.A = A; c.b = r.b; c.lb = r.lb; c.ub = r.ub; c.x0 = r.x0; c.uniforms = (solver == CCQP_SOLVER_SPG) ? r.uniforms : nullptr;
         c.x_out = r.x_out;
     }
     c.bound_stride = n;
@@ -209,9 +186,11 @@ int batched_solve(const BatchedRequest& r, cudaStream_t stream, int sm_count, cu
     c.n_uniforms = (solver == CCQP_SOLVER_SPG) ? n_uniforms : 0;
     c.out = dout; c.counter = counter;
     c.batch = (int)batch; c.n = (int)n;
-    c.tma_ok = ((n * 8) % 16 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 15) == 0) ? 1 : 0;
-    c.vec_ok = (n % 4 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 31) == 0) ? 1 : 0;
-    c.pf_ok = ((n * n * 8) % 16 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 15) == 0) ? 1 : 0;
+    // an fp32 A with n % 4 != 0 (rows not 16-byte multiples) or a base off a 16-byte boundary takes the per-element global
+    // loads: no copy is ever rounded up past the end of [batch][n][n]
+    c.tma_ok = ((n * esz) % 16 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 15) == 0) ? 1 : 0;
+    c.vec_ok = (!f32 && n % 4 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 31) == 0) ? 1 : 0;
+    c.pf_ok = ((n * n * esz) % 16 == 0 && (reinterpret_cast<uintptr_t>(c.A) & 15) == 0) ? 1 : 0;
     c.vtma_ok = (n % 2 == 0 && ((reinterpret_cast<uintptr_t>(c.b) | reinterpret_cast<uintptr_t>(c.lb) | reinterpret_cast<uintptr_t>(c.ub)) & 15) == 0) ? 1 : 0;
     if (table) {    // a parameter row is staged with b when every row is 16-byte aligned and fits vstage[1..2] (2 N doubles)
         const long long N = n <= kBN ? kBN : kBNMax;
@@ -229,10 +208,13 @@ int batched_solve(const BatchedRequest& r, cudaStream_t stream, int sm_count, cu
     BCU(cudaEventRecord(ev0, stream));
     const bool wreg = prm.m == kBWinReg;
     const bool use_sym = r.symmetric && !table && batched_sym_supported(solver, n);
-    const cudaError_t launch = use_sym ? launch_batched_sym(c, solver, wreg, sm_count, stream)
-                               : table ? launch_batched<true>(c, solver, wreg, sm_count, stream)
-                                       : launch_batched<false>(c, solver, wreg, sm_count, stream);
-    BCU(launch);
+    auto launch = [&](auto elem) {
+        using TA = decltype(elem);
+        return use_sym ? launch_batched_sym<TA>(c, solver, wreg, sm_count, stream)
+               : table ? launch_batched<true, TA>(c, solver, wreg, sm_count, stream)
+                       : launch_batched<false, TA>(c, solver, wreg, sm_count, stream);
+    };
+    BCU(f32 ? launch(float{}) : launch(double{}));
     launches += 1;
     BCU(cudaEventRecord(ev1, stream));
     if (host) BCU(cudaMemcpyAsync(r.x_out, c.x_out, szV, cudaMemcpyDeviceToHost, stream));
@@ -243,8 +225,8 @@ int batched_solve(const BatchedRequest& r, cudaStream_t stream, int sm_count, cu
     BCU(cudaEventElapsedTime(&ms, ev0, ev1));
     long long tot_mv = 0, tot_gemv = 0, tot_it = 0, tot_dr = 0, nconv = 0;
     int first_status = 0;
-    double hbmA = 8.0 * n * n;                  // bytes of A[i] the kernel reads
-    if (use_sym) { hbmA = 0; for (long long i = 0; i < n; ++i) hbmA += 8.0 * (double)(n - 8 * (i / 8)); }
+    double hbmA = (double)esz * n * n;          // bytes of A[i] the kernel reads
+    if (use_sym) { hbmA = 0; for (long long i = 0; i < n; ++i) hbmA += (double)esz * (double)(n - 8 * (i / 8)); }
     if (per_problem) hbmA += 8.0 * (double)np;  // the problem's parameter row
     for (long long i = 0; i < batch; ++i) {
         const BatchedOut& o = hout[(size_t)i];

@@ -34,7 +34,11 @@
 //   Problems are handed out through an atomic counter (iteration counts differ per problem); results do not depend on the
 //   schedule.
 //
-// Bounds: HBM bytes/problem = 8 n^2 + 32 n (+8 n for x0, + uniforms read by SPG);
+// fp32 Hessians (the _f32 entry points): the same kernels with A's element type TA = float.  Only the staging changes -- a
+// float tile, 4 bytes per entry on the mbarrier, and a register fill that widens every entry exactly (cvt.f64.f32) -- so the
+// registers hold what the fp64 kernel holds for the widened matrix and solve_one, which never sees TA, returns the same bits.
+//
+// Bounds: HBM bytes/problem = 8 n^2 + 32 n (fp32 A: 4 n^2 + 32 n) (+8 n for x0, + uniforms read by SPG);
 //         fp64 flops/problem = 2 n^2 * (mat-vecs executed).
 #pragma once
 #include <cmath>
@@ -61,6 +65,9 @@ struct BL {
                                                        // bytes further into the 128-byte bank window (conflict-free LDS.128)
     static constexpr int XS = NB * SLICE;
     static constexpr int PITCH = N + 2;                // tile row pitch (doubles): conflict-free LDS.128 register fill
+    static constexpr int PITCH_F32 = N + 4;            // ... (floats, rows 16-byte aligned): NT = 64 conflict-free (4 wavefronts per
+                                                       // LDS.128); NT = 256 2 per quarter warp, 8 per LDS.128 at any pitch (the
+                                                       // lane pairs that share a row sit 32 bytes apart), the fp64 fill's total
     static constexpr uint32_t XS_BYTES = XS * 8, RED_BYTES = WARPS * 32;
 };
 constexpr int kBN = 64;                 // the small layout's limit
@@ -76,7 +83,7 @@ struct BatchedOut {
 };
 
 struct BatchedCtx {
-    const double* A;        // [batch][n][n]
+    const void* A;          // [batch][n][n] of the kernel's element type (double, or float for the _f32 entry points)
     const double* b;        // [batch][n]
     const double* x0;       // [batch][n] or null
     const double* lb;       // [batch][n] (Box per problem; unused by the general table)
@@ -97,9 +104,9 @@ struct BatchedCtx {
     BatchedOut* out;        // [batch]
     unsigned* counter;      // work queue head
     int batch, n;
-    int tma_ok;             // rows of A can be moved with 16-byte bulk copies (8n % 16 == 0, 16-byte aligned base)
-    int vec_ok;             // rows of A can be read with 256-bit loads (n % 4 == 0, 32-byte aligned base)
-    int pf_ok;              // whole problems can be bulk-prefetched into L2 (16-byte granularity)
+    int tma_ok;             // rows of A can be moved with 16-byte bulk copies (n * sizeof(entry) % 16 == 0, 16-byte aligned base)
+    int vec_ok;             // rows of A can be read with 256-bit loads (fp64 A, n % 4 == 0, 32-byte aligned base)
+    int pf_ok;              // whole problems can be bulk-prefetched into L2 (n^2 * sizeof(entry) % 16 == 0, 16-byte aligned base)
     int vtma_ok;            // b / lb / ub rows (general table: b and parameter rows) can be moved with 16-byte bulk copies
                             // (n even, 16-byte aligned bases; general table: see prow_bytes)
     double tol, max_mv, step, tau, sig1, sig2;
@@ -114,9 +121,10 @@ struct BatchedCtx {
                             // vstage[1..2] area); 0: no parameters
 };
 
-template <bool GEN, int NT>
+template <bool GEN, int NT, class TA>
 struct BatchedSmem {
-    double tile[BL<NT>::N * BL<NT>::PITCH];   // the NEXT problem's A, landed by TMA while the current one iterates
+    static constexpr int PITCH = sizeof(TA) == 8 ? BL<NT>::PITCH : BL<NT>::PITCH_F32;
+    TA tile[BL<NT>::N * PITCH];               // the NEXT problem's A, landed by TMA while the current one iterates
     double vstage[3][BL<NT>::N];              // ... and its b / lower / upper bounds (general table: b / parameter row
                                               // of up to 2 N entries in vstage[1..2]) on the same mbarrier
     double xs[2][BL<NT>::XS];                 // mat-vec input, double buffered
@@ -146,6 +154,12 @@ __device__ __forceinline__ double lds_f64(uint32_t addr) {
 }
 __device__ __forceinline__ void lds_f64x2(uint32_t addr, double& x, double& y) {
     asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(x), "=d"(y) : "r"(addr) : "memory");
+}
+// four floats of an fp32 tile, widened exactly: d[0..3] <- (double)tile[addr .. addr + 15]
+__device__ __forceinline__ void lds_f32x4_widen(uint32_t addr, double* d) {
+    float f0, f1, f2, f3;
+    asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(f0), "=f"(f1), "=f"(f2), "=f"(f3) : "r"(addr) : "memory");
+    d[0] = (double)f0; d[1] = (double)f1; d[2] = (double)f2; d[3] = (double)f3;
 }
 
 __device__ __forceinline__ double shfl_xor_f64(double v, int mask) { return __shfl_xor_sync(0xffffffffu, v, mask); }
@@ -636,13 +650,16 @@ constexpr int batched_min_ctas(int solver) {
 
 extern __shared__ __align__(16) unsigned char batched_dyn_smem[];       // NT = 256: the 141 KB of BatchedSmem are dynamic
 
-template <int SOLVER, bool WREG, bool GEN, int NT>
+// TA: the element type of A in memory (double / float); the registers and everything after the fill are fp64 either way
+template <int SOLVER, bool WREG, bool GEN, int NT, class TA>
 __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOLVER)) : 1) batched_kernel(const BatchedCtx c) {
     using L = BL<NT>;
-    BatchedSmem<GEN, NT>* smp;
-    if constexpr (NT == 64) { __shared__ __align__(16) BatchedSmem<GEN, 64> sm_static; smp = &sm_static; }
-    else smp = reinterpret_cast<BatchedSmem<GEN, NT>*>(batched_dyn_smem);
-    BatchedSmem<GEN, NT>& sm = *smp;
+    using Smem = BatchedSmem<GEN, NT, TA>;
+    constexpr uint32_t ESZ = sizeof(TA);
+    Smem* smp;
+    if constexpr (NT == 64) { __shared__ __align__(16) Smem sm_static; smp = &sm_static; }
+    else smp = reinterpret_cast<Smem*>(batched_dyn_smem);
+    Smem& sm = *smp;
     const int t = threadIdx.x, n = c.n;
     const int cb = t & (L::NB - 1), key = cb >> L::SH, row0 = kBRows * (t / L::NB), col0 = kBCols * cb;
     const int u = row0 + key;               // the unknown this thread holds (NT = 64: u == t)
@@ -653,29 +670,35 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
     sh.xs_rd = smem_u32(&sm.xs[0][L::SLICE * cb]);
     sh.red = smem_u32(&sm.red[0][0][0]);
     const size_t prob_elems = (size_t)n * n;
+    // (c.A is cast to const TA* where it is used: a typed copy taken here moves the load of c.A, and with it the schedule
+    // ptxas picks for the fp64 instantiations)
 
     auto prefetch_l2 = [&](int prob) {      // the whole next problem, one instruction (TMA engine)
         if (c.pf_ok && t == 0)
-            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(c.A + (size_t)prob * prob_elems),
-                         "r"((unsigned)(prob_elems * 8)) : "memory");
+            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;"
+                         ::"l"(static_cast<const TA*>(c.A) + (size_t)prob * prob_elems), "r"((unsigned)(prob_elems * ESZ)) : "memory");
     };
     const bool staged = c.tma_ok != 0;
     const bool vstaged = staged && c.vtma_ok != 0;
     unsigned phase = 0;
     if (t == 0) { mbar_init(&sm.mbar, 1); mbar_fence_init(); }
-    auto issue_load = [&](int prob) {       // one 8n-byte bulk copy per row into the padded tile (+ 3 for the vectors), one mbarrier
+    auto issue_load = [&](int prob) {       // one n * ESZ-byte bulk copy per row into the padded tile (+ 3 for the vectors), one mbarrier
         if constexpr (GEN) {
             // b into vstage[0], the problem's parameter row into vstage[1..2].  bb / pb are the one definition of what is
             // copied: thread 0 announces exactly bb + pb bytes besides A, and a copy is issued iff its size is non-zero
             // (announced bytes that never arrive would leave mbar_wait spinning forever).
             const uint32_t bb = vstaged ? (uint32_t)(n * 8) : 0u, pb = vstaged ? (uint32_t)c.prow_bytes : 0u;
-            if (t == 0) mbar_expect_tx(&sm.mbar, (uint32_t)(prob_elems * 8) + bb + pb);
-            if (t < n) bulk_g2s(sm.tile + t * L::PITCH, c.A + (size_t)prob * prob_elems + (size_t)t * n, (uint32_t)(n * 8), &sm.mbar);
+            if (t == 0) mbar_expect_tx(&sm.mbar, (uint32_t)(prob_elems * ESZ) + bb + pb);
+            if (t < n)
+                bulk_g2s(sm.tile + t * Smem::PITCH, static_cast<const TA*>(c.A) + (size_t)prob * prob_elems + (size_t)t * n,
+                         (uint32_t)n * ESZ, &sm.mbar);
             if (bb != 0u && t == NT - 1) bulk_g2s(sm.vstage[0], c.b + (size_t)prob * n, bb, &sm.mbar);
             if (pb != 0u && t == NT - 2) bulk_g2s(sm.vstage[1], c.params + (size_t)prob * c.param_stride, pb, &sm.mbar);
         } else {
-            if (t == 0) mbar_expect_tx(&sm.mbar, (uint32_t)(prob_elems * 8) + (vstaged ? 3u * (uint32_t)(n * 8) : 0u));
-            if (t < n) bulk_g2s(sm.tile + t * L::PITCH, c.A + (size_t)prob * prob_elems + (size_t)t * n, (uint32_t)(n * 8), &sm.mbar);
+            if (t == 0) mbar_expect_tx(&sm.mbar, (uint32_t)(prob_elems * ESZ) + (vstaged ? 3u * (uint32_t)(n * 8) : 0u));
+            if (t < n)
+                bulk_g2s(sm.tile + t * Smem::PITCH, static_cast<const TA*>(c.A) + (size_t)prob * prob_elems + (size_t)t * n,
+                         (uint32_t)n * ESZ, &sm.mbar);
             if (vstaged && t >= NT - 3) {   // three otherwise idle-ish threads (the mbarrier's expect_tx is program-ordered only in thread 0,
                 const int w = t - (NT - 3); // but a complete_tx that arrives first just drives the pending count negative: legal)
                 const double* src = w == 0 ? c.b + (size_t)prob * n : (w == 1 ? c.lb : c.ub) + (size_t)prob * c.bound_stride;
@@ -692,7 +715,7 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
     while (cur < c.batch) {
         // ---- register fill: this thread's sub-block; register row r <- row row0 + (r ^ key) (see matvec)
         double a[kBRows][kBCols];
-        const double* Ap = c.A + (size_t)cur * prob_elems;
+        const TA* Ap = static_cast<const TA*>(c.A) + (size_t)cur * prob_elems;
         BState s;
         s.u = u;
         s.act = u < n;
@@ -706,10 +729,18 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
 #pragma unroll
             for (int r = 0; r < kBRows; ++r) {
                 const int row = row0 + (r ^ key);
+                if constexpr (ESZ == 8) {
 #pragma unroll
-                for (int j = 0; j < kBCols; j += 2) {
-                    if (row < n && col0 + j < n) lds_f64x2(tb + (uint32_t)(row * L::PITCH + col0 + j) * 8u, a[r][j], a[r][j + 1]);
-                    else { a[r][j] = 0.0; a[r][j + 1] = 0.0; }
+                    for (int j = 0; j < kBCols; j += 2) {
+                        if (row < n && col0 + j < n) lds_f64x2(tb + (uint32_t)(row * L::PITCH + col0 + j) * 8u, a[r][j], a[r][j + 1]);
+                        else { a[r][j] = 0.0; a[r][j + 1] = 0.0; }
+                    }
+                } else {            // staged implies n % 4 == 0: a 4-float group is inside the row or wholly past its end
+#pragma unroll
+                    for (int j = 0; j < kBCols; j += 4) {
+                        if (row < n && col0 + j < n) lds_f32x4_widen(tb + (uint32_t)(row * Smem::PITCH + col0 + j) * 4u, &a[r][j]);
+                        else { a[r][j] = 0.0; a[r][j + 1] = 0.0; a[r][j + 2] = 0.0; a[r][j + 3] = 0.0; }
+                    }
                 }
             }
             if (vstaged) {
@@ -719,17 +750,19 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
                     s.hi = s.act ? sm.vstage[2][u] : 0.0;
                 }
             }
-        } else if (c.vec_ok) {
+        } else if (ESZ == 8 && c.vec_ok) {       // fp64 only (the host never sets vec_ok for an fp32 A)
+            if constexpr (ESZ == 8) {
 #pragma unroll
-            for (int r = 0; r < kBRows; ++r) {
+                for (int r = 0; r < kBRows; ++r) {
 #pragma unroll
-                for (int j = 0; j < kBCols; j += 4) {
-                    const int row = row0 + (r ^ key);
-                    if (row < n && col0 + j < n) {
-                        double v[4];
-                        ldg_vec4_stream<false>(Ap + (size_t)row * n + col0 + j, v);
-                        a[r][j] = v[0]; a[r][j + 1] = v[1]; a[r][j + 2] = v[2]; a[r][j + 3] = v[3];
-                    } else { a[r][j] = 0.0; a[r][j + 1] = 0.0; a[r][j + 2] = 0.0; a[r][j + 3] = 0.0; }
+                    for (int j = 0; j < kBCols; j += 4) {
+                        const int row = row0 + (r ^ key);
+                        if (row < n && col0 + j < n) {
+                            double v[4];
+                            ldg_vec4_stream<false>(Ap + (size_t)row * n + col0 + j, v);
+                            a[r][j] = v[0]; a[r][j + 1] = v[1]; a[r][j + 2] = v[2]; a[r][j + 3] = v[3];
+                        } else { a[r][j] = 0.0; a[r][j + 1] = 0.0; a[r][j + 2] = 0.0; a[r][j + 3] = 0.0; }
+                    }
                 }
             }
         } else {
@@ -737,7 +770,7 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
             for (int r = 0; r < kBRows; ++r)
 #pragma unroll
                 for (int j = 0; j < kBCols; ++j)
-                    a[r][j] = (row0 + (r ^ key) < n && col0 + j < n) ? ldg_stream(Ap + (size_t)(row0 + (r ^ key)) * n + col0 + j) : 0.0;
+                    a[r][j] = (row0 + (r ^ key) < n && col0 + j < n) ? (double)ldg_stream(Ap + (size_t)(row0 + (r ^ key)) * n + col0 + j) : 0.0;
         }
         if (!vstaged) {
             s.b = s.act ? c.b[vo] : 0.0;
@@ -789,8 +822,40 @@ __global__ void __launch_bounds__(NT, NT == 64 ? (GEN ? 5 : batched_min_ctas(SOL
 // dynamic shared memory) with as many CTAs as fit on the device, at most one per problem
 cudaError_t launch_persistent(const void* kern, int threads, size_t dyn, const BatchedCtx& c, int sm_count, cudaStream_t stream);
 
-// batched_sym.cu: the one-warp-per-problem kernels for symmetric Hessians (n <= 64; PGD / BBPGD / BBPGDf / SPG, Box per problem)
+// n <= 64: 64 threads per problem, A in 128 registers per thread, up to 6 problems per SM; 64 < n <= 128: 256 threads, one per SM
+template <int SOLVER, bool WREG, bool GEN, class TA>
+cudaError_t launch_nt(const BatchedCtx& c, int sm_count, cudaStream_t stream) {
+    if (c.n <= kBN) return launch_persistent((const void*)batched_kernel<SOLVER, WREG, GEN, 64, TA>, 64, 0, c, sm_count, stream);
+    return launch_persistent((const void*)batched_kernel<SOLVER, WREG, GEN, 256, TA>, 256, sizeof(BatchedSmem<GEN, 256, TA>), c,
+                             sm_count, stream);
+}
+
+// GEN: the general table instead of a Box per problem; TA: A's element type.  Unknown solvers, and MPRGP with a table, are
+// rejected before.  The fp64 kernels are instantiated in batched.cu, the fp32 ones in batched_f32.cu.
+template <bool GEN, class TA>
+cudaError_t launch_batched(const BatchedCtx& c, int solver, bool wreg, int sm_count, cudaStream_t stream) {
+    switch (solver) {
+        case CCQP_SOLVER_PGD: return launch_nt<CCQP_SOLVER_PGD, true, GEN, TA>(c, sm_count, stream);
+        case CCQP_SOLVER_APGD: return launch_nt<CCQP_SOLVER_APGD, true, GEN, TA>(c, sm_count, stream);
+        case CCQP_SOLVER_APGD_AR: return launch_nt<CCQP_SOLVER_APGD_AR, true, GEN, TA>(c, sm_count, stream);
+        case CCQP_SOLVER_BBPGD: return launch_nt<CCQP_SOLVER_BBPGD, true, GEN, TA>(c, sm_count, stream);
+        case CCQP_SOLVER_BBPGDF: return launch_nt<CCQP_SOLVER_BBPGDF, true, GEN, TA>(c, sm_count, stream);
+        case CCQP_SOLVER_SPG:
+            return wreg ? launch_nt<CCQP_SOLVER_SPG, true, GEN, TA>(c, sm_count, stream)
+                        : launch_nt<CCQP_SOLVER_SPG, false, GEN, TA>(c, sm_count, stream);
+        case CCQP_SOLVER_MPRGP:
+            if constexpr (!GEN) return launch_nt<CCQP_SOLVER_MPRGP, true, false, TA>(c, sm_count, stream);
+            else return cudaErrorInvalidValue;
+        default: return cudaErrorInvalidValue;
+    }
+}
+extern template cudaError_t launch_batched<false, float>(const BatchedCtx&, int, bool, int, cudaStream_t);
+extern template cudaError_t launch_batched<true, float>(const BatchedCtx&, int, bool, int, cudaStream_t);
+
+// batched_sym.cu: the one-warp-per-problem kernels for symmetric Hessians (n <= 64; PGD / BBPGD / BBPGDf / SPG, Box per
+// problem), TA = double / float
 bool batched_sym_supported(int solver, long long n);
+template <class TA>
 cudaError_t launch_batched_sym(const BatchedCtx& c, int solver, bool wreg, int sm_count, cudaStream_t stream);
 
 }  // namespace ccqp

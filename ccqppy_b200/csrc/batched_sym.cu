@@ -31,6 +31,10 @@
 // over two sub-partitions.  The DFMA count per problem is the same in both layouts, so is their operand traffic; what the
 // symmetric layout buys is register space (and half of the HBM reads), what it costs is the exchange through shared memory.
 // Hence: an opt-in for callers whose solver is SPG (or whose batch is HBM- or capacity-bound), not the default.
+//
+// fp32 Hessians (ccqp_solve_batched_sym_f32): the same kernel with TA = float -- a compact float tile (rows padded by 4 floats,
+// 16-byte aligned), row pieces of (n - c0) * 4 bytes, and a fill that widens every entry exactly; registers and solver loop
+// are those of the fp64 kernel on the widened matrix, so the results are the same bits.
 #include "batched.cuh"
 
 namespace ccqp {
@@ -43,18 +47,22 @@ constexpr int kSlots = 7;
 constexpr int kCtPitch = 82;            // doubles per slot: 41 16-byte chunks = 1 (mod 8), so that a lane's slot and its row block both move
                                         // its 16-byte chunk inside the 128-byte bank window (6 wavefronts per store instead of 9 at 90)
 constexpr int kRowPad = 2;
+constexpr int kRowPadF32 = 4;           // floats: rows start 16-byte aligned; register fill 174 wavefronts (fp64 tile: 516)
+template <class TA> constexpr int kRowPadOf = sizeof(TA) == 8 ? kRowPad : kRowPadF32;
 constexpr int kCtas = 8;                // resident CTAs (= problems) per SM
 
-// offset (doubles) of row i inside the compact tile: row block rb = i / 8 stores columns 8 rb .. 63 (+ kRowPad)
-__host__ __device__ constexpr int tile_row_off(int i) {
+// offset (entries) of row i inside the compact tile: row block rb = i / 8 stores columns 8 rb .. 63 (+ pad)
+__host__ __device__ constexpr int tile_row_off(int i, int pad = kRowPad) {
     const int rb = i >> 3;
-    return 8 * rb * (kN + kRowPad) - 32 * rb * (rb - 1) + (i & 7) * (kN - 8 * rb + kRowPad);
+    return 8 * rb * (kN + pad) - 32 * rb * (rb - 1) + (i & 7) * (kN - 8 * rb + pad);
 }
 constexpr int kTile = tile_row_off(kN);
 static_assert(kTile == 2432, "compact tile");
+static_assert(tile_row_off(kN, kRowPadF32) % 4 == 0, "fp32 tile: the vectors behind it stay 16-byte aligned");
 
+template <class TA>
 struct Smem {
-    double tile[kTile];             // the NEXT problem: upper block triangle, row by row
+    TA tile[tile_row_off(kN, kRowPadOf<TA>)];   // the NEXT problem: upper block triangle, row by row
     double vstage[3][kN];           // ... its b / lb / ub
     double vcur[3][kN];             // b / lb / ub of the problem being solved (12 registers per lane that the mat-vec needs more)
     double xs[kXS];                 // mat-vec input
@@ -350,9 +358,11 @@ __device__ __forceinline__ void solve_one(const BatchedCtx& c, const double (&a)
 #endif
 }
 
-template <int SOLVER, bool WREG>
+template <int SOLVER, bool WREG, class TA>
 __global__ void __launch_bounds__(32, kCtas) batched_sym_kernel(const BatchedCtx c) {
-    __shared__ __align__(16) Smem sm;
+    __shared__ __align__(16) Smem<TA> sm;
+    constexpr int PAD = kRowPadOf<TA>;
+    constexpr uint32_t ESZ = sizeof(TA);
     const int lane = threadIdx.x, n = c.n;
     // lane -> block (r, cc), r < cc, row-major over the 28 blocks above the diagonal
     int r = 0, cc = 1;
@@ -377,20 +387,20 @@ __global__ void __launch_bounds__(32, kCtas) batched_sym_kernel(const BatchedCtx
     L.ct_rd = ct0 + (uint32_t)(u0 + 2 * k) * 8u;
     const size_t prob_elems = (size_t)n * n;
 
-    const bool staged = c.tma_ok != 0;                  // n even, 16-byte aligned A: every row piece is a legal bulk copy
+    const bool staged = c.tma_ok != 0;                  // n * ESZ % 16 == 0, 16-byte aligned A: every row piece is a legal bulk copy
     const bool vstaged = staged && c.vtma_ok != 0;
     uint32_t tx_bytes = vstaged ? 3u * (uint32_t)(n * 8) : 0u;
-    for (int i = 0; i < n; ++i) tx_bytes += (uint32_t)(n - 8 * (i >> 3)) * 8u;
+    for (int i = 0; i < n; ++i) tx_bytes += (uint32_t)(n - 8 * (i >> 3)) * ESZ;
     unsigned phase = 0;
     if (lane == 0) { mbar_init(&sm.mbar, 1); mbar_fence_init(); }
     __syncwarp();
     auto issue_load = [&](int prob) {       // one bulk copy per row: columns 8 * (i / 8) .. n-1 (+ 3 for the vectors), one mbarrier
-        const double* Ap = c.A + (size_t)prob * prob_elems;
+        const TA* Ap = static_cast<const TA*>(c.A) + (size_t)prob * prob_elems;
         if (lane == 0) mbar_expect_tx(&sm.mbar, tx_bytes);
         __syncwarp();
         for (int i = lane; i < n; i += 32) {
             const int c0 = 8 * (i >> 3);
-            bulk_g2s(sm.tile + tile_row_off(i), Ap + (size_t)i * n + c0, (uint32_t)(n - c0) * 8u, &sm.mbar);
+            bulk_g2s(sm.tile + tile_row_off(i, PAD), Ap + (size_t)i * n + c0, (uint32_t)(n - c0) * ESZ, &sm.mbar);
         }
         if (vstaged && lane >= 29) {
             const int w = lane - 29;
@@ -404,7 +414,7 @@ __global__ void __launch_bounds__(32, kCtas) batched_sym_kernel(const BatchedCtx
     if (staged && cur < c.batch) { fence_proxy_async(); issue_load(cur); }
     while (cur < c.batch) {
         double a[8][8], dg[2][8];
-        const double* Ap = c.A + (size_t)cur * prob_elems;
+        const TA* Ap = static_cast<const TA*>(c.A) + (size_t)cur * prob_elems;
         State s;
         const size_t vo = (size_t)cur * n + u0;
         const size_t bo = (size_t)cur * c.bound_stride + u0;
@@ -412,22 +422,35 @@ __global__ void __launch_bounds__(32, kCtas) batched_sym_kernel(const BatchedCtx
             mbar_wait(&sm.mbar, phase);
             phase ^= 1u;
             const uint32_t tb = smem_u32(sm.tile);
+            // fp64: two doubles per LDS.128; fp32 (staged implies n % 4 == 0): four floats, widened -- a group of
+            // 16 / ESZ entries lies inside the row or wholly past its end
+            constexpr int V = 16 / ESZ;
+            auto ld = [&](uint32_t addr, double* d) {
+                if constexpr (ESZ == 8) lds_f64x2(addr, d[0], d[1]);
+                else lds_f32x4_widen(addr, d);
+            };
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
-                const uint32_t ro = tb + (uint32_t)(tile_row_off(8 * r) + i * (kN - 8 * r + kRowPad) + 8 * (cc - r)) * 8u;
+                const uint32_t ro = tb + (uint32_t)(tile_row_off(8 * r, PAD) + i * (kN - 8 * r + PAD) + 8 * (cc - r)) * ESZ;
 #pragma unroll
-                for (int j = 0; j < 8; j += 2) {
-                    if (L.has_blk && 8 * r + i < n && 8 * cc + j < n) lds_f64x2(ro + j * 8, a[i][j], a[i][j + 1]);
-                    else { a[i][j] = 0.0; a[i][j + 1] = 0.0; }
+                for (int j = 0; j < 8; j += V) {
+                    if (L.has_blk && 8 * r + i < n && 8 * cc + j < n) ld(ro + j * ESZ, &a[i][j]);
+                    else {
+#pragma unroll
+                        for (int q = 0; q < V; ++q) a[i][j + q] = 0.0;
+                    }
                 }
             }
 #pragma unroll
             for (int t = 0; t < 2; ++t) {
-                const uint32_t ro = tb + (uint32_t)tile_row_off(u0 + t) * 8u;
+                const uint32_t ro = tb + (uint32_t)tile_row_off(u0 + t, PAD) * ESZ;
 #pragma unroll
-                for (int j = 0; j < 8; j += 2) {
-                    if (u0 + t < n && 8 * k + j < n) lds_f64x2(ro + j * 8, dg[t][j], dg[t][j + 1]);
-                    else { dg[t][j] = 0.0; dg[t][j + 1] = 0.0; }
+                for (int j = 0; j < 8; j += V) {
+                    if (u0 + t < n && 8 * k + j < n) ld(ro + j * ESZ, &dg[t][j]);
+                    else {
+#pragma unroll
+                        for (int q = 0; q < V; ++q) dg[t][j + q] = 0.0;
+                    }
                 }
             }
         } else {
@@ -435,12 +458,12 @@ __global__ void __launch_bounds__(32, kCtas) batched_sym_kernel(const BatchedCtx
             for (int i = 0; i < 8; ++i)
 #pragma unroll
                 for (int j = 0; j < 8; ++j)
-                    a[i][j] = (L.has_blk && 8 * r + i < n && 8 * cc + j < n) ? ldg_stream(Ap + (size_t)(8 * r + i) * n + 8 * cc + j) : 0.0;
+                    a[i][j] = (L.has_blk && 8 * r + i < n && 8 * cc + j < n) ? (double)ldg_stream(Ap + (size_t)(8 * r + i) * n + 8 * cc + j) : 0.0;
 #pragma unroll
             for (int t = 0; t < 2; ++t)
 #pragma unroll
                 for (int j = 0; j < 8; ++j)
-                    dg[t][j] = (u0 + t < n && 8 * k + j < n) ? ldg_stream(Ap + (size_t)(u0 + t) * n + 8 * k + j) : 0.0;
+                    dg[t][j] = (u0 + t < n && 8 * k + j < n) ? (double)ldg_stream(Ap + (size_t)(u0 + t) * n + 8 * k + j) : 0.0;
         }
         {
             V2 vb, vl, vh;
@@ -465,8 +488,8 @@ __global__ void __launch_bounds__(32, kCtas) batched_sym_kernel(const BatchedCtx
         if (nxt < c.batch) {                   // the next problem travels while this one iterates
             if (staged) { fence_proxy_async(); issue_load(nxt); }
             else if (c.pf_ok && lane == 0)
-                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(c.A + (size_t)nxt * prob_elems),
-                             "r"((unsigned)(prob_elems * 8)) : "memory");
+                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(static_cast<const TA*>(c.A) + (size_t)nxt * prob_elems),
+                             "r"((unsigned)(prob_elems * ESZ)) : "memory");
             if (c.x0 && L.act0) asm volatile("prefetch.global.L2 [%0];" ::"l"(c.x0 + (size_t)nxt * n + u0));
             if (lane == 0) after = atomicAdd(c.counter, 1u);     // consumed at the end of the solve
         } else if (lane == 0) after = (unsigned)c.batch;
@@ -488,19 +511,22 @@ bool batched_sym_supported(int solver, long long n) {
                              solver == CCQP_SOLVER_SPG);
 }
 
+template <class TA>
 cudaError_t launch_batched_sym(const BatchedCtx& c, int solver, bool wreg, int sm_count, cudaStream_t stream) {
     const void* kern;
     switch (solver) {
-        case CCQP_SOLVER_PGD: kern = (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_PGD, true>; break;
-        case CCQP_SOLVER_BBPGD: kern = (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_BBPGD, true>; break;
-        case CCQP_SOLVER_BBPGDF: kern = (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_BBPGDF, true>; break;
+        case CCQP_SOLVER_PGD: kern = (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_PGD, true, TA>; break;
+        case CCQP_SOLVER_BBPGD: kern = (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_BBPGD, true, TA>; break;
+        case CCQP_SOLVER_BBPGDF: kern = (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_BBPGDF, true, TA>; break;
         case CCQP_SOLVER_SPG:
-            kern = wreg ? (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_SPG, true>
-                        : (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_SPG, false>;
+            kern = wreg ? (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_SPG, true, TA>
+                        : (const void*)bsym::batched_sym_kernel<CCQP_SOLVER_SPG, false, TA>;
             break;
         default: return cudaErrorInvalidValue;
     }
     return launch_persistent(kern, 32, 0, c, sm_count, stream);
 }
+template cudaError_t launch_batched_sym<double>(const BatchedCtx&, int, bool, int, cudaStream_t);
+template cudaError_t launch_batched_sym<float>(const BatchedCtx&, int, bool, int, cudaStream_t);
 
 }  // namespace ccqp

@@ -813,7 +813,7 @@ ccqp_status ccqp_projected_gradient(ccqp_handle* h, const double* x, const doubl
 // Every batched call: the checks of its arguments, then batched.cu.
 static ccqp_status solve_batched(ccqp_handle* h, const BatchedRequest& r) {
     const bool box = r.set == BatchedSet::kBox;
-    if (!h || !params_ok(r.params, r.solver) || r.batch <= 0 || r.n <= 0 || !r.A || !r.b || !r.x_out ||
+    if (!h || !params_ok(r.params, r.solver) || r.batch <= 0 || r.n <= 0 || !(r.A || r.A32) || !r.b || !r.x_out ||
         (box ? (!r.lb || !r.ub)
              : (!r.blocks || r.n_blocks <= 0 || (r.n_params > 0 && !r.block_params) || (r.set == BatchedSet::kTables && r.n_params < 0))))
         return CCQP_ERR_INVALID_ARG;
@@ -851,6 +851,41 @@ ccqp_status ccqp_solve_batched_tables(ccqp_handle* h, int solver, const ccqp_par
                                       double* x_out, int memtype, ccqp_result* results, ccqp_result* summary) {
     return solve_batched(h, {solver, params, batch, n, A, b, x0, uniforms, n_uniforms, x_out, memtype, results, summary,
                              BatchedSet::kTables, nullptr, nullptr, false, blocks, n_blocks, block_params, n_params});
+}
+
+// The fp32 twins: the same requests with A32 in place of A
+ccqp_status ccqp_solve_batched_f32(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
+                                   const float* A, const double* b, const double* x0, const double* lb, const double* ub,
+                                   const double* uniforms, int64_t n_uniforms, double* x_out, int memtype,
+                                   ccqp_result* results, ccqp_result* summary) {
+    return solve_batched(h, {solver, params, batch, n, nullptr, b, x0, uniforms, n_uniforms, x_out, memtype, results, summary,
+                             BatchedSet::kBox, lb, ub, false, nullptr, 0, nullptr, 0, A});
+}
+
+ccqp_status ccqp_solve_batched_sym_f32(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
+                                       const float* A, const double* b, const double* x0, const double* lb, const double* ub,
+                                       const double* uniforms, int64_t n_uniforms, double* x_out, int memtype,
+                                       ccqp_result* results, ccqp_result* summary) {
+    return solve_batched(h, {solver, params, batch, n, nullptr, b, x0, uniforms, n_uniforms, x_out, memtype, results, summary,
+                             BatchedSet::kBox, lb, ub, true, nullptr, 0, nullptr, 0, A});
+}
+
+ccqp_status ccqp_solve_batched_table_f32(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
+                                         const float* A, const double* b, const double* x0, const ccqp_block* blocks,
+                                         int64_t n_blocks, const double* block_params, int64_t n_params, const double* uniforms,
+                                         int64_t n_uniforms, double* x_out, int memtype, ccqp_result* results,
+                                         ccqp_result* summary) {
+    return solve_batched(h, {solver, params, batch, n, nullptr, b, x0, uniforms, n_uniforms, x_out, memtype, results, summary,
+                             BatchedSet::kTable, nullptr, nullptr, false, blocks, n_blocks, block_params, n_params, A});
+}
+
+ccqp_status ccqp_solve_batched_tables_f32(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch, int64_t n,
+                                          const float* A, const double* b, const double* x0, const ccqp_block* blocks,
+                                          int64_t n_blocks, const double* block_params, int64_t n_params, const double* uniforms,
+                                          int64_t n_uniforms, double* x_out, int memtype, ccqp_result* results,
+                                          ccqp_result* summary) {
+    return solve_batched(h, {solver, params, batch, n, nullptr, b, x0, uniforms, n_uniforms, x_out, memtype, results, summary,
+                             BatchedSet::kTables, nullptr, nullptr, false, blocks, n_blocks, block_params, n_params, A});
 }
 
 namespace {

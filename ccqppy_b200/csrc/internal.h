@@ -1,5 +1,6 @@
-// Entry points between the translation units of libccqp_b200.so: capi.cu (C-ABI, host code), batched.cu (batched kernels
-// and the host side of every batched call) + batched_sym.cu (batched kernels for symmetric Hessians), upload.cu (host -> device matrix copies), and the four compilations of the dense solver kernels, one
+// Entry points between the translation units of libccqp_b200.so: capi.cu (C-ABI, host code), batched.cu (fp64 batched kernels
+// and the host side of every batched call) + batched_f32.cu (the same kernels for fp32 A) + batched_sym.cu (batched kernels
+// for symmetric Hessians, fp64 and fp32 A), upload.cu (host -> device matrix copies), and the four compilations of the dense solver kernels, one
 // unit each because each sees dense.cuh with different macros: dense_f64.cu (fp64 Hessians), dense_f32.cu (fp32-stored
 // Hessians), csr.cu (CSR Hessians), emu.cu (emulated ranks, a test vehicle).  The rest are separate units only so that
 // they compile in parallel.
@@ -67,6 +68,8 @@ struct BatchedRequest {
     long long n_blocks;
     const double* block_params;
     long long n_params;
+    // the _f32 entry points: A is null and this is the [batch][n][n] Hessian, stored as fp32 (widened exactly in registers)
+    const float* A32;
 };
 
 // batched.cu (+ batched_sym.cu: the kernels behind `symmetric`) -- the request's arguments are checked for null and

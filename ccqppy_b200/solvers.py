@@ -22,7 +22,10 @@ Extensions beyond the reference API (all optional):
   * a float32 dense A stays float32 (`ccqp_set_matrix_f32`): the kernels stream it at 4 bytes per entry and widen every
     entry exactly in a register, which is what NumPy does for the reference's `A.dot(v)` with a float32 A -- the result
     has the same bits as the solve of `A.astype(np.float64)`, for half the HBM and PCIe bytes and half the device memory.
-    `symmetric=True`, sparse A and `solve_batched` widen a float32 A to float64 as before.
+    `symmetric=True` and sparse A widen a float32 A to float64 as before.
+  * `solve_batched` keeps a float32 dense A [batch, n, n] float32 as well, for every feasible-set form (the `_f32` batched
+    entry points): the kernels widen each entry exactly in a register when they load the problem, so the results are the
+    bits of the widened call, for half the bytes of A moved over PCIe and HBM and no float64 copy on the device.
 """
 import ctypes
 import time
@@ -94,15 +97,17 @@ def _as_f64(a, like_device=None):
     return arr
 
 
-def _as_f32_matrix(a):
+def _as_f32_matrix(a, aligned=True):
     """A float32 dense NumPy array / torch tensor as the C-contiguous float32 array / tensor ccqp_set_matrix_f32 takes
     (no widening); None for any other input.  A CUDA tensor is used as it is when it is contiguous and 16-byte aligned;
-    otherwise ONE contiguous copy is made, so its rows take the same mat-vec loop as a widened copy of `a` would."""
+    otherwise ONE contiguous copy is made, so its rows take the same mat-vec loop as a widened copy of `a` would.
+    aligned=False (batched solves, whose load path never changes the values): a contiguous CUDA tensor is used as it is
+    at any alignment."""
     if isinstance(a, np.ndarray):
         return np.ascontiguousarray(a) if a.dtype == np.float32 else None
     if not _is_torch(a) or str(a.dtype) != "torch.float32" or str(a.layout) != "torch.strided":
         return None
-    if a.is_contiguous() and (not a.is_cuda or a.data_ptr() % 16 == 0):
+    if a.is_contiguous() and (not a.is_cuda or not aligned or a.data_ptr() % 16 == 0):
         return a
     import torch
     return a.clone(memory_format=torch.contiguous_format)
@@ -303,7 +308,12 @@ class CCQPSolverBase(ABC):
         `symmetric=True` declares every A[i] symmetric (what the reference's objective assumes): with per-problem
         boxes, n <= 64 and PGD / BBPGD / BBPGDf / SPG the one-warp-per-problem kernels then read only the upper block
         triangle of A[i] (entries [r][c] with c >= 8 * (r // 8); `ccqp_solve_batched_sym`); every other case runs the
-        general kernels.  The caller vouches for the symmetry: it is not checked."""
+        general kernels.  The caller vouches for the symmetry: it is not checked.
+
+        A float32 A (NumPy array, or a strided torch tensor on the host or on CUDA) is not widened: it goes to the `_f32`
+        twin of the entry point (a contiguous CUDA tensor is read in place at any alignment, anything non-contiguous gets
+        one contiguous float32 copy) and the results equal bit for bit those of `A.astype(np.float64)`.  Any other dtype
+        is widened to float64.  An A that is not [batch, n, n] raises ValueError, a sparse torch tensor TypeError."""
         time_start = time.time()
         if not self.quiet:
             print("solving " + self._label)
@@ -311,8 +321,13 @@ class CCQPSolverBase(ABC):
         dev = A.device if on_device else None
         if on_device:
             device = A.device.index if A.device.index is not None else -1
-        A64 = _as_f64(A, dev)
-        batch, n = int(A64.shape[0]), int(A64.shape[1])
+        if _is_torch(A) and str(A.layout) != "torch.strided":
+            raise TypeError("solve_batched takes a dense A [batch, n, n], got a %s tensor" % A.layout)
+        A32 = _as_f32_matrix(A, aligned=False)      # a float32 batch stays float32 (the _f32 entry points)
+        Ad = A32 if A32 is not None else _as_f64(A, dev)
+        if Ad.ndim != 3 or Ad.shape[1] != Ad.shape[2]:
+            raise ValueError("A must be [batch, n, n], got shape %s" % (tuple(Ad.shape),))
+        batch, n = int(Ad.shape[0]), int(Ad.shape[1])
         b64 = _as_f64(b, dev)
         P64 = None          # per-problem parameter rows [batch, n_params], where A lives
         if op_params is not None and convex_proj_op is None:
@@ -375,23 +390,25 @@ class CCQPSolverBase(ABC):
             xout = torch.empty((batch, n), dtype=torch.float64, device=dev)
         else:
             xout = np.empty((batch, n), dtype=np.float64)
-        ptrs = [_capi.f64_ptr(v) for v in (A64, b64, x064, lb64, ub64, uni, xout)]
+        ptrs = [_capi.f64_ptr(Ad, "float64" if A32 is None else "float32")]
+        ptrs += [_capi.f64_ptr(v) for v in (b64, x064, lb64, ub64, uni, xout)]
+        f32 = "" if A32 is None else "_f32"            # the twin of each entry point that takes a float32 A
         mem = ptrs[0][1]
         results = (_capi.Result * batch)()
         summary = _capi.Result()
         prm = self._params()
         if P64 is not None:
             pp, _, _kp = _capi.f64_ptr(P64)
-            st = lib.ccqp_solve_batched_tables(h.h, self._solver_id, ctypes.byref(prm), batch, n, ptrs[0][0], ptrs[1][0],
-                                               ptrs[2][0], blocks.ptr, len(blocks), pp, int(P64.shape[1]), ptrs[5][0], K,
-                                               ptrs[6][0], mem, results, ctypes.byref(summary))
+            entry = getattr(lib, "ccqp_solve_batched_tables" + f32)
+            st = entry(h.h, self._solver_id, ctypes.byref(prm), batch, n, ptrs[0][0], ptrs[1][0], ptrs[2][0], blocks.ptr,
+                       len(blocks), pp, int(P64.shape[1]), ptrs[5][0], K, ptrs[6][0], mem, results, ctypes.byref(summary))
         elif convex_proj_op is not None:
             pp, _, _kp = _capi.f64_ptr(params if params.size else np.zeros(1))
-            st = lib.ccqp_solve_batched_table(h.h, self._solver_id, ctypes.byref(prm), batch, n, ptrs[0][0], ptrs[1][0],
-                                              ptrs[2][0], blocks.ptr, len(blocks), pp, params.size, ptrs[5][0], K,
-                                              ptrs[6][0], mem, results, ctypes.byref(summary))
+            entry = getattr(lib, "ccqp_solve_batched_table" + f32)
+            st = entry(h.h, self._solver_id, ctypes.byref(prm), batch, n, ptrs[0][0], ptrs[1][0], ptrs[2][0], blocks.ptr,
+                       len(blocks), pp, params.size, ptrs[5][0], K, ptrs[6][0], mem, results, ctypes.byref(summary))
         else:
-            entry = lib.ccqp_solve_batched_sym if symmetric else lib.ccqp_solve_batched
+            entry = getattr(lib, ("ccqp_solve_batched_sym" if symmetric else "ccqp_solve_batched") + f32)
             st = entry(h.h, self._solver_id, ctypes.byref(prm), batch, n, ptrs[0][0], ptrs[1][0],
                        ptrs[2][0], ptrs[3][0], ptrs[4][0], ptrs[5][0], K, ptrs[6][0], mem, results,
                        ctypes.byref(summary))

@@ -254,6 +254,37 @@ ccqp_status ccqp_solve_batched_tables(ccqp_handle* h, int solver, const ccqp_par
                                       int64_t n_params, const double* uniforms, int64_t n_uniforms, double* x_out,
                                       int memtype, ccqp_result* results, ccqp_result* summary);
 
+/* The four batched calls for a Hessian batch STORED as IEEE fp32: A is float [batch][n][n], contiguous; every other argument,
+ * check and status code is that of the fp64 function of the same name without _f32.  The arithmetic stays fp64: every
+ * entry is widened exactly in a register when the problem's A is loaded, which is what NumPy does for the reference's
+ * A.dot(v) with a float32 A (solvers.py:133), and nothing after that load depends on the storage type -- on every path
+ * (host or device A, any alignment, any n, symmetric or general kernels, box or table) the solutions, residuals, counts,
+ * converged flags and statuses equal bit for bit those of the fp64 call on A widened to double.  A DEVICE batch is read in
+ * place (any 4-byte alignment: a base off a 16-byte boundary, or n % 4 != 0, loads entry by entry instead of by bulk row
+ * copies); a HOST batch is copied to the device at 4 bytes per entry (asynchronous from pinned memory).  Half the HBM and
+ * PCIe bytes of A: result.hbm_bytes and summary.hbm_bytes count 4 bytes per entry of A read (ccqp_solve_batched_sym_f32:
+ * per entry of the upper block triangle, where that kernel runs). */
+ccqp_status ccqp_solve_batched_f32(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch,
+                                   int64_t n, const float* A, const double* b, const double* x0,
+                                   const double* lb, const double* ub, const double* uniforms,
+                                   int64_t n_uniforms, double* x_out, int memtype,
+                                   ccqp_result* results, ccqp_result* summary);
+ccqp_status ccqp_solve_batched_sym_f32(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch,
+                                       int64_t n, const float* A, const double* b, const double* x0,
+                                       const double* lb, const double* ub, const double* uniforms,
+                                       int64_t n_uniforms, double* x_out, int memtype,
+                                       ccqp_result* results, ccqp_result* summary);
+ccqp_status ccqp_solve_batched_table_f32(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch,
+                                         int64_t n, const float* A, const double* b, const double* x0,
+                                         const ccqp_block* blocks, int64_t n_blocks, const double* block_params,
+                                         int64_t n_params, const double* uniforms, int64_t n_uniforms, double* x_out,
+                                         int memtype, ccqp_result* results, ccqp_result* summary);
+ccqp_status ccqp_solve_batched_tables_f32(ccqp_handle* h, int solver, const ccqp_params* params, int64_t batch,
+                                          int64_t n, const float* A, const double* b, const double* x0,
+                                          const ccqp_block* blocks, int64_t n_blocks, const double* block_params,
+                                          int64_t n_params, const double* uniforms, int64_t n_uniforms, double* x_out,
+                                          int memtype, ccqp_result* results, ccqp_result* summary);
+
 /* ---- unit-test hooks for the pieces of the path ---------------------------------------------- */
 /* y = A v for the handle's row shard (y has n_rows entries).  A.dot(v), solvers.py:133 etc. */
 ccqp_status ccqp_gemv(ccqp_handle* h, const double* v, double* y, int memtype);
