@@ -220,8 +220,11 @@ Tiling choose_tiling(const ccqp_handle* h) {
     };
     for (;;) {
         layout();
-        if (t.smem <= kDenseSmemTarget || t.SW >= t.CW) break;
-        t.SW *= 2;   // fewer, wider segments when a CTA owns many rows of a very wide matrix
+        // fewer, wider segments when a CTA owns many rows of a very wide matrix; only while 2 SW still divides CW: the
+        // psum slot of (panel p, segment s) is p * (CW / SW) + s, so a width that does not divide CW would give a full
+        // panel more segments than slots and its last segment would land in the next panel's first slot
+        if (t.smem <= kDenseSmemTarget || t.CW % (2 * t.SW) != 0) break;
+        t.SW *= 2;
     }
     if (t.smem > kDenseSmemTarget) {
         // very wide matrices (n beyond ~100k on one GPU): one partial sum per (row, segment of the whole row) no

@@ -44,7 +44,7 @@ class EmulatedBox:
 
     def solve(self, solver, b, x0=None, uniforms=None):
         """solver: a ccqppy_b200.solvers object (tolerance / limits / hyper-parameters).  Returns a list of
-        per-rank dicts (solution, mv, gemv, converged, residual, status)."""
+        per-rank dicts (solution, mv, gemv, converged, residual, status, draws = SPG uniforms consumed)."""
         n, world = self.n, self.world
         b64 = np.ascontiguousarray(b, dtype=np.float64)
         x064 = None if x0 is None else np.ascontiguousarray(x0, dtype=np.float64)
@@ -59,7 +59,8 @@ class EmulatedBox:
             raise NotImplementedError("Cone normal not implemented, yet.")
         _capi.check(self.handles[0].h, st)
         return [dict(solution=xout[r].copy(), mv=int(res[r].mv_count), gemv=int(res[r].gemv_count), converged=bool(res[r].converged),
-                     residual=float(res[r].residual), status=int(res[r].status), gpu_seconds=float(res[r].gpu_seconds))
+                     residual=float(res[r].residual), status=int(res[r].status), gpu_seconds=float(res[r].gpu_seconds),
+                     draws=int(res[r].uniforms_used))
                 for r in range(world)]
 
     def close(self):

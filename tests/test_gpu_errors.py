@@ -73,7 +73,7 @@ def test_spg_uniform_stream_and_range_errors():
 
 def test_mv_limit_edge_cases_do_not_raise():
     """SURVEY Q16: where the reference would die with NameError (limit hit before the first residual exists) the
-    result is residual = NaN, converged = False."""
+    result is residual = NaN, converged = False.  test_gpu_trajectories.py compares every such stop with the oracle."""
     n = 30
     A, b = pr.shift_problem(n, 2)
     tab = pr.box_table(n)
